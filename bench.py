@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - the headline benchmark of the hot path on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -29,6 +29,8 @@ the measured path and says so in ``config``).  ``cpu_baseline`` is the reference
 path (its own C++ sum-factorisation templates when oracle/_ref is built, else the C
 port) timed on this host's cores on a bounded sample of the same workload.
 ``--workload linear_piston|nonlinear_bowl`` time BASELINE.json's other demo configs.
+``--dump-outputs DIR`` writes the state the K timed steps leave behind, so that two builds
+run with the same arguments (hence the same inputs) can be compared output for output.
 """
 
 from __future__ import annotations
@@ -281,6 +283,36 @@ def reference_cuda_arm(n, degree, dtype, reps=10):
 
 
 # --------------------------------------------------------------------------- #
+# outputs of the timed path, for comparing two builds
+# --------------------------------------------------------------------------- #
+
+DUMP_BYTES = 32 << 20  # every rank's arrays together: within 64 MB with the .npy headers
+DUMP_SEED = 20261020
+
+
+def dump_indices(n, itemsize, narrays, rank=0, world=1):
+    """Sorted indices of the first ``n`` entries that one of ``world`` ranks writes for each of its
+    ``narrays`` arrays of ``itemsize``-byte floats, so that all ranks together write at most
+    DUMP_BYTES.  All ``n`` when they fit the rank's share; else the share split into k equal
+    strata of [0, n) with one index drawn in each, seeded by DUMP_SEED and the rank: the same
+    indices for every run with the same arguments, at O(k) cost."""
+    k = DUMP_BYTES // (world * narrays * itemsize)
+    if n <= k:
+        return np.arange(n, dtype=np.int64)
+    edges = np.arange(k + 1, dtype=np.int64) * n // k
+    rng = np.random.default_rng([DUMP_SEED, rank])
+    return edges[:-1] + (rng.random(k) * np.diff(edges)).astype(np.int64)
+
+
+def dump_outputs(out_dir, arrays, rank=0, world=1):
+    """Write each tensor of ``arrays`` to ``out_dir/<name>.npy`` (``<name>_rank<r>.npy`` with
+    several ranks) in its own float type."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{'' if world == 1 else f'_rank{rank}'}.npy"), t.cpu().numpy())
+
+
+# --------------------------------------------------------------------------- #
 # main
 # --------------------------------------------------------------------------- #
 
@@ -317,8 +349,16 @@ def main():
     ap.add_argument("--cpu-kind", default=None, choices=["numba", "cpp", "port"], help="CPU arm implementation")
     ap.add_argument("--sustain-steps", type=int, default=250, help="steps of the extra >= 1 s sustained measurement")
     ap.add_argument("--watchdog", type=int, default=0, help="dump all Python stacks to stderr after this many seconds")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the state they leave (u, v) to DIR/<name>.npy, "
+                         "DIR/<name>_rank<r>.npy with several GPUs; on large meshes a seeded sample, all files "
+                         "together at most 32 MiB")
     ap.add_argument("-v", "--verbose", action="store_true")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs: the timed path of --impl ours only")
     if a.watchdog > 0:
         import faulthandler
 
@@ -481,6 +521,8 @@ def main():
     except Exception:
         pass
     cvd = [v for v in os.environ.get("CUDA_VISIBLE_DEVICES", "").split(",") if v.strip().isdigit()]
+    if a.dump_outputs:
+        dump_idx = torch.from_numpy(dump_indices(info["nlocal"], s, 2, rank, world)).cuda()
     clocks = Clocks(uuid or (int(cvd[local_rank]) if local_rank < len(cvd) else local_rank))
     clocks.start()
     solver.init()
@@ -500,6 +542,9 @@ def main():
     gdofs_global = info["global_dofs"]
     value = gdofs_global * NST * a.steps / elapsed / 1e9
     log(f"timed region done: {elapsed * 1e3 / a.steps:.3f} ms/step")
+    # the state the timed steps leave, gathered on the device before the next steps overwrite it;
+    # copied to the host and written once the clock sampling below has stopped
+    dumped = {"u": solver.u[dump_idx], "v": solver.v[dump_idx]} if a.dump_outputs else None
 
     # ---- sustained: the same steps for >= 1 s (the contract's K is short); the clocks are sampled
     #      from the start of the timed region to the end of this one (all of it the same workload) ----
@@ -518,6 +563,8 @@ def main():
     w1 = time.time()
     clk = clocks.stop(w0, w1)
     clk["window"] = "timed region + sustained run (same steps)"
+    if dumped is not None:
+        dump_outputs(a.dump_outputs, dumped, rank, world)
     if world > 1:  # every rank's GPU, not only rank 0's
         allc = [None] * world
         dist.all_gather_object(allc, clk)

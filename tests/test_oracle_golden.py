@@ -37,7 +37,7 @@ def test_operators_match_reference(golden_dir, P, tag):
 @pytest.mark.parametrize("tag", ["f64", "f32"])
 def test_compiled_reference_templates_match(golden_dir, P, tag):
     if orc.ref_lib() is None:
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
+        pytest.skip("oracle/_ref not built: needs the reference's C++ sources, which the repository does not hold")
     g = _load(golden_dir, f"operators_P{P}_{tag}.npz")
     y = np.zeros(g["x"].size, g["x"].dtype)
     orc.ref_stiffness_operator(P, g["x"], g["coeff"], y, g["G"], g["dofmap"], g["dphi_1D"])
