@@ -23,10 +23,7 @@ from __future__ import annotations
 import numpy as np
 
 from . import _lib
-from ._lib import check, current_stream, dev, fn
-
-FUS_TABLES_RESIDENT = 1
-FUS_NO_ATOMICS = 2
+from ._lib import FUS_NO_ATOMICS, FUS_TABLES_RESIDENT, check, current_stream, dev, fn
 
 
 class _Kernel:

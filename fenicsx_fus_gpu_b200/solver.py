@@ -56,19 +56,18 @@ from collections import namedtuple
 import numpy as np
 
 from . import _lib
-from ._lib import check, current_stream, fn
+from ._lib import FUS_TABLES_RESIDENT, check, current_stream, fn
 
 # a contiguous range of (permuted) cells that one kernel launch covers:
 # kind 0 rectilinear, 1 affine, 2 streamed G; c0/n cell range; g0 first row of the streamed G / detJ
 # arrays; ninterior: the first ninterior cells of the range touch no ghost dof (peer-memory halo: the
 # launch waits for the forward exchange only before its remaining, interface, cells)
 Seg = namedtuple("Seg", "kind c0 n g0 ninterior")
+KIND_SUFFIX = ("_rect", "_affine", "")  # cell-kernel symbol fus_<form><suffix> per Seg.kind
 
 A_RUNGE = (0.0, 0.5, 0.5, 1.0)
 B_RUNGE = (1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0)
 C_RUNGE = (0.0, 0.5, 0.5, 1.0)
-
-FUS_TABLES_RESIDENT = 1
 
 
 def _torch():
@@ -118,10 +117,16 @@ def westervelt_source(t, f0, p0, c0, alpha=4.0):
 
 
 class _RK4:
-    """State vectors, boundary diagonals, graph capture and the step loop shared
-    by the linear and Westervelt solvers."""
+    """State vectors, boundary diagonals, graph capture, the stage sequence and the step loop
+    shared by the linear and Westervelt solvers.
+
+    A solver class states its cell-kernel form (``form``: the kernels ``fus_<form>[_rect|_affine]``,
+    and ``_operands``: their leading arguments for a cell range) and its close (``_close_name``:
+    the bulk close kernel, ``_close_variant``: its variant of ``fus_rk_close_shared``, ``_masses``:
+    the (m, m0, m2, m5) it reads)."""
 
     westervelt = False
+    integrator = "rk4"
 
     def __init__(self, P, float_type, ndofs, dofmap, G, dphi_1D, halo=None, source=None,
                  source_at_stage_time=True, use_graph=True, geometry="stream", weights=None,
@@ -197,7 +202,7 @@ class _RK4:
         self._weights = None if weights is None else _dev(weights, self.T)
         self.nrect = 0  # number of rectilinear cells (affine, diagonal Gc)
         self.naff = 0  # number of affine cells (rectilinear ones included)
-        self.Gc = self.detJc = None
+        self.detJ = self.Gc = self.detJc = None
         self._rect_tables = None
         self.cell_perm = None
         # cell ranges, one launch each (per geometry kind; interior cells first inside a range)
@@ -242,21 +247,27 @@ class _RK4:
                                              dofmap.data_ptr(), dofmap.shape[0], dofmap.shape[1],
                                              current_stream()), "fus_mass")
 
-    def _boundary_setup(self, terms):
-        """``terms``: list of (slot, bfacet_dofmap, detJ_f, facet_coeff) with slot in
-        {"src", "src2", "absb"}.  Builds the compact unique-dof list and the
-        diagonals = the facet mass operator applied to ones (cuda/demo_linear_box.py:546-551)."""
+    def _facets(self, bfacet_dofmap, detJ_f, facet_coeff):
+        """(bfacet_dofmap, detJ_f, facet_coeff) of a boundary facet group on the device, or None
+        when the group is empty."""
+        if bfacet_dofmap is None:
+            return None
+        bd = _dev(bfacet_dofmap, _torch().int32)
+        return (bd, _dev(detJ_f, self.T), _dev(facet_coeff, self.T)) if bd.shape[0] else None
+
+    def _boundary_setup(self, **groups):
+        """``groups``: slot ("src", "src2", "absb") -> facet group of ``_facets`` or None.  Builds
+        the compact unique-dof list and the diagonals = the facet mass operator applied to ones
+        (cuda/demo_linear_box.py:546-551)."""
         torch = _torch()
-        ones = torch.ones(self.ndofs, dtype=self.T, device="cuda")
-        dofs = [t[1].reshape(-1) for t in terms if t[1].shape[0]]
-        if not dofs:
+        groups = {slot: g for slot, g in groups.items() if g is not None}
+        if not groups:
             self._bdofs = torch.zeros(0, dtype=torch.int32, device="cuda")
             return
-        self._bdofs = torch.unique(torch.cat(dofs)).to(torch.int32).contiguous()
+        self._bdofs = torch.unique(torch.cat([g[0].reshape(-1) for g in groups.values()])).to(torch.int32).contiguous()
         idx = self._bdofs.to(torch.int64)
-        for slot, bdm, dJ, coeff in terms:
-            if not bdm.shape[0]:
-                continue
+        ones = torch.ones(self.ndofs, dtype=self.T, device="cuda")
+        for slot, (bdm, dJ, coeff) in groups.items():
             tmp = torch.zeros(self.ndofs, dtype=self.T, device="cuda")
             self._mass(ones, coeff, tmp, dJ, bdm)
             setattr(self, "_" + slot, tmp[idx].contiguous())
@@ -301,6 +312,7 @@ class _RK4:
             iface = torch.zeros(nc, dtype=torch.bool, device="cuda")
         key = kind * 2 + iface.to(torch.int32)  # rect [interior | interface], affine [..], streamed [..]
         counts = torch.bincount(key, minlength=6).cpu().tolist()
+        perm = None
         if not bool((key[1:] >= key[:-1]).all().item()):
             perm = torch.argsort(key, stable=True)  # original order kept inside every range
             self.cell_perm = perm
@@ -309,13 +321,11 @@ class _RK4:
                 setattr(self, name, getattr(self, name)[perm].contiguous())
             if Gc is not None:
                 Gc, detJc = Gc[perm], detJc[perm]
-            rows = perm[kind[perm] == 2] if self.naff else perm
+        if perm is not None or self.naff:
+            # G / detJ rows of the streamed cells only, in launch order (the caller's tensors are not touched)
+            rows = torch.arange(nc, device="cuda") if perm is None else perm
+            rows = rows[kind[rows] == 2]
             self.G = self.G[rows].contiguous() if rows.numel() else None
-            if detJ is not None:
-                self.detJ = detJ[rows].contiguous() if rows.numel() else None
-        elif self.naff:  # already ordered (e.g. every cell affine): drop the rows nothing streams
-            rows = torch.nonzero(kind == 2).reshape(-1)
-            self.G = self.G[rows].contiguous() if rows.numel() else None  # (the caller's tensor is not touched)
             if detJ is not None:
                 self.detJ = detJ[rows].contiguous() if rows.numel() else None
         if self.naff:
@@ -374,15 +384,6 @@ class _RK4:
             self.halo.barrier()  # nobody's first put may land before this rank is set up
         self._opened = True
 
-    def _assemble(self, stage, g, dg, use_table, x, vn, wait=False):  # pragma: no cover - abstract
-        raise NotImplementedError
-
-    def _close(self, stage, dt, count_step, base, acc, skip=None, n=None):  # pragma: no cover - abstract
-        raise NotImplementedError
-
-    def _close_shared(self, stage, dt, base, acc):  # pragma: no cover - abstract
-        raise NotImplementedError
-
     def _sptr(self, t, row):
         """Device address of row ``row`` of a per-cell tensor (no view objects on the launch path)."""
         return t.data_ptr() + int(row) * t.stride(0) * t.element_size()
@@ -410,67 +411,89 @@ class _RK4:
         if first is not None:
             self.halo.arm_stiffness_wait(first)
 
-    def _enqueue_step(self, dt, t, use_table, parity=None):
-        """The launches of one RK4 step whose base state is ``_uv[parity]`` (default: the current
-        one); the new state is left in ``_uv[1 - parity]``.  Does not flip ``_parity``."""
-        parity = self._parity if parity is None else parity
-        base, acc = self._uv[parity], self._uv[1 - parity]
-        if self.p2p:
-            return self._enqueue_step_p2p(dt, t, use_table, base, acc)
-        for i in range(4):
-            g = dg = 0.0
-            if not use_table and self.source is not None:
-                g, dg = self.source(t + C_RUNGE[i] * dt if self.source_at_stage_time else t)
-            # stage input: the base state itself in stage 0 (a_0 = 0), un / vn (= ku) afterwards
-            x, vn = base if i == 0 else (self.un, self.ku)
-            if self.halo is not None:
-                self.halo.forward(x, vn)
-            self._assemble(i, g, dg, use_table, x, vn)
-            self._boundary(i, g, dg, use_table, vn)
-            if self.halo is not None:
-                if self._m_accum:
-                    self.halo.reverse(self.b, self.m)
-                else:
-                    self.halo.reverse(self.b)
-            self._close(i, dt, use_table, base, acc)
+    def _cell_kernels(self, x, vn, wait=False):
+        """The cell-kernel launches of a stage: ``fus_<form><KIND_SUFFIX>`` over every cell range, with
+        the form's operands, then the range's geometry (G or Gc; detJ or detJc when the form carries
+        the cell-mass pair; the quadrature weights for affine cells), then the common tail."""
+        st, sp = current_stream(), self._sptr
+        for sg, first in self._launches(wait):
+            G, dJ, row = (self.G, self.detJ, sg.g0) if sg.kind == 2 else (self.Gc, self.detJc, sg.c0)
+            geo = (sp(G, row), sp(dJ, row)) if self._m_accum else (sp(G, row),)
+            if sg.kind == 1:
+                geo += (self._weights.data_ptr(),)
+            self._arm(first)
+            name = f"fus_{self.form}{KIND_SUFFIX[sg.kind]}"
+            check(fn(name, self.dtype)(*self._operands(x, vn, sg.c0), *geo, sp(self.dofmap, sg.c0), None, sg.n,
+                                       self.P, FUS_TABLES_RESIDENT, st), name)
 
-    def _enqueue_step_p2p(self, dt, t, use_table, base, acc):
-        """One RK4 step with the peer-memory halo overlapped with compute (module docstring).
+    def _assemble(self, x, vn, wait=False):
+        """The cell kernels of a stage as one group for ``probe``."""
+        self._probed(lambda: self._cell_kernels(x, vn, wait))
 
-        Per stage, main stream: a one-warp wait for the neighbours' puts (issued beside the
-        previous stage's close, so normally long since landed; ``split_mode`` selects the variants
-        that launch the interior cells before waiting); the stiffness launches; the boundary
-        terms, whose last block signals "my ghost sums are complete"; the close on the dofs nobody
-        shares.  Exchange stream, beside that close: a one-warp wait for the neighbours' signals,
-        then ONE kernel that gathers their ghost sums, closes the shared dofs and puts the next
-        stage input into the neighbours' ghost slots.
+    def _assemble_exchanged(self, stage, g, dg, use_table, x, vn):
+        """b (, m) of a stage with the halo as blocking rounds: forward exchange of the input, cell
+        kernels, boundary terms, reverse exchange of the sums."""
+        if self.halo is not None:
+            self.halo.forward(x, vn)
+        self._assemble(x, vn)
+        self._boundary(stage, g, dg, use_table, vn)
+        if self.halo is not None:
+            self.halo.reverse(*((self.b, self.m) if self._m_accum else (self.b,)))
+
+    def _source_at(self, stage, dt, t, use_table):
+        """(g, dg) of ``stage`` of the step from ``t``, evaluated on the host; zeros when the
+        launches read them from the device table."""
+        if use_table or self.source is None:
+            return 0.0, 0.0
+        return self.source(t + C_RUNGE[stage] * dt if self.source_at_stage_time else t)
+
+    def _stage(self, stage, dt, t, use_table, base, acc):
+        """The launches of one stage of the step from ``base`` into ``acc``, under any halo.
+
+        Peer-memory halo (module docstring), main stream: a one-warp wait for the neighbours' puts
+        (issued beside the previous stage's close, so normally long since landed; ``split_mode``
+        selects the variants that launch the interior cells before waiting); the cell kernels; the
+        boundary terms, whose last block signals "my ghost sums are complete"; the close on the
+        dofs nobody shares.  Exchange stream, beside that close: a one-warp wait for the
+        neighbours' signals, then ONE kernel that gathers their ghost sums, closes the shared dofs
+        and puts the next stage input into the neighbours' ghost slots.
 
         Ordering across GPUs: every wait depends only on signals the neighbours raise from kernels
         that are stream-ordered after kernels of EARLIER phases of this rank, so the step can be
         captured and replayed as a graph without deadlock.  A neighbour's put of stage i+1 is
         issued by the kernel that gathered (and cleared) my ghost sums of stage i, so its FWD epoch
         also says the ghost accumulators are clean."""
+        g, dg = self._source_at(stage, dt, t, use_table)
+        # stage input: the base state itself in stage 0 (a_0 = 0), un / vn (= ku) afterwards; with the
+        # peer-memory halo it is on its way to (or already in) the ghost slots: put there by
+        # begin_steps() or by the previous stage's close of the shared dofs
+        x, vn = base if stage == 0 else (self.un, self.ku)
         h = self.halo
+        if not self.p2p:
+            self._assemble_exchanged(stage, g, dg, use_table, x, vn)
+            self._close(stage, dt, use_table, base, acc)
+            return
+        # (the leapfrog step always waits before its launches)
+        in_kernel = self.integrator == "rk4" and self.split_cells and self.split_mode in ("two", "fused")
+        if in_kernel:
+            h.sync_point()
+        else:
+            h.wait_forward()
+        self._assemble(x, vn, wait=in_kernel)
+        self._boundary(stage, g, dg, use_table, vn, signal=True, consume=in_kernel)
+        h.fork()
+        with h.side():
+            h.wait_reverse()
+            self._close_shared(stage, dt, base, acc)
+        self._close(stage, dt, use_table, base, acc, **h.bulk_close())
+        h.join()
+
+    def _enqueue_step(self, dt, t, use_table, parity=None):
+        """The launches of one RK4 step whose base state is ``_uv[parity]`` (default: the current
+        one); the new state is left in ``_uv[1 - parity]``.  Does not flip ``_parity``."""
+        parity = self._parity if parity is None else parity
         for i in range(4):
-            g = dg = 0.0
-            if not use_table and self.source is not None:
-                g, dg = self.source(t + C_RUNGE[i] * dt if self.source_at_stage_time else t)
-            # the stage input is on its way to (or already in) the ghost slots: put there by
-            # begin_steps() or by the previous stage's close of the shared dofs
-            x, vn = base if i == 0 else (self.un, self.ku)
-            in_kernel = self.split_cells and self.split_mode in ("two", "fused")
-            if in_kernel:
-                h.sync_point()
-            else:
-                h.wait_forward()
-            self._assemble(i, g, dg, use_table, x, vn, wait=in_kernel)
-            self._boundary(i, g, dg, use_table, vn, signal=True, consume=in_kernel)
-            h.fork()
-            with h.side():
-                h.wait_reverse()
-                self._close_shared(i, dt, base, acc)
-            self._close(i, dt, use_table, base, acc, **h.bulk_close())
-            h.join()
+            self._stage(i, dt, t, use_table, self._uv[parity], self._uv[1 - parity])
 
     def begin_steps(self):
         """Peer-memory halo: send the current state to the neighbours' ghost slots before a run
@@ -478,7 +501,7 @@ class _RK4:
         otherwise."""
         if self.p2p:
             self.halo.barrier()  # the neighbours are done reading the ghost values about to be replaced
-            self.halo.put(*self._uv[self._parity])
+            self.halo.put(self.u, self.v)
 
     def end_steps(self):
         """Consume the put the last step of a run left pending (keeps puts and waits paired)."""
@@ -492,6 +515,25 @@ class _RK4:
         adt = 0.0 if stage == 3 else A_RUNGE[stage + 1] * dt
         return (acc[0].data_ptr(), acc[1].data_ptr(), base[0].data_ptr(), base[1].data_ptr(),
                 B_RUNGE[stage] * dt, adt, mode)
+
+    def _close(self, stage, dt, count_step, base, acc, skip=None, n=None):
+        """Close of ``stage`` on the dofs this rank updates alone: every owned one, or beside
+        ``_close_shared`` the prefix ``n`` / the dofs outside the ``skip`` mask."""
+        u, v, u0, v0, bdt, adt, mode = self._close_args(stage, dt, base, acc)
+        masses = [t.data_ptr() for t in self._masses() if t is not None]
+        check(fn(self._close_name, self.dtype)(
+            u, v, u0, v0, self.ku.data_ptr(), None, self.un.data_ptr(), self.b.data_ptr(), *masses, bdt, adt, mode,
+            self.nupd if n is None else n, self.step_dev.data_ptr() if count_step else None, skip, current_stream()),
+            self._close_name)
+
+    def _close_shared(self, stage, dt, base, acc):
+        """Close of ``stage`` on the shared dofs (peer-memory halo): gathers the neighbours' ghost
+        sums, closes and puts the next stage input into their ghost slots."""
+        u, v, u0, v0, bdt, adt, mode = self._close_args(stage, dt, base, acc)
+        ku, un = (self.ku.data_ptr(), self.un.data_ptr()) if self.integrator == "rk4" else (None, None)
+        check(fn("fus_rk_close_shared", self.dtype)(
+            self.halo.handle, self._close_variant, 1, 1, u, v, u0, v0, ku, un, self.b.data_ptr(),
+            *(self._ptr(t) for t in self._masses()), bdt, adt, mode, current_stream()), "fus_rk_close_shared")
 
     # ---- public --------------------------------------------------------------
     def init(self):
@@ -509,9 +551,7 @@ class _RK4:
         t = t0
         for k in range(nsteps):
             for i in range(4):
-                if self.source is not None:
-                    tab[k, 2 * i], tab[k, 2 * i + 1] = self.source(
-                        t + C_RUNGE[i] * dt if self.source_at_stage_time else t)
+                tab[k, 2 * i], tab[k, 2 * i + 1] = self._source_at(i, dt, t, False)
             t += dt
         return tab
 
@@ -614,14 +654,19 @@ class _RK4:
     def _state(self):
         return [*self._uv[0], *self._uv[1], self.ku, self.un, self.b, self.m]
 
-    # algorithmic HBM bytes of one RK stage (SURVEY.md section 8d)
-    def stage_bytes(self):
+    # algorithmic HBM bytes (SURVEY.md section 8d)
+    def _stiffness_bytes(self):
+        """One stiffness action: dofmap, G (or the compressed factors) and a coefficient per cell,
+        x read and b written per dof."""
         s = self.dtype.itemsize
         Nd = self.n**3
         nstream = self.ncells - self.naff
-        stiff = nstream * (Nd * 4 + 6 * Nd * s + s) + self.naff * (Nd * 4 + 7 * s) + 2 * s * self.ndofs
-        # vector passes of the close kernels per step: 9 + 12 + 12 + 8 (ping-pong), i.e. 10.25 a stage
-        return stiff + 10.25 * s * self.ndofs
+        return nstream * (Nd * 4 + 6 * Nd * s + s) + self.naff * (Nd * 4 + 7 * s) + 2 * s * self.ndofs
+
+    def stage_bytes(self):
+        """One RK stage: vector passes of the close kernels per step 9 + 12 + 12 + 8 (ping-pong),
+        i.e. 10.25 a stage."""
+        return self._stiffness_bytes() + 10.25 * self.dtype.itemsize * self.ndofs
 
     def stage_bytes_survey(self):
         """SURVEY.md section 8(d)'s model of a fused linear stage: 6s + stiffness + 8s per dof."""
@@ -654,54 +699,24 @@ class LinearSpectral3D(_RK4):
         self._mass(ones, c1, self.m, dJ, self.dofmap)
         if self.halo is not None:
             self.halo.reverse(self.m)
-        terms = []
-        e = lambda w: torch.zeros((0, self.n**2), dtype=w, device="cuda")  # noqa: E731
-        bd1 = _dev(bfacet_dofmap1, torch.int32) if bfacet_dofmap1 is not None else e(torch.int32)
-        bd2 = _dev(bfacet_dofmap2, torch.int32) if bfacet_dofmap2 is not None else e(torch.int32)
-        if bd1.shape[0]:
-            terms.append(("src", bd1, _dev(detJ_f1, self.T), _dev(facet_coeff1, self.T)))
-        if bd2.shape[0]:
-            terms.append(("absb", bd2, _dev(detJ_f2, self.T), _dev(facet_coeff2, self.T)))
-        self._boundary_setup(terms)
-        self._abs_facets = (bd2, _dev(detJ_f2, self.T), _dev(facet_coeff2, self.T)) if bd2.shape[0] else None
+        self._abs_facets = self._facets(bfacet_dofmap2, detJ_f2, facet_coeff2)
+        self._boundary_setup(src=self._facets(bfacet_dofmap1, detJ_f1, facet_coeff1), absb=self._abs_facets)
         self._setup_geometry(None, ["cell_coeff2"])
 
+    # b += K(-1/rho; un)                                      (cuda/demo_linear_box.py:543-545)
+    form = "stiffness"
+
+    def _operands(self, x, vn, c0):
+        return x.data_ptr(), self._sptr(self.cell_coeff2, c0), self.b.data_ptr()
+
     def _stiffness(self, x=None, wait=False):
-        x = self.un if x is None else x
-        st, xp, bp, sp = current_stream(), x.data_ptr(), self.b.data_ptr(), self._sptr
-        for sg, first in self._launches(wait):
-            cf, dm = sp(self.cell_coeff2, sg.c0), sp(self.dofmap, sg.c0)
-            self._arm(first)
-            if sg.kind == 0:  # rectilinear cells: three decoupled 1-D stiffness products
-                check(fn("fus_stiffness_rect", self.dtype)(
-                    xp, cf, bp, sp(self.Gc, sg.c0), dm, None, sg.n, self.P, FUS_TABLES_RESIDENT, st),
-                    "fus_stiffness_rect")
-            elif sg.kind == 1:  # affine cells: 6 factors per cell, nothing streamed but the dofmap
-                check(fn("fus_stiffness_affine", self.dtype)(
-                    xp, cf, bp, sp(self.Gc, sg.c0), self._weights.data_ptr(), dm, None, sg.n, self.P,
-                    FUS_TABLES_RESIDENT, st), "fus_stiffness_affine")
-            else:
-                check(fn("fus_stiffness", self.dtype)(
-                    xp, cf, bp, sp(self.G, sg.g0), dm, None, sg.n, self.P, FUS_TABLES_RESIDENT, st),
-                    "fus_stiffness")
+        self._cell_kernels(self.un if x is None else x, None, wait)
 
-    def _assemble(self, stage, g, dg, use_table, x, vn, wait=False):
-        # b += K(-1/rho; un)                                  (cuda/demo_linear_box.py:543-545)
-        self._probed(lambda: self._stiffness(x, wait))
+    # close with the lumped mass: fus_rk_close, variant 0 of fus_rk_close_shared
+    _close_name, _close_variant = "fus_rk_close", 0
 
-    def _close(self, stage, dt, count_step, base, acc, skip=None, n=None):
-        u, v, u0, v0, bdt, adt, mode = self._close_args(stage, dt, base, acc)
-        check(fn("fus_rk_close", self.dtype)(
-            u, v, u0, v0, self.ku.data_ptr(), None, self.un.data_ptr(), self.b.data_ptr(), self.m.data_ptr(),
-            bdt, adt, mode, self.nupd if n is None else n, self.step_dev.data_ptr() if count_step else None, skip, current_stream()),
-            "fus_rk_close")
-
-    def _close_shared(self, stage, dt, base, acc):
-        u, v, u0, v0, bdt, adt, mode = self._close_args(stage, dt, base, acc)
-        check(fn("fus_rk_close_shared", self.dtype)(
-            self.halo.handle, 0, 1, 1, u, v, u0, v0, self.ku.data_ptr(), self.un.data_ptr(),
-            self.b.data_ptr(), self.m.data_ptr(), None, None, None, bdt, adt, mode, current_stream()),
-            "fus_rk_close_shared")
+    def _masses(self):
+        return self.m, None, None, None
 
 
 class LinearLeapfrog3D(LinearSpectral3D):
@@ -747,11 +762,6 @@ class LinearLeapfrog3D(LinearSpectral3D):
     def v(self):
         return self._uv[0][1]
 
-    def begin_steps(self):
-        if self.p2p:
-            self.halo.barrier()
-            self.halo.put(*self._uv[0])
-
     def _lf_close(self, m, dt_v, dt_u, count_step, skip=None, n=None):
         u, v = self._uv[0]
         check(fn("fus_leapfrog_close", self.dtype)(
@@ -760,14 +770,8 @@ class LinearLeapfrog3D(LinearSpectral3D):
 
     def _kick(self, t0, dt):
         """v(t0) -> v(t0 - dt/2): half a step backwards with the acceleration at t0."""
-        u, v = self._uv[0]
-        g = self.source(t0)[0] if self.source is not None else 0.0
-        if self.halo is not None:
-            self.halo.forward(u, v)
-        self._assemble(0, g, 0.0, False, u, v)
-        self._boundary(0, g, 0.0, False, v)
-        if self.halo is not None:
-            self.halo.reverse(self.b)
+        g, dg = self._source_at(0, dt, t0, False)
+        self._assemble_exchanged(0, g, dg, False, self.u, self.v)
         self._lf_close(self.m, -0.5 * dt, 0.0, False)
         if self.p2p and self.ndofs > self.nupd:
             self.b[self.nupd:].zero_()  # the stand-alone reverse keeps the ghost sums; the steps expect them cleared
@@ -790,38 +794,24 @@ class LinearLeapfrog3D(LinearSpectral3D):
         raise NotImplementedError("LinearLeapfrog3D: use rk4 / steps")
 
     def _enqueue_step(self, dt, t, use_table, parity=None):
-        u, v = self._uv[0]
-        g = 0.0
-        if not use_table and self.source is not None:
-            g = self.source(t)[0]
-        h = self.halo
-        if self.p2p:
-            h.wait_forward()
-            self._assemble(0, g, 0.0, use_table, u, v)
-            self._boundary(0, g, 0.0, use_table, v, signal=True)
-            h.fork()
-            with h.side():
-                h.wait_reverse()
-                check(fn("fus_rk_close_shared", self.dtype)(
-                    h.handle, 3, 1, 1, u.data_ptr(), v.data_ptr(), None, None, None, None, self.b.data_ptr(),
-                    self._mlf.data_ptr(), None, None, None, dt, dt, 4, current_stream()), "fus_rk_close_shared")
-            self._lf_close(self._mlf, dt, dt, use_table, **h.bulk_close())
-            h.join()
-            return
-        if h is not None:
-            h.forward(u, v)
-        self._assemble(0, g, 0.0, use_table, u, v)
-        self._boundary(0, g, 0.0, use_table, v)
-        if h is not None:
-            h.reverse(self.b)
-        self._lf_close(self._mlf, dt, dt, use_table)
+        """One leapfrog step: one stage on ``_uv[0]`` (the ping-pong ``parity`` plays no role)."""
+        self._stage(0, dt, t, use_table, self._uv[0], self._uv[0])
+
+    # close with m - dt/2 absb: fus_leapfrog_close, variant 3 of fus_rk_close_shared (u, v are put)
+    _close_variant = 3
+
+    def _masses(self):
+        return self._mlf, None, None, None
+
+    def _close_args(self, stage, dt, base, acc):
+        return base[0].data_ptr(), base[1].data_ptr(), None, None, dt, dt, 4
+
+    def _close(self, stage, dt, count_step, base, acc, skip=None, n=None):
+        self._lf_close(self._mlf, dt, dt, count_step, skip, n)
 
     def stage_bytes(self):
         """Algorithmic HBM bytes of one leapfrog STEP: one stiffness action + 7 vector passes."""
-        s = self.dtype.itemsize
-        Nd = self.n**3
-        nstream = self.ncells - self.naff
-        return nstream * (Nd * 4 + 6 * Nd * s + s) + self.naff * (Nd * 4 + 7 * s) + 2 * s * self.ndofs + 7 * s * self.ndofs
+        return self._stiffness_bytes() + 7 * self.dtype.itemsize * self.ndofs
 
 
 class WesterveltSpectral3D(_RK4):
@@ -862,25 +852,19 @@ class WesterveltSpectral3D(_RK4):
         self.c2, self.c3 = _dev(cell_coeff2, self.T), _dev(cell_coeff3, self.T)
         self.c4, self.c5 = _dev(cell_coeff4, self.T), _dev(cell_coeff5, self.T)
         c1 = _dev(cell_coeff1, self.T)
-        e = lambda w: torch.zeros((0, self.n**2), dtype=w, device="cuda")  # noqa: E731
-        bd1 = _dev(bfacet_dofmap1, torch.int32) if bfacet_dofmap1 is not None else e(torch.int32)
-        bd2 = _dev(bfacet_dofmap2, torch.int32) if bfacet_dofmap2 is not None else e(torch.int32)
         # steady LHS m0 (cuda/demo_nonlinear_bowl.py:459-469)
         ones = torch.ones(self.ndofs, dtype=self.T, device="cuda")
         self.m0 = self._zx()  # reverse-exchanged once below: peer-addressable with the P2P halo
         self._mass(ones, c1, self.m0, self.detJ, self.dofmap)
-        if bd2.shape[0]:
-            self._mass(ones, _dev(facet_coeff1_2, self.T), self.m0, _dev(detJ_f2, self.T), bd2)
+        absorbing = self._facets(bfacet_dofmap2, detJ_f2, facet_coeff1_2)
+        if absorbing is not None:
+            bd2, dJ2, fc = absorbing
+            self._mass(ones, fc, self.m0, dJ2, bd2)
         if self.halo is not None:
             self.halo.reverse(self.m0)
-        terms = []
-        if bd1.shape[0]:
-            dJ1 = _dev(detJ_f1, self.T)
-            terms.append(("src", bd1, dJ1, _dev(facet_coeff1_1, self.T)))
-            terms.append(("src2", bd1, dJ1, _dev(facet_coeff2_1, self.T)))
-        if bd2.shape[0]:
-            terms.append(("absb", bd2, _dev(detJ_f2, self.T), _dev(facet_coeff2_2, self.T)))
-        self._boundary_setup(terms)
+        self._boundary_setup(src=self._facets(bfacet_dofmap1, detJ_f1, facet_coeff1_1),
+                             src2=self._facets(bfacet_dofmap1, detJ_f1, facet_coeff2_1),
+                             absb=self._facets(bfacet_dofmap2, detJ_f2, facet_coeff2_2))
         self.m.zero_()  # "cells" form: state-dependent part, accumulated per stage, zeroed by the close kernel
         self.m2 = self.m5 = None
         if not self._m_accum:
@@ -893,73 +877,27 @@ class WesterveltSpectral3D(_RK4):
         self._setup_geometry(self.detJ if self._m_accum else None, ["c2", "c3", "c4", "c5"])
         if not self._m_accum:
             self.detJ = None  # only the set-up needed it
+        # b += K(c3; un) + K(c4; vn) [+ M(c5; vn^2) and m += M(c2; un)]: ONE pass over G (, detJ)
+        # and the dofmap, un / vn gathered once                    (:609-612, :620-628)
+        self.form = "stiffness_westervelt" if self._m_accum else "stiffness2"
+        self._close_name, self._close_variant = (("fus_rk_close_westervelt", 1) if self._m_accum else
+                                                 ("fus_rk_close_westervelt_pw", 2))
 
     def _state(self):
         return super()._state() + [self.m0]
 
-    def _assemble(self, stage, g, dg, use_table, x, vn, wait=False):
-        # b += K(c3; un) + K(c4; vn) [+ M(c5; vn^2) and m += M(c2; un)]: ONE pass over G (, detJ)
-        # and the dofmap, un / vn gathered once                    (:609-612, :620-628)
-        self._probed(lambda: self._stage_kernel(x, vn, wait))
+    def _operands(self, x, vn, c0):
+        sp = self._sptr
+        if self._m_accum:
+            return (x.data_ptr(), sp(self.c3, c0), vn.data_ptr(), sp(self.c4, c0), sp(self.c2, c0), sp(self.c5, c0),
+                    self.m.data_ptr(), self.b.data_ptr())
+        return x.data_ptr(), sp(self.c3, c0), vn.data_ptr(), sp(self.c4, c0), self.b.data_ptr()
 
     def _stage_kernel(self, x=None, vn=None, wait=False):
-        x = self.un if x is None else x
-        vn = self.ku if vn is None else vn
-        st, sp, P, R = current_stream(), self._sptr, self.P, FUS_TABLES_RESIDENT
-        xp, vp, bp = x.data_ptr(), vn.data_ptr(), self.b.data_ptr()
-        for sg, first in self._launches(wait):
-            c0 = sg.c0
-            c3, c4, dm = sp(self.c3, c0), sp(self.c4, c0), sp(self.dofmap, c0)
-            self._arm(first)
-            if not self._m_accum:
-                # b += K(c3; un) + K(c4; vn): the dual stiffness action, one pass over G
-                if sg.kind == 0:
-                    check(fn("fus_stiffness2_rect", self.dtype)(
-                        xp, c3, vp, c4, bp, sp(self.Gc, c0), dm, None, sg.n, P, R, st), "fus_stiffness2_rect")
-                elif sg.kind == 1:
-                    check(fn("fus_stiffness2_affine", self.dtype)(
-                        xp, c3, vp, c4, bp, sp(self.Gc, c0), self._weights.data_ptr(), dm, None, sg.n, P, R, st),
-                        "fus_stiffness2_affine")
-                else:
-                    check(fn("fus_stiffness2", self.dtype)(
-                        xp, c3, vp, c4, bp, sp(self.G, sg.g0), dm, None, sg.n, P, R, st), "fus_stiffness2")
-                continue
-            c2, c5, mp = sp(self.c2, c0), sp(self.c5, c0), self.m.data_ptr()
-            if sg.kind == 0:
-                check(fn("fus_stiffness_westervelt_rect", self.dtype)(
-                    xp, c3, vp, c4, c2, c5, mp, bp, sp(self.Gc, c0), sp(self.detJc, c0), dm, None, sg.n, P, R, st),
-                    "fus_stiffness_westervelt_rect")
-            elif sg.kind == 1:
-                check(fn("fus_stiffness_westervelt_affine", self.dtype)(
-                    xp, c3, vp, c4, c2, c5, mp, bp, sp(self.Gc, c0), sp(self.detJc, c0),
-                    self._weights.data_ptr(), dm, None, sg.n, P, R, st), "fus_stiffness_westervelt_affine")
-            else:
-                check(fn("fus_stiffness_westervelt", self.dtype)(
-                    xp, c3, vp, c4, c2, c5, mp, bp, sp(self.G, sg.g0), sp(self.detJ, sg.g0), dm, None, sg.n,
-                    P, R, st), "fus_stiffness_westervelt")
+        self._cell_kernels(self.un if x is None else x, self.ku if vn is None else vn, wait)
 
-    def _close(self, stage, dt, count_step, base, acc, skip=None, n=None):
-        u, v, u0, v0, bdt, adt, mode = self._close_args(stage, dt, base, acc)
-        step = self.step_dev.data_ptr() if count_step else None
-        n = self.nupd if n is None else n
-        if not self._m_accum:
-            check(fn("fus_rk_close_westervelt_pw", self.dtype)(
-                u, v, u0, v0, self.ku.data_ptr(), None, self.un.data_ptr(), self.b.data_ptr(), self.m0.data_ptr(),
-                self.m2.data_ptr(), self.m5.data_ptr(), bdt, adt, mode, n, step, skip, current_stream()),
-                "fus_rk_close_westervelt_pw")
-            return
-        check(fn("fus_rk_close_westervelt", self.dtype)(
-            u, v, u0, v0, self.ku.data_ptr(), None, self.un.data_ptr(), self.b.data_ptr(), self.m.data_ptr(),
-            self.m0.data_ptr(), bdt, adt, mode, n, step, skip, current_stream()), "fus_rk_close_westervelt")
-
-    def _close_shared(self, stage, dt, base, acc):
-        u, v, u0, v0, bdt, adt, mode = self._close_args(stage, dt, base, acc)
-        pw = not self._m_accum
-        check(fn("fus_rk_close_shared", self.dtype)(
-            self.halo.handle, 2 if pw else 1, 1, 1, u, v, u0, v0, self.ku.data_ptr(), self.un.data_ptr(),
-            self.b.data_ptr(), None if pw else self.m.data_ptr(), self.m0.data_ptr(),
-            self.m2.data_ptr() if pw else None, self.m5.data_ptr() if pw else None, bdt, adt, mode,
-            current_stream()), "fus_rk_close_shared")
+    def _masses(self):
+        return (self.m, self.m0, None, None) if self._m_accum else (None, self.m0, self.m2, self.m5)
 
     def stage_bytes(self):
         s = self.dtype.itemsize

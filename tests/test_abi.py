@@ -28,6 +28,23 @@ def test_binding_table_matches_header():
     assert sorted(_lib.exported_symbols()) == _declared()
 
 
+def test_binding_table_arity_matches_header_prototypes():
+    """ctypes accepts EXTRA arguments silently when argtypes is set, so a table entry one short
+    would shift every later argument of a call without an error: every entry must have the
+    prototype's argument count, with "T" exactly at the by-value double / float parameters."""
+    src = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "fus_b200.h")).read(), flags=re.S)
+    protos = dict(re.findall(r"\b(fus_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", src))
+    checked = 0
+    for base, args in _lib._sigs().items():
+        for sfx in ("f64", "f32"):
+            params = [p.strip() for p in protos[f"{base}_{sfx}"].split(",")]
+            assert len(params) == len(args), (base, sfx, len(params), len(args))
+            by_value = [re.fullmatch(r"(const\s+)?(double|float)\s+\w+", p) is not None for p in params]
+            assert by_value == [a == "T" for a in args], (base, sfx)
+            checked += 1
+    assert checked == 2 * len(_lib._sigs()) > 80
+
+
 def test_error_reporting_without_gpu():
     lib = _lib.lib()
     # argument validation happens before any CUDA call
