@@ -412,15 +412,20 @@ int close_entry(T* u, T* v, T* u0, T* v0, T* ku, T* kv, T* un, T* b, T* m, const
   if (next_mode < 0 || next_mode > 4) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close: next_mode");
   if (next_mode == 0 && kv == nullptr)
     return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close: kv must be stored when not chained");
-  if (n == 0) return 0;
   if (WEST == 2 && (m0 == nullptr || m2 == nullptr || m5 == nullptr))
     return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close_westervelt_pw: null m0 / m2 / m5");
   if (WEST == 3 && (u == nullptr || v == nullptr || b == nullptr || m == nullptr))
     return fus_set_error(FUS_ERR_BAD_ARGUMENT, "leapfrog_close: null vector");
+  const bool counts_step = step != nullptr && (next_mode == 2 || next_mode == 4);
+  if (n == 0 && !counts_step) return 0;
   CloseArgs<T> a{u, v, u0, v0, ku, kv, un, b, m, m0, m2, m5, bdt, adt_next, next_mode, n,
                  reinterpret_cast<long long*>(step), skip};
   cudaStream_t st_ = static_cast<cudaStream_t>(stream);
-  if (aligned16({u, v, u0, v0, ku, kv, un, b, m, m0, m2, m5})) {
+  if (n == 0) {
+    // an empty range still ends the step (a rank whose owned dofs are all closed by
+    // fus_rk_close_shared_*): one block touches no dof and advances the counter
+    rk_close_kernel<T, false, WEST><<<1, kThreads, 0, st_>>>(a);
+  } else if (aligned16({u, v, u0, v0, ku, kv, un, b, m, m0, m2, m5})) {
     rk_close_kernel<T, true, WEST><<<grid_for(n / Vec<T>::W + 1), kThreads, 0, st_>>>(a);
   } else {
     rk_close_kernel<T, false, WEST><<<grid_for(n), kThreads, 0, st_>>>(a);

@@ -391,9 +391,9 @@ int fus_rk_open_f32(const float* u, const float* v, float* u0, float* v0, float*
  *                A step run as 3 / 1 / 1 / 4 makes 9 + 12 + 12 + 8 vector passes instead of
  *                the 4 x 12 of 1 / 1 / 1 / 2, with the same arithmetic bit for bit.
  * kv is stored when non-NULL; it may be NULL in modes 1-4 (nothing reads
- * it again).  step_dev (may be NULL) is a device step counter incremented in
- * modes 2 and 4 - it indexes the source table of fus_boundary_terms, so a whole RK
- * step can be replayed as a CUDA graph with no host work.
+ * it again).  step_dev (may be NULL) is a device step counter incremented once per
+ * call in modes 2 and 4, also when n == 0 - it indexes the source table of
+ * fus_boundary_terms, so a whole RK step can be replayed as a CUDA graph with no host work.
  * skip_mask (DEVICE, may be NULL): bit d%8 of byte d/8 set => dof d is left untouched here
  * (multi-GPU: the shared dofs, closed by fus_rk_close_shared_* after the reverse halo). */
 int fus_rk_close_f64(double* u, double* v, double* u0, double* v0, double* ku, double* kv,

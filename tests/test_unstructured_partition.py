@@ -358,10 +358,15 @@ def test_shared_last_numbering_properties(kind):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("kind,halo,tag", [("box", "p2p", "f64"), ("box", "nccl-shaped", "f64"), ("blob", "p2p", "f64"),
-                                           ("box", "p2p", "f32"), ("blob", "p2p", "f32")])
+                                           ("box", "p2p", "f32"), ("blob", "p2p", "f32"),
+                                           ("blob-empty-bulk", "p2p", "f32")])
 def test_linear_rk4_with_shared_last_numbering_vs_serial_oracle(kind, halo, tag):
     """The partitioned solve in the renumbered local ordering (what problem.box_setup hands the
-    solvers on > 1 rank) against the single-rank oracle, ranks emulated on one GPU."""
+    solvers on > 1 rank) against the single-rank oracle, ranks emulated on one GPU.
+
+    ``blob-empty-bulk``: one rank owns fewer unshared dofs than one close pack, so its bulk close
+    has n = 0, and it owns source facets.  Its step counter, which selects the source amplitude
+    row, must still advance once per step."""
     import torch
 
     if not torch.cuda.is_available():
@@ -373,7 +378,10 @@ def test_linear_rk4_with_shared_last_numbering_vs_serial_oracle(kind, halo, tag)
 
     dtt = np.float64 if tag == "f64" else np.float32  # f32: packs of 4, the tail starts on a multiple of 4
     P, N, L, R, nsteps = 3, (4, 4, 4), (0.012, 0.01, 0.011), 8, 8
-    serial = problems.linear_problem(P, N, L, dtt, perturb=0.1, seed=11)
+    src = (2,)
+    if kind == "blob-empty-bulk":
+        P, N, src = 2, (4, 4, 3), (0,)
+    serial = problems.linear_problem(P, N, L, dtt, perturb=0.1, seed=11, src_facets=src)
     dt = problems.cfl_dt(P, min(L[i] / N[i] for i in range(3)), serial.c0, serial.f0)
     m = np.zeros(serial.ndofs, dtt)
     orc.mass_operator(np.ones(serial.ndofs, dtt), serial.cell_coeff1, m, serial.detJ, serial.dofmap)
@@ -390,12 +398,20 @@ def test_linear_rk4_with_shared_last_numbering_vs_serial_oracle(kind, halo, tag)
                                   shuffle_seed=2, owner_rule="hash")
     ren = _renumbered(parts, utils.compute_scatterer_data_all([p.index_map for p in parts]))
     ndmax = max(q.index_map.size_local + q.index_map.num_ghosts for q in parts)
+    if kind == "blob-empty-bulk":
+        pack = 16 // np.dtype(dtt).itemsize
+        empty = []
+        for p, (_, _, _, gd, _) in zip(parts, ren):
+            ns = np.unique(np.concatenate([np.asarray(a) for a in gd[0]])).size if sum(len(a) for a in gd[0]) else 0
+            if ns and (p.index_map.size_local - ns) // pack == 0 and S.boundary_facets(p.mesh, src[0]).shape[0]:
+                empty.append(p.rank)
+        assert empty, "no rank with an empty bulk close that owns source facets"
 
     def body(r, transport):
         p = parts[r]
         dm, _, od, gd, _ = ren[r]
         nl, ng = p.index_map.size_local, p.index_map.num_ghosts
-        d = problems.linear_problem(P, None, None, dtt, mesh=p.mesh, dofmap=dm, ndofs=nl + ng)
+        d = problems.linear_problem(P, None, None, dtt, mesh=p.mesh, dofmap=dm, ndofs=nl + ng, src_facets=src)
         if halo == "p2p":
             fab = local_fabric(transport.cluster, r, P2PHaloExchange.arena_bytes(ndmax, dtt))
             h = P2PHaloExchange(fab, od, gd, nl, ng, dtt)
