@@ -31,8 +31,10 @@ def parser(desc, degree, cells):
     ap.add_argument("--cells", type=int, default=cells, help="cells per direction PER GPU (default: the reference demo's mesh)")
     ap.add_argument("--steps", type=int, default=0, help="number of steps (default: run to the demo's final time)")
     ap.add_argument("--dtype", default="f64", choices=["f64", "f32"])
-    ap.add_argument("--geometry", default="stream", choices=["stream", "auto"],
-                    help="auto: affine cells keep 6 geometric factors instead of 6 n^3 (same results to rounding)")
+    ap.add_argument("--geometry", default="stream", choices=["stream", "auto", "vertex"],
+                    help="auto: affine cells keep 6 geometric factors instead of 6 n^3; vertex: as auto, and the "
+                         "other cells rebuild their geometry from 36 values instead of streaming it (no per-point "
+                         "tables; same results to rounding)")
     ap.add_argument("--integrator", default="rk4", choices=["rk4", "leapfrog"],
                     help="time integrator of the linear demos: rk4 (the reference's) or leapfrog")
     ap.add_argument("--sample-dir", default=None,

@@ -18,7 +18,7 @@ def main():
     grid = S.block_grid(world)
     ncells = tuple(a.cells * g for g in grid)
     lengths = tuple(h * n for n in ncells)
-    su = problem.box_setup(a.degree, ncells, lengths, dtype, rank, world, grid=grid)
+    su = problem.box_setup(a.degree, ncells, lengths, dtype, rank, world, grid=grid, geometry=a.geometry)
     solver = problem.linear_solver(su, source_facets=[2], absorbing_facets=[3], rho=rho, c0=c0, f0=f0, p0=p0,
                                    geometry=a.geometry, integrator=a.integrator)
     dt = problem.cfl_time_step(a.degree, h, c0, f0, 0.65)  # :116-120

@@ -20,7 +20,7 @@ def main():
     grid = S.block_grid(world)
     ncells = tuple(a.cells * g for g in grid)
     lengths = tuple(h * n for n in ncells)
-    su = problem.box_setup(a.degree, ncells, lengths, dtype, rank, world, grid=grid)
+    su = problem.box_setup(a.degree, ncells, lengths, dtype, rank, world, grid=grid, geometry=a.geometry)
     centre = (0.5 * lengths[0], 0.5 * lengths[1])
     piston = problem.disc(0, 1, centre, 0.01)
     solver = problem.linear_solver(

@@ -22,7 +22,7 @@ def main():
     grid = S.block_grid(world)
     ncells = tuple(a.cells * g for g in grid)
     lengths = tuple(h * n for n in ncells)
-    su = problem.box_setup(a.degree, ncells, lengths, dtype, rank, world, grid=grid)
+    su = problem.box_setup(a.degree, ncells, lengths, dtype, rank, world, grid=grid, geometry=a.geometry)
     centre = (0.5 * lengths[1], 0.5 * lengths[2])
     solver = problem.westervelt_solver(
         su, source_facets=[2], absorbing_facets=[0, 1, 2, 3, 4, 5], rho=rho, c0=c0, f0=f0, p0=p0, beta=3.5,

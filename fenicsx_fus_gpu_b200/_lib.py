@@ -44,6 +44,8 @@ def _sigs():
         "fus_set_vertex_tables": [I, P, P, P],
         "fus_stiffness_vertex": [P, P, P, P, P, P, L, I, I, P],
         "fus_stiffness2_vertex": [P, P, P, P, P, P, P, P, L, I, I, P],
+        "fus_stiffness_westervelt_vertex": [P, P, P, P, P, P, P, P, P, P, P, L, I, I, P],
+        "fus_mass_vertex": [P, P, P, P, P, L, I, P],
         "fus_rk_close_westervelt_pw": [P, P, P, P, P, P, P, P, P, P, P, T, T, I, L, P, P, P],
         "fus_compress_geometry": [P, P, P, P, P, P, L, I, T, P],
         "fus_mass": [P, P, P, P, P, L, I, P],

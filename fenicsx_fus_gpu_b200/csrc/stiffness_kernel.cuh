@@ -181,6 +181,8 @@ __device__ __forceinline__ G6<float> load_g6(const float* p) {
 //   adj J), det = t_0 . c_0, one division, and the product
 //       f_a = (w / |det|) c_a . (g_0 c_0 + g_1 c_1 + g_2 c_2)         ( = sum_b G_ab g_b )
 //   without ever forming G: ~60 flops per point against 6 streamed values.
+//   MODE 2 takes w |det| of the same point for the cell-mass pair: cm xa and cy xb^2 are kept per
+//   point from the gather until the transform loop, where m and the x-pencil sum receive them.
 template <typename T, int n, int MODE, bool ATOMIC, int GEO, bool WAIT>
 __global__ void __launch_bounds__(Cfg<T, n>::THREADS, Cfg<T, n>::MINB)
     stiffness_kernel(const StiffArgs<T> a) {
@@ -188,7 +190,6 @@ __global__ void __launch_bounds__(Cfg<T, n>::THREADS, Cfg<T, n>::MINB)
   constexpr bool AFF = GEO == 1 || GEO == 2;
   constexpr bool NOSTREAM = GEO >= 1;  // no G ring (AFF or TRI)
   constexpr bool RECT = GEO == 2;
-  static_assert(!(TRI && MODE == 2), "trilinear mode: stiffness (MODE 0 / 1) only");
   constexpr bool DUAL = MODE >= 1;
   constexpr bool WEST = MODE == 2;
   using L = Layout<T, n>;
@@ -348,9 +349,11 @@ __global__ void __launch_bounds__(Cfg<T, n>::THREADS, Cfg<T, n>::MINB)
   (void)xw;
   (void)xwn;
   T dj[WEST ? n : 1], djn[WEST ? n : 1], bex[WEST ? n : 1];  // Westervelt: detJ pencil, extra b term
+  T mx[WEST && TRI ? n : 1];  // Westervelt, trilinear: cm xa until w |det| is known
   (void)dj;
   (void)djn;
   (void)bex;
+  (void)mx;
 
   // Rectilinear mode uses the per-cell scalars right at the top of a batch (the other modes
   // first need them two barriers later), so they ride the register pipeline one batch ahead:
@@ -493,14 +496,19 @@ __global__ void __launch_bounds__(Cfg<T, n>::THREADS, Cfg<T, n>::MINB)
           const T cy = RECT ? csc[NCS > 6 ? 6 : 0] : a.cy[cell0 + cs];
 #pragma unroll
           for (int i = 0; i < n; ++i) {
-            T dji;
-            if constexpr (AFF) {
-              dji = wreg[i] * djc;
+            if constexpr (TRI) {
+              mx[i] = xv[i] * cm;                // times w |det| in the transform loop
+              bex[i] = (xw[i] * xw[i]) * cy;
             } else {
-              dji = dj[i];
+              T dji;
+              if constexpr (AFF) {
+                dji = wreg[i] * djc;
+              } else {
+                dji = dj[i];
+              }
+              atomicAdd(a.m + dof[i], xv[i] * dji * cm);   // m += cm detJ un
+              bex[i] = (xw[i] * xw[i]) * dji * cy;          // b += cy detJ vn^2 (joins the scatter)
             }
-            atomicAdd(a.m + dof[i], xv[i] * dji * cm);   // m += cm detJ un
-            bex[i] = (xw[i] * xw[i]) * dji * cy;          // b += cy detJ vn^2 (joins the scatter)
           }
         }
 #pragma unroll
@@ -606,7 +614,7 @@ __global__ void __launch_bounds__(Cfg<T, n>::THREADS, Cfg<T, n>::MINB)
       const T* Gc = Gs + cs * (L::GC / L::S) + t2 * 6;
 #pragma unroll
       for (int l = 0; l < n; ++l) {
-        if constexpr (WEST) {
+        if constexpr (WEST && !TRI) {
           ry[l] = bex[l];
         } else {
           ry[l] = T(0);
@@ -659,6 +667,11 @@ __global__ void __launch_bounds__(Cfg<T, n>::THREADS, Cfg<T, n>::MINB)
           f0 = sc * (c00 * v0 + c01 * v1 + c02 * v2);
           f1 = sc * (c10 * v0 + c11 * v1 + c12 * v2);
           f2 = sc * (c20 * v0 + c21 * v1 + c22 * v2);
+          if constexpr (WEST) {
+            const T wdet = (wab * KT::w(i)) * fabs(det);  // detJ of the streamed form at this point
+            atomicAdd(a.m + dof[i], mx[i] * wdet);        // m += cm detJ un
+            ry[i] += bex[i] * wdet;                       // b += cy detJ vn^2
+          }
         } else {
           G6<T> g;
           T sc;

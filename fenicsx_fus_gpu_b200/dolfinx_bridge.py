@@ -28,10 +28,9 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from . import precompute as pre
 from . import substrate as S
 from . import utils
-from .problem import Setup, _d
+from .problem import Setup, _cell_geometry, _d
 
 
 @dataclass
@@ -81,14 +80,14 @@ def basix_tables(P: int, float_type, order: str = "basix"):
 
 
 def setup_from_dolfinx(mesh, V, basis_degree, float_type=np.float64, comm=None, halo_kind="nccl",
-                       tables=None, perm=None, max_halo_vecs=3, renumber_shared=True) -> Setup:
+                       tables=None, perm=None, max_halo_vecs=3, renumber_shared=True, geometry="stream") -> Setup:
     """``Setup`` of this rank from a DOLFINx ``mesh`` and function space ``V``
     (cuda/demo_linear_box.py:99-113, 175-207, 232-253).
 
     ``tables`` / ``perm`` override the Basix look-ups (``perm`` reorders ``V.dofmap.list``
     columns into tensor-product order; identity when the space was created on the
-    tensor-product element).  ``comm``: torch.distributed group for the halo."""
-    import torch
+    tensor-product element).  ``comm``: torch.distributed group for the halo.  ``geometry``: as for
+    ``problem.box_setup`` ("vertex": ``dev["Tc"]`` instead of the ``G`` / ``detJ`` tables)."""
     import torch.distributed as dist
 
     float_type = np.dtype(float_type)
@@ -123,13 +122,9 @@ def setup_from_dolfinx(mesh, V, basis_degree, float_type=np.float64, comm=None, 
             from .scatterer import HaloExchange
 
             halo = HaloExchange(comm, od, gd, nlocal, float_type, max_vecs=max_halo_vecs)
-    tdt = torch.float64 if float_type == np.float64 else torch.float32
-    nd3 = tables.n**3
     dev = dict(dofmap=_d(dofmap), x_dofs=_d(x_dofs), x_g=_d(x_g), dphi=_d(tables.dphi), wts=_d(tables.wts),
                dphi_f=_d(tables.dphi_f), wts_f=_d(tables.wts_f))
-    dev["G"] = torch.empty((num_cells, nd3, 6), dtype=tdt, device="cuda")
-    dev["detJ"] = torch.empty((num_cells, nd3), dtype=tdt, device="cuda")
-    pre.compute_geometry(dev["G"], dev["detJ"], (dev["x_dofs"], dev["x_g"]), num_cells, dev["dphi"], dev["wts"])
+    _cell_geometry(dev, num_cells, tables, geometry)
     # smallest cell diameter of this rank (cpp.mesh.h, cuda/demo_linear_box.py:103-108): longest vertex distance
     cc = x_g[x_dofs].astype(np.float64)
     h = float(np.sqrt(((cc[:, :, None, :] - cc[:, None, :, :]) ** 2).sum(-1)).max(axis=(1, 2)).min()) if num_cells else np.inf

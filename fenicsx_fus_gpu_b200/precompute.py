@@ -158,6 +158,37 @@ def compress_geometry(G, detJ, weights, tol=None):
     return affine, Gc, detJc
 
 
+def compress_trilinear(Tc, tol=None):
+    """Affine-cell detection and compression from the trilinear coefficients alone (the
+    ``compress_geometry`` of a solver that holds no ``G`` table).
+
+    ``Tc`` (Nc, 36) as ``trilinear_coefficients`` returns it: per cell and reference direction
+    ``d`` the tangent ``t_d = Tc[d,0] + u Tc[d,1] + v Tc[d,2] + u v Tc[d,3]``.  A cell is affine
+    when every non-constant coefficient vector ``Tc[d, 1..3]`` lies within ``tol`` (relative to
+    the largest constant tangent ``Tc[d, 0]`` of the cell; default 2048 machine epsilons, as for
+    ``compress_geometry``) of zero.  Returns ``(affine, Gc, detJc)`` as device tensors in the
+    type of ``Tc``: ``affine`` (Nc,) int32, ``Gc = |det J| (J^T J)^-1`` (Nc, 6) in the order
+    ``[G00 G01 G02 G11 G12 G22]`` and ``detJc = |det J|`` (Nc,), J the constant tangents.  The
+    tables of an affine cell factor as ``G = w_q Gc``, ``detJ = w_q detJc`` for any quadrature
+    rule, so no weights are needed.  Set-up only: plain torch in float64, on the device of ``Tc``
+    (a CUDA tensor, a CPU tensor or numpy)."""
+    import torch
+
+    Tc = torch.as_tensor(Tc)
+    if tol is None:
+        tol = 2048.0 * float(torch.finfo(Tc.dtype).eps)
+    t = Tc.to(torch.float64).reshape(-1, 3, 4, 3)
+    t0, t1, t2 = t[:, 0, 0], t[:, 1, 0], t[:, 2, 0]
+    scale = t[:, :, 0].abs().amax(dim=(1, 2))
+    affine = (t[:, :, 1:].abs().amax(dim=(1, 2, 3)) <= tol * scale).to(torch.int32)
+    # rows of adj J (as the GEO = 3 kernel forms them): G = (1/|det|) c_a . c_b
+    c = torch.stack([torch.linalg.cross(t1, t2), torch.linalg.cross(t2, t0), torch.linalg.cross(t0, t1)], dim=1)
+    det = (t0 * c[:, 0]).sum(-1).abs()
+    ia, ib = [0, 0, 0, 1, 1, 2], [0, 1, 2, 1, 2, 2]
+    Gc = (c[:, ia] * c[:, ib]).sum(-1) / det[:, None]
+    return affine, Gc.to(Tc.dtype).contiguous(), det.to(Tc.dtype).contiguous()
+
+
 def trilinear_expansion(dphi, points):
     """``M`` (3, 4, 8) float64 with ``dphi[d, q, :] = sum_m {1, u, v, u v}_m(points[q]) M[d, m, :]``,
     ``(u, v)`` the two reference coordinates other than ``d``: the bilinear expansion of the

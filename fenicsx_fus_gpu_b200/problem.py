@@ -45,7 +45,7 @@ class Setup:
     global_dofs: int
     global_cells: tuple
     halo: object | None
-    dev: dict = field(default_factory=dict)  # device tensors: dofmap, G, detJ, x_dofs, x_g, tables
+    dev: dict = field(default_factory=dict)  # device tensors: dofmap, G and detJ (or Tc), x_dofs, x_g, tables
     h: float = 0.0
     local_to_serial: np.ndarray | None = None  # (ndofs,) index of every local dof in the unpartitioned box
     # multi-rank set-ups renumber the owned dofs so that the shared ones are contiguous
@@ -61,7 +61,7 @@ def _d(a):
 
 def box_setup(P, ncells, lengths, dtype=np.float64, rank=0, world=1, comm=None, grid=None,
               perturb=0.0, seed=0, order="basix", max_halo_vecs=3, scatter_data=None,
-              halo_kind="nccl", fabric=None, partition="block", renumber_shared=True) -> Setup:
+              halo_kind="nccl", fabric=None, partition="block", renumber_shared=True, geometry="stream") -> Setup:
     """Mesh part, dofmap, halo and device geometry of rank ``rank`` of ``world``.
 
     ``comm``: torch.distributed group / transport for the halo (None = world
@@ -70,11 +70,11 @@ def box_setup(P, ncells, lengths, dtype=np.float64, rank=0, world=1, comm=None, 
     irregular connected parts, shuffled cell / dof / ghost order, pseudo-random ownership of
     the shared dofs), which exercises the generic index-map -> halo path the way a graph
     partitioner's output would.  ``renumber_shared``: move the owned dofs that neighbours ghost
-    to the end of the owned block (``utils.shared_last_numbering``; ``Setup.local_perm``)."""
-    import torch
-
+    to the end of the owned block (``utils.shared_last_numbering``; ``Setup.local_perm``).
+    ``geometry``: the solvers' geometry mode this set-up serves; with ``"vertex"`` the (Nc, n^3)
+    tables ``G`` and ``detJ`` are not built, ``dev["Tc"]`` holds the 36 trilinear coefficients
+    per cell instead."""
     dtype = np.dtype(dtype)
-    tdt = torch.float64 if dtype == np.float64 else torch.float32
     if np.isscalar(ncells):
         ncells = (int(ncells),) * 3
     if np.isscalar(lengths):
@@ -119,16 +119,43 @@ def box_setup(P, ncells, lengths, dtype=np.float64, rank=0, world=1, comm=None, 
         else:
             halo = HaloExchange(comm, od, gd, nlocal, dtype, max_vecs=max_halo_vecs)
     nc = mesh.num_cells
-    nd3 = tb.n**3
     dev = dict(dofmap=_d(dofmap), x_dofs=_d(mesh.x_dofs), x_g=_d(mesh.x_g), dphi=_d(tb.dphi), wts=_d(tb.wts),
                dphi_f=_d(tb.dphi_f), wts_f=_d(tb.wts_f))
+    _cell_geometry(dev, nc, tb, geometry)
+    h = min(lengths[i] / ncells[i] for i in range(3))
+    return Setup(P, dtype, rank, world, mesh, tb, dofmap, ndofs, nlocal, S.num_dofs(ncells, P),
+                 tuple(ncells), halo, dev, h, l2s, lperm)
+
+
+def _cell_geometry(dev, nc, tb, geometry):
+    """The per-cell geometry the solvers read: G and detJ tables, or Tc alone for geometry='vertex'."""
+    import torch
+
+    if geometry not in ("stream", "auto", "vertex"):
+        raise ValueError("geometry must be 'stream', 'auto' or 'vertex'")
+    if geometry == "vertex":
+        dev["Tc"] = pre.trilinear_coefficients((dev["x_dofs"], dev["x_g"]), nc, tb.dphi, tb.pts)
+        return
+    tdt = dev["x_g"].dtype
+    nd3 = tb.n**3
     dev["G"] = torch.empty((nc, nd3, 6), dtype=tdt, device="cuda")
     dev["detJ"] = torch.empty((nc, nd3), dtype=tdt, device="cuda")
     # one pass for both tables (the reference makes two: cuda/demo_linear_box.py:245-253)
     pre.compute_geometry(dev["G"], dev["detJ"], (dev["x_dofs"], dev["x_g"]), nc, dev["dphi"], dev["wts"])
-    h = min(lengths[i] / ncells[i] for i in range(3))
-    return Setup(P, dtype, rank, world, mesh, tb, dofmap, ndofs, nlocal, S.num_dofs(ncells, P),
-                 tuple(ncells), halo, dev, h, l2s, lperm)
+
+
+def _geometry_kw(su: Setup, kw):
+    """Solver keywords of the geometry mode: the quadrature weights, and for 'vertex' the trilinear
+    coefficients (computed here when the set-up was built for another mode)."""
+    geometry = kw.get("geometry", "stream")
+    if geometry != "stream":
+        kw.setdefault("weights", su.tables.wts)
+    if geometry == "vertex":
+        if "Tc" not in su.dev:
+            su.dev["Tc"] = pre.trilinear_coefficients((su.dev["x_dofs"], su.dev["x_g"]), su.mesh.num_cells,
+                                                      su.tables.dphi, su.tables.pts)
+        kw.setdefault("trilinear", (su.dev["Tc"], su.tables.pts_1d, su.tables.wts_1d))
+    return kw
 
 
 def facet_group(su: Setup, local_facets, predicate=None):
@@ -178,12 +205,11 @@ def linear_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0=150
         raise ValueError("integrator must be 'rk4' or 'leapfrog'")
     cls = LinearLeapfrog3D if integrator == "leapfrog" else LinearSpectral3D
     nc = su.mesh.num_cells
-    if kw.get("geometry") == "auto":
-        kw.setdefault("weights", su.tables.wts)
+    _geometry_kw(su, kw)
     fd1, dJ1, bd1 = facet_group(su, source_facets, source_predicate)
     fd2, dJ2, bd2 = facet_group(su, absorbing_facets, absorbing_predicate)
     return cls(
-        su.P, su.dtype, su.ndofs, su.dev["dofmap"], su.dev["G"], su.dev["detJ"], su.tables.dphi_1D,
+        su.P, su.dtype, su.ndofs, su.dev["dofmap"], su.dev.get("G"), su.dev.get("detJ"), su.tables.dphi_1D,
         _full(su, nc, 1.0 / rho / c0 / c0), _full(su, nc, -1.0 / rho),
         fd1, dJ1, _full(su, bd1.shape[0], 1.0 / rho), fd2, dJ2, _full(su, bd2.shape[0], -1.0 / rho / c0),
         halo=su.halo, source=lambda t: linear_source(t, f0, p0, c0), **kw)
@@ -197,13 +223,12 @@ def westervelt_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0
         p0 = rho * c0 * 0.38557513826589934  # source velocity of the bowl demo (:66-67)
     delta = utils.compute_diffusivity_of_sound(2.0 * np.pi * f0, c0, alpha_dB)
     nc = su.mesh.num_cells
-    if kw.get("geometry") == "auto":
-        kw.setdefault("weights", su.tables.wts)
+    _geometry_kw(su, kw)
     fd1, dJ1, bd1 = facet_group(su, source_facets, source_predicate)
     fd2, dJ2, bd2 = facet_group(su, absorbing_facets, absorbing_predicate)
     n1, n2 = bd1.shape[0], bd2.shape[0]
     return WesterveltSpectral3D(
-        su.P, su.dtype, su.ndofs, su.dev["dofmap"], su.dev["G"], su.dev["detJ"], su.tables.dphi_1D,
+        su.P, su.dtype, su.ndofs, su.dev["dofmap"], su.dev.get("G"), su.dev.get("detJ"), su.tables.dphi_1D,
         _full(su, nc, 1.0 / rho / c0 / c0), _full(su, nc, -2.0 * beta / rho / rho / c0**4),
         _full(su, nc, -1.0 / rho), _full(su, nc, -delta / rho / c0 / c0),
         _full(su, nc, 2.0 * beta / rho / rho / c0**4),

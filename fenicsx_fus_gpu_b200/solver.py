@@ -59,11 +59,12 @@ from . import _lib
 from ._lib import FUS_TABLES_RESIDENT, check, current_stream, fn
 
 # a contiguous range of (permuted) cells that one kernel launch covers:
-# kind 0 rectilinear, 1 affine, 2 streamed G; c0/n cell range; g0 first row of the streamed G / detJ
-# arrays; ninterior: the first ninterior cells of the range touch no ghost dof (peer-memory halo: the
-# launch waits for the forward exchange only before its remaining, interface, cells)
+# kind 0 rectilinear, 1 affine, 2 streamed G, 3 trilinear (geometry rebuilt from Tc); c0/n cell range;
+# g0 first row of the streamed G / detJ arrays (kind 3: of Tc); ninterior: the first ninterior cells
+# of the range touch no ghost dof (peer-memory halo: the launch waits for the forward exchange only
+# before its remaining, interface, cells)
 Seg = namedtuple("Seg", "kind c0 n g0 ninterior")
-KIND_SUFFIX = ("_rect", "_affine", "")  # cell-kernel symbol fus_<form><suffix> per Seg.kind
+KIND_SUFFIX = ("_rect", "_affine", "", "_vertex")  # cell-kernel symbol fus_<form><suffix> per Seg.kind
 
 A_RUNGE = (0.0, 0.5, 0.5, 1.0)
 B_RUNGE = (1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0)
@@ -130,7 +131,7 @@ class _RK4:
 
     def __init__(self, P, float_type, ndofs, dofmap, G, dphi_1D, halo=None, source=None,
                  source_at_stage_time=True, use_graph=True, geometry="stream", weights=None,
-                 split_cells=True):
+                 split_cells=True, trilinear=None):
         torch = _torch()
         if not torch.cuda.is_available():
             raise _lib.FusError("no CUDA device: this package has no CPU path")
@@ -141,7 +142,28 @@ class _RK4:
         self.ndofs = int(ndofs)
         self.dofmap = _dev(dofmap, torch.int32)
         self.ncells = int(self.dofmap.shape[0])
-        self.G = _dev(G, self.T)
+        # geometry = "stream": G (and detJ) are read in full every stage, as the reference does;
+        # "auto": cells whose Jacobian is constant (precompute.compress_geometry) keep 6 (+1)
+        # values instead of 6 (+1) n^3 and go through the affine kernels, the others are streamed;
+        # "vertex": the same split from the trilinear coefficients alone (precompute.compress_trilinear),
+        # the other cells rebuild their geometry in the kernel from 36 values each
+        # (``trilinear = (Tc, points_1d, weights_1d)``): no (Nc, n^3) table is ever held
+        if geometry not in ("stream", "auto", "vertex"):
+            raise ValueError("geometry must be 'stream', 'auto' or 'vertex'")
+        if geometry != "stream" and weights is None:
+            raise ValueError(f"geometry='{geometry}' needs the quadrature weights (n^3,)")
+        if geometry == "vertex" and trilinear is None:
+            raise ValueError("geometry='vertex' needs trilinear=(Tc, points_1d, weights_1d)")
+        if geometry != "vertex" and G is None:
+            raise ValueError(f"geometry='{geometry}' needs G")
+        self.G = _dev(G, self.T) if geometry != "vertex" else None
+        self._Tc = self._vertex_tables = None
+        if geometry == "vertex":
+            Tc, x1, w1 = trilinear
+            self._Tc = _dev(Tc, self.T)
+            host = lambda a: np.ascontiguousarray(a.cpu().numpy() if isinstance(a, torch.Tensor) else a,  # noqa: E731
+                                                  dtype=self.dtype)
+            self._vertex_tables = (host(x1), host(w1))
         self.halo = halo
         self.source = source
         self.source_at_stage_time = bool(source_at_stage_time)
@@ -191,22 +213,16 @@ class _RK4:
         self._bdofs = None
         self._src = self._src2 = self._absb = None
         self.probe = None  # list: (start, stop) CUDA events around every stage-kernel launch (eager mode)
-        # geometry = "stream": G (and detJ) are read in full every stage, as the reference does;
-        # "auto": cells whose Jacobian is constant (precompute.compress_geometry) keep 6 (+1)
-        # values instead of 6 (+1) n^3 and go through the affine kernels, the others are streamed
-        if geometry not in ("stream", "auto"):
-            raise ValueError("geometry must be 'stream' or 'auto'")
-        if geometry == "auto" and weights is None:
-            raise ValueError("geometry='auto' needs the quadrature weights (n^3,)")
         self.geometry = geometry
         self._weights = None if weights is None else _dev(weights, self.T)
         self.nrect = 0  # number of rectilinear cells (affine, diagonal Gc)
         self.naff = 0  # number of affine cells (rectilinear ones included)
+        self.ntri = 0  # number of trilinear cells (geometry="vertex": the cells that are not affine)
         self.detJ = self.Gc = self.detJc = None
         self._rect_tables = None
         self.cell_perm = None
         # cell ranges, one launch each (per geometry kind; interior cells first inside a range)
-        self._segs = [Seg(2, 0, self.ncells, 0, self.ncells)]
+        self._segs = [Seg(3 if geometry == "vertex" else 2, 0, self.ncells, 0, self.ncells)]
         self.ninterface = 0
 
     # the solution between steps (device tensors; write initial data into them before rk4)
@@ -226,6 +242,10 @@ class _RK4:
             k1, w1 = self._rect_tables
             check(fn("fus_set_rect_tables", self.dtype)(self.P, k1.ctypes.data, w1.ctypes.data, current_stream()),
                   "fus_set_rect_tables")
+        if self._vertex_tables is not None:
+            x1, w1 = self._vertex_tables
+            check(fn("fus_set_vertex_tables", self.dtype)(self.P, x1.ctypes.data, w1.ctypes.data, current_stream()),
+                  "fus_set_vertex_tables")
 
     def _tensor_weights(self):
         """1-D weights w1 with weights[i n^2 + j n + k] = w1[i] w1[j] w1[k], or None when the rule
@@ -246,6 +266,16 @@ class _RK4:
             check(fn("fus_mass", self.dtype)(x.data_ptr(), coeff.data_ptr(), y.data_ptr(), detJ.data_ptr(),
                                              dofmap.data_ptr(), dofmap.shape[0], dofmap.shape[1],
                                              current_stream()), "fus_mass")
+
+    def _cell_mass(self, x, coeff, y, detJ):
+        """Lumped cell mass y += M(coeff; x): from the detJ table, or in vertex mode from Tc."""
+        if self._Tc is None:
+            self._mass(x, coeff, y, detJ, self.dofmap)
+        elif self.ncells:
+            self._set_tables()
+            check(fn("fus_mass_vertex", self.dtype)(x.data_ptr(), coeff.data_ptr(), y.data_ptr(), self._Tc.data_ptr(),
+                                                    self.dofmap.data_ptr(), self.ncells, self.P, current_stream()),
+                  "fus_mass_vertex")
 
     def _facets(self, bfacet_dofmap, detJ_f, facet_coeff):
         """(bfacet_dofmap, detJ_f, facet_coeff) of a boundary facet group on the device, or None
@@ -275,30 +305,36 @@ class _RK4:
     def _setup_geometry(self, detJ, cell_arrays):
         """Order the cells for the launches of a stage and build the launch ranges.
 
-        geometry='auto' classifies the cells (rectilinear / affine / streamed G); the peer-memory
-        halo splits them into interior and interface cells (those with a ghost dof).  Cells are
-        sorted by (interface, kind), every per-cell array follows (``cell_arrays``: attribute
-        names of (Nc,) / (Nc, n^3) tensors; the dofmap, G and detJ are handled here), G / detJ
-        are kept for the streamed cells only.  Summation order inside the atomics aside, a cell
-        permutation does not change the result."""
+        geometry='auto' classifies the cells (rectilinear / affine / streamed G), geometry='vertex'
+        the same way from Tc (rectilinear / affine / trilinear); the peer-memory halo splits them
+        into interior and interface cells (those with a ghost dof).  Cells are sorted by
+        (interface, kind), every per-cell array follows (``cell_arrays``: attribute names of (Nc,) /
+        (Nc, n^3) tensors; the dofmap, G, detJ and Tc are handled here), G / detJ are kept for the
+        streamed cells only, Tc for the trilinear ones.  Summation order inside the atomics aside, a
+        cell permutation does not change the result."""
         torch = _torch()
         nc = self.ncells
         if nc == 0:
             return
-        kind = torch.full((nc,), 2, dtype=torch.int32, device="cuda")
+        other = 3 if self.geometry == "vertex" else 2  # the kind of a cell that is not affine
+        kind = torch.full((nc,), other, dtype=torch.int32, device="cuda")
         Gc = detJc = None
-        if self.geometry == "auto":
+        if self.geometry != "stream":
             from . import precompute as pre
 
-            affine, Gc, detJc = pre.compress_geometry(self.G, detJ, self._weights)
+            if self.geometry == "vertex":
+                affine, Gc, detJc = pre.compress_trilinear(self._Tc)
+            else:
+                affine, Gc, detJc = pre.compress_geometry(self.G, detJ, self._weights)
             # rectilinear = affine with a diagonal Gc (off-diagonal factors at rounding-noise level)
             w1 = self._tensor_weights()
             tol = 2048.0 * float(np.finfo(self.dtype).eps)
             diag = Gc[:, [0, 3, 5]].abs().amax(dim=1)
             off = Gc[:, [1, 2, 4]].abs().amax(dim=1)
             rect = (affine > 0) & (off <= tol * diag) if w1 is not None else torch.zeros_like(affine, dtype=torch.bool)
-            kind = torch.where(rect, 0, torch.where(affine > 0, 1, 2)).to(torch.int32)
+            kind = torch.where(rect, 0, torch.where(affine > 0, 1, other)).to(torch.int32)
             self.naff = int((kind < 2).sum().item())
+            self.ntri = int((kind == 3).sum().item())
             self.nrect = int((kind == 0).sum().item())
             if self.nrect:
                 D = self._dphi_host.astype(np.float64)
@@ -310,8 +346,8 @@ class _RK4:
             self.ninterface = int(iface.sum().item())
         else:
             iface = torch.zeros(nc, dtype=torch.bool, device="cuda")
-        key = kind * 2 + iface.to(torch.int32)  # rect [interior | interface], affine [..], streamed [..]
-        counts = torch.bincount(key, minlength=6).cpu().tolist()
+        key = kind * 2 + iface.to(torch.int32)  # rect [interior | interface], affine [..], streamed / trilinear [..]
+        counts = torch.bincount(key, minlength=8).cpu().tolist()
         perm = None
         if not bool((key[1:] >= key[:-1]).all().item()):
             perm = torch.argsort(key, stable=True)  # original order kept inside every range
@@ -322,23 +358,27 @@ class _RK4:
             if Gc is not None:
                 Gc, detJc = Gc[perm], detJc[perm]
         if perm is not None or self.naff:
-            # G / detJ rows of the streamed cells only, in launch order (the caller's tensors are not touched)
+            # G / detJ (Tc) rows of the streamed (trilinear) cells only, in launch order (the caller's
+            # tensors are not touched)
             rows = torch.arange(nc, device="cuda") if perm is None else perm
-            rows = rows[kind[rows] == 2]
-            self.G = self.G[rows].contiguous() if rows.numel() else None
+            rows = rows[kind[rows] == other]
+            if self._Tc is not None:
+                self._Tc = self._Tc[rows].contiguous() if rows.numel() else None
+            else:
+                self.G = self.G[rows].contiguous() if rows.numel() else None
             if detJ is not None:
                 self.detJ = detJ[rows].contiguous() if rows.numel() else None
         if self.naff:
             self.Gc = Gc.contiguous()
-            self.detJc = detJc.contiguous() if detJ is not None else None
+            self.detJc = detJc.contiguous() if self._m_accum else None
         # launch ranges: one per geometry kind
         self._segs, c0, g0 = [], 0, 0
-        for k in (0, 1, 2):
+        for k in (0, 1, 2, 3):
             nint, nif = counts[2 * k], counts[2 * k + 1]
             if nint + nif:
                 self._segs.append(Seg(k, c0, nint + nif, g0, nint if split else nint + nif))
             c0 += nint + nif
-            if k == 2:
+            if k >= 2:
                 g0 += nint + nif
 
     # ---- stage pieces --------------------------------------------------------
@@ -401,7 +441,7 @@ class _RK4:
                 out.append((sg, 0))
             elif self.split_mode == "two" and 0 < sg.ninterior < sg.n:
                 out.append((Seg(sg.kind, sg.c0, sg.ninterior, sg.g0, sg.ninterior), None))
-                g1 = sg.g0 + (sg.ninterior if sg.kind == 2 else 0)
+                g1 = sg.g0 + (sg.ninterior if sg.kind >= 2 else 0)
                 out.append((Seg(sg.kind, sg.c0 + sg.ninterior, sg.n - sg.ninterior, g1, 0), 0))
             else:
                 out.append((sg, sg.ninterior if sg.ninterior < sg.n else None))
@@ -414,11 +454,15 @@ class _RK4:
     def _cell_kernels(self, x, vn, wait=False):
         """The cell-kernel launches of a stage: ``fus_<form><KIND_SUFFIX>`` over every cell range, with
         the form's operands, then the range's geometry (G or Gc; detJ or detJc when the form carries
-        the cell-mass pair; the quadrature weights for affine cells), then the common tail."""
+        the cell-mass pair; the quadrature weights for affine cells; Tc alone for trilinear cells),
+        then the common tail."""
         st, sp = current_stream(), self._sptr
         for sg, first in self._launches(wait):
-            G, dJ, row = (self.G, self.detJ, sg.g0) if sg.kind == 2 else (self.Gc, self.detJc, sg.c0)
-            geo = (sp(G, row), sp(dJ, row)) if self._m_accum else (sp(G, row),)
+            if sg.kind == 3:
+                geo = (sp(self._Tc, sg.g0),)
+            else:
+                G, dJ, row = (self.G, self.detJ, sg.g0) if sg.kind == 2 else (self.Gc, self.detJc, sg.c0)
+                geo = (sp(G, row), sp(dJ, row)) if self._m_accum else (sp(G, row),)
             if sg.kind == 1:
                 geo += (self._weights.data_ptr(),)
             self._arm(first)
@@ -656,12 +700,13 @@ class _RK4:
 
     # algorithmic HBM bytes (SURVEY.md section 8d)
     def _stiffness_bytes(self):
-        """One stiffness action: dofmap, G (or the compressed factors) and a coefficient per cell,
-        x read and b written per dof."""
+        """One stiffness action: dofmap, G (or the compressed factors, or the 36 trilinear
+        coefficients) and a coefficient per cell, x read and b written per dof."""
         s = self.dtype.itemsize
         Nd = self.n**3
-        nstream = self.ncells - self.naff
-        return nstream * (Nd * 4 + 6 * Nd * s + s) + self.naff * (Nd * 4 + 7 * s) + 2 * s * self.ndofs
+        nstream = self.ncells - self.naff - self.ntri
+        return (nstream * (Nd * 4 + 6 * Nd * s + s) + self.naff * (Nd * 4 + 7 * s) + self.ntri * (Nd * 4 + 37 * s)
+                + 2 * s * self.ndofs)
 
     def stage_bytes(self):
         """One RK stage: vector passes of the close kernels per step 9 + 12 + 12 + 8 (ping-pong),
@@ -687,16 +732,16 @@ class LinearSpectral3D(_RK4):
                  bfacet_dofmap1=None, detJ_f1=None, facet_coeff1=None, bfacet_dofmap2=None,
                  detJ_f2=None, facet_coeff2=None, halo=None, source=None,
                  source_at_stage_time=True, use_graph=True, geometry="stream", weights=None,
-                 split_cells=True):
+                 split_cells=True, trilinear=None):
         super().__init__(P, float_type, ndofs, dofmap, G, dphi_1D, halo, source,
-                         source_at_stage_time, use_graph, geometry, weights, split_cells)
+                         source_at_stage_time, use_graph, geometry, weights, split_cells, trilinear)
         torch = _torch()
         self.cell_coeff2 = _dev(cell_coeff2, self.T)
         c1 = _dev(cell_coeff1, self.T)
-        dJ = _dev(detJ, self.T)
+        dJ = _dev(detJ, self.T) if self._Tc is None else None
         # lumped mass: fill(1) -> mass -> scatter_rev  (cuda/demo_linear_box.py:421-428)
         ones = torch.ones(self.ndofs, dtype=self.T, device="cuda")
-        self._mass(ones, c1, self.m, dJ, self.dofmap)
+        self._cell_mass(ones, c1, self.m, dJ)
         if self.halo is not None:
             self.halo.reverse(self.m)
         self._abs_facets = self._facets(bfacet_dofmap2, detJ_f2, facet_coeff2)
@@ -840,22 +885,22 @@ class WesterveltSpectral3D(_RK4):
                  facet_coeff1_1=None, facet_coeff2_1=None, bfacet_dofmap2=None, detJ_f2=None,
                  facet_coeff1_2=None, facet_coeff2_2=None, halo=None, source=None,
                  source_at_stage_time=True, use_graph=True, geometry="stream", weights=None,
-                 mass_form="pointwise", split_cells=True):
+                 mass_form="pointwise", split_cells=True, trilinear=None):
         super().__init__(P, float_type, ndofs, dofmap, G, dphi_1D, halo, source,
-                         source_at_stage_time, use_graph, geometry, weights, split_cells)
+                         source_at_stage_time, use_graph, geometry, weights, split_cells, trilinear)
         torch = _torch()
         if mass_form not in ("pointwise", "cells"):
             raise ValueError("mass_form must be 'pointwise' or 'cells'")
         self.mass_form = mass_form
         self._m_accum = mass_form == "cells"
-        self.detJ = _dev(detJ, self.T)
+        self.detJ = _dev(detJ, self.T) if self._Tc is None else None
         self.c2, self.c3 = _dev(cell_coeff2, self.T), _dev(cell_coeff3, self.T)
         self.c4, self.c5 = _dev(cell_coeff4, self.T), _dev(cell_coeff5, self.T)
         c1 = _dev(cell_coeff1, self.T)
         # steady LHS m0 (cuda/demo_nonlinear_bowl.py:459-469)
         ones = torch.ones(self.ndofs, dtype=self.T, device="cuda")
         self.m0 = self._zx()  # reverse-exchanged once below: peer-addressable with the P2P halo
-        self._mass(ones, c1, self.m0, self.detJ, self.dofmap)
+        self._cell_mass(ones, c1, self.m0, self.detJ)
         absorbing = self._facets(bfacet_dofmap2, detJ_f2, facet_coeff1_2)
         if absorbing is not None:
             bd2, dJ2, fc = absorbing
@@ -870,8 +915,8 @@ class WesterveltSpectral3D(_RK4):
         if not self._m_accum:
             # lumped M(c2; 1) and M(c5; 1), owner-complete like m0
             self.m2, self.m5 = self._zx(), self._zx()
-            self._mass(ones, self.c2, self.m2, self.detJ, self.dofmap)
-            self._mass(ones, self.c5, self.m5, self.detJ, self.dofmap)
+            self._cell_mass(ones, self.c2, self.m2, self.detJ)
+            self._cell_mass(ones, self.c5, self.m5, self.detJ)
             if self.halo is not None:
                 self.halo.reverse(self.m2, self.m5)
         self._setup_geometry(self.detJ if self._m_accum else None, ["c2", "c3", "c4", "c5"])
@@ -903,6 +948,6 @@ class WesterveltSpectral3D(_RK4):
         s = self.dtype.itemsize
         Nd = self.n**3
         if self._m_accum:  # + detJ stream, second gather, m read-modify-write, m0, m zero
-            return super().stage_bytes() + (self.ncells - self.naff) * Nd * s + 6 * s * self.ndofs
+            return super().stage_bytes() + (self.ncells - self.naff - self.ntri) * Nd * s + 6 * s * self.ndofs
         # pointwise: + second gather (vn) in the stage kernel; close passes 11 + 15 + 15 + 11 per step
         return super().stage_bytes() + s * self.ndofs + (13 - 10.25) * s * self.ndofs

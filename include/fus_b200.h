@@ -201,6 +201,25 @@ int fus_stiffness2_vertex_f64(const double* xa, const double* ca, const double* 
 int fus_stiffness2_vertex_f32(const float* xa, const float* ca, const float* xb, const float* cb, float* y,
                               const float* Tc, const int32_t* dofmap, const float* dphi, int64_t ncells,
                               int P, int flags, void* stream);
+/* fus_stiffness_westervelt_vertex_* : fus_stiffness_westervelt_* on trilinear cells, Tc in place of G and detJ:
+ *     b += K(c3 ; un) + K(c4 ; vn) + M(c5 ; vn^2)        m += M(c2 ; un)
+ *     with M(c ; w)[dm] = c * w_q |det J(X_q)| * w[dm] taken from the same tangents as the stiffness.
+ *     Not combinable with FUS_NO_ATOMICS.
+ * fus_mass_vertex_* : the lumped mass y[dm[c,q]] += coeff[c] * w_q |det J_c(X_q)| * x[dm[c,q]] (fus_mass_* with
+ *     ncols = n^3 and the detJ table recomputed from Tc); reads the tables of fus_set_vertex_tables_*.  A solver
+ *     on trilinear cells builds its masses with it and never holds a (ncells, n^3) table. */
+int fus_stiffness_westervelt_vertex_f64(const double* un, const double* c3, const double* vn, const double* c4,
+                                        const double* c2, const double* c5, double* m, double* b, const double* Tc,
+                                        const int32_t* dofmap, const double* dphi, int64_t ncells, int P, int flags,
+                                        void* stream);
+int fus_stiffness_westervelt_vertex_f32(const float* un, const float* c3, const float* vn, const float* c4,
+                                        const float* c2, const float* c5, float* m, float* b, const float* Tc,
+                                        const int32_t* dofmap, const float* dphi, int64_t ncells, int P, int flags,
+                                        void* stream);
+int fus_mass_vertex_f64(const double* x, const double* coeff, double* y, const double* Tc, const int32_t* dofmap,
+                        int64_t ncells, int P, void* stream);
+int fus_mass_vertex_f32(const float* x, const float* coeff, float* y, const float* Tc, const int32_t* dofmap,
+                        int64_t ncells, int P, void* stream);
 
 /* Per cell: Gc[c,:] = mean_q G[c,q,:] / wq[q], detJc[c] = mean_q detJ[c,q] / wq[q] (detJ may be
  * NULL) and affine[c] = 1 when every G[c,q,:] / wq[q] (and detJ[c,q] / wq[q]) lies within
