@@ -72,6 +72,8 @@ def _sigs():
         "fus_rk_close_westervelt": [P, P, P, P, P, P, P, P, P, P, T, T, I, L, P, P, P],
         "fus_boundary_terms": [P, P, P, P, P, P, T, T, P, P, I, I, L, P],
         "fus_boundary_terms_signal": [P, P, P, P, P, P, P, T, T, P, P, I, I, L, I, P],
+        "fus_boundary_terms_elements": [P, P, P, P, P, P, P, P, P, P, I, I, L, P],
+        "fus_boundary_terms_elements_signal": [P, P, P, P, P, P, P, P, P, P, P, I, I, L, I, P],
         "fus_westervelt_mass": [P, P, P, P, P, P, P, P, L, I, P],
         "fus_geometry": [P, P, P, P, P, P, L, I, P],
         "fus_facet_geometry": [P, P, P, P, P, P, L, I, P],

@@ -340,6 +340,17 @@ __global__ void __launch_bounds__(kSharedThreads) rk_close_shared_kernel(const C
   }
 }
 
+// The end of a multi-GPU stage's boundary launch: the last block raises the REV epoch on every owner
+// of my ghosts (= fus_halo_signal_reverse, without a launch of its own on the critical path).
+__device__ __forceinline__ void boundary_signal(const FusHaloDev& h, int consume_fwd) {
+  if (fus_last_block(&h.ctr[FUS_CTR_TICKET_BOUNDARY])) {
+    // the stiffness launches of this stage have consumed one FWD epoch (their in-kernel wait
+    // reads the counter, this kernel - the next one on the stream - advances it)
+    if (threadIdx.x == 0 && consume_fwd) h.ctr[FUS_CTR_FWD_WAITED] += 1ULL;
+    fus_signal(&h.ctr[FUS_CTR_TICKET_BOUNDARY], &h.ctr[FUS_CTR_REV_SENT], h.rev_targets, h.n_owner_ranks);
+  }
+}
+
 // b[dof[i]] += g*src[i] + dg*src2[i] + vn[dof[i]]*absb[i]; the dof list is unique.
 // SIGNAL (multi-GPU): this is the last kernel of a stage that writes ghost partial sums, so its
 // last block raises the REV epoch on every owner of my ghosts (= fus_halo_signal_reverse, without
@@ -365,14 +376,40 @@ __global__ void __launch_bounds__(kThreads)
     if (absb != nullptr) acc += vn[d] * absb[i];
     b[d] += acc;
   }
-  if constexpr (SIGNAL) {
-    if (fus_last_block(&h.ctr[FUS_CTR_TICKET_BOUNDARY])) {
-      // the stiffness launches of this stage have consumed one FWD epoch (their in-kernel wait
-      // reads the counter, this kernel - the next one on the stream - advances it)
-      if (threadIdx.x == 0 && consume_fwd) h.ctr[FUS_CTR_FWD_WAITED] += 1ULL;
-      fus_signal(&h.ctr[FUS_CTR_TICKET_BOUNDARY], &h.ctr[FUS_CTR_REV_SENT], h.rev_targets, h.n_owner_ranks);
+  if constexpr (SIGNAL) boundary_signal(h, consume_fwd);
+}
+
+// Phased-array source: every source dof carries one (element, weight) entry per array element whose
+// facets contain it (CSR rows over the same compact dof list; a dof that only absorbs has an empty
+// row), and the element's own stage amplitudes come from the table
+//   G = etab + step*8E + stage*2E,  DG = G + E          (layout (rows, 4 stages, 2, E))
+//   b[dof[i]] += sum_{k in row i} (w[k] G[elem[k]] + w2[k] DG[elem[k]]) + vn[dof[i]] absb[i]
+// One thread per dof, the sum in row order: deterministic, no atomics.  The 2E stage values are read
+// through the read-only path: E <= a few thousand values shared by every thread stay in L1 / L2.
+template <typename T, bool SIGNAL>
+__global__ void __launch_bounds__(kThreads)
+    boundary_elements_kernel(T* b, const T* __restrict__ vn, const int32_t* __restrict__ dof,
+                             const int32_t* __restrict__ row, const int32_t* __restrict__ elem,
+                             const T* __restrict__ w, const T* __restrict__ w2, const T* __restrict__ absb,
+                             const T* __restrict__ etab, const long long* __restrict__ step, int E, int stage,
+                             long long n, const FusHaloDev h, int consume_fwd) {
+  const long long s = step != nullptr ? *step : 0;
+  const T* __restrict__ G = etab + s * 8LL * E + 2LL * stage * E;
+  const T* __restrict__ DG = G + E;
+  const long long stride = (long long)gridDim.x * kThreads;
+  for (long long i = (long long)blockIdx.x * kThreads + threadIdx.x; i < n; i += stride) {
+    const int d = dof[i];
+    const int k1 = row[i + 1];
+    T acc = T(0);
+    for (int k = row[i]; k < k1; ++k) {
+      const int e = elem[k];
+      acc += w[k] * __ldg(G + e);
+      if (w2 != nullptr) acc += w2[k] * __ldg(DG + e);
     }
+    if (absb != nullptr) acc += vn[d] * absb[i];
+    b[d] += acc;
   }
+  if constexpr (SIGNAL) boundary_signal(h, consume_fwd);
 }
 
 inline unsigned grid_for(long long n) {
@@ -489,6 +526,32 @@ int boundary_entry(T* b, const T* vn, const int32_t* dof, const T* src, const T*
   return 0;
 }
 
+template <typename T>
+int boundary_elements_entry(T* b, const T* vn, const int32_t* dof, const int32_t* row, const int32_t* elem,
+                            const T* w, const T* w2, const T* absb, const T* etab, const int64_t* step, int E,
+                            int stage, int64_t n, void* stream, fus_halo* halo = nullptr, int consume_fwd = 0) {
+  if (n < 0) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "boundary_terms_elements: n < 0");
+  if (E < 1) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "boundary_terms_elements: num_elements < 1");
+  if (stage < 0 || stage > 3) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "boundary_terms_elements: stage 0..3");
+  if (n > 0 && (b == nullptr || dof == nullptr || etab == nullptr || row == nullptr || elem == nullptr || w == nullptr))
+    return fus_set_error(FUS_ERR_BAD_ARGUMENT, "boundary_terms_elements: null b / dof / etab / row / elem / w");
+  if (n > 0 && absb != nullptr && vn == nullptr)
+    return fus_set_error(FUS_ERR_BAD_ARGUMENT, "boundary_terms_elements: null vn with absb");
+  const bool signal = halo != nullptr && fus_halo_dev_of(halo)->n_owner_ranks > 0;
+  if (n == 0 && !signal) return 0;
+  cudaStream_t st_ = static_cast<cudaStream_t>(stream);
+  const long long* stp = reinterpret_cast<const long long*>(step);
+  if (signal) {
+    boundary_elements_kernel<T, true><<<grid_for(n), kThreads, 0, st_>>>(
+        b, vn, dof, row, elem, w, w2, absb, etab, stp, E, stage, n, *fus_halo_dev_of(halo), consume_fwd);
+  } else {
+    boundary_elements_kernel<T, false><<<grid_for(n), kThreads, 0, st_>>>(
+        b, vn, dof, row, elem, w, w2, absb, etab, stp, E, stage, n, FusHaloDev{}, 0);
+  }
+  FUS_LAUNCH_CHECK("boundary_elements_kernel");
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -545,6 +608,23 @@ extern "C" {
       return fus_set_error(FUS_ERR_BAD_ARGUMENT, "boundary_terms_signal: null halo handle");     \
     return boundary_entry<T>(b, vn, dof, src, src2, absb, g, dg, gtab, step_dev, gstride, goff,  \
                              n, s, halo, consume_forward);                                       \
+  }                                                                                              \
+  int fus_boundary_terms_elements_##SFX(T* b, const T* vn, const int32_t* dof, const int32_t* row,  \
+                                        const int32_t* elem, const T* w, const T* w2,            \
+                                        const T* absb, const T* etab, const int64_t* step_dev,   \
+                                        int num_elements, int stage, int64_t n, void* s) {       \
+    return boundary_elements_entry<T>(b, vn, dof, row, elem, w, w2, absb, etab, step_dev,        \
+                                      num_elements, stage, n, s);                                \
+  }                                                                                              \
+  int fus_boundary_terms_elements_signal_##SFX(                                                  \
+      fus_halo_t* halo, T* b, const T* vn, const int32_t* dof, const int32_t* row,               \
+      const int32_t* elem, const T* w, const T* w2, const T* absb, const T* etab,                \
+      const int64_t* step_dev, int num_elements, int stage, int64_t n, int consume_forward,      \
+      void* s) {                                                                                 \
+    if (halo == nullptr)                                                                         \
+      return fus_set_error(FUS_ERR_BAD_ARGUMENT, "boundary_terms_elements_signal: null halo handle"); \
+    return boundary_elements_entry<T>(b, vn, dof, row, elem, w, w2, absb, etab, step_dev,        \
+                                      num_elements, stage, n, s, halo, consume_forward);         \
   }
 
 FUS_RK_API(f64, double)

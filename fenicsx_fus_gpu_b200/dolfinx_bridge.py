@@ -14,7 +14,8 @@ touch - and returns the ``problem.Setup`` the fused solvers are built from, so
     bd_abs = utils.facet_integration_domain(absorbing_facets, mesh)
     solver = problem.linear_solver(su, bd_src, bd_abs, rho=..., c0=..., f0=..., p0=...)
 
-replaces everything between ``functionspace(...)`` and the time loop.  The mesh may be
+replaces everything between ``functionspace(...)`` and the time loop.  A phased-array source takes one
+element index per row of ``bd_src`` (``problem.linear_solver(..., source_elements=..., element_delays=...)``).  The mesh may be
 unstructured: nothing here assumes a box.  DOLFINx and Basix are not in this image, so
 the bridge is exercised with stand-in objects exposing the same attributes
 (tests/test_host_logic.py); with Basix importable the element tables come from Basix

@@ -196,35 +196,147 @@ def cfl_time_step(P, h, c0, f0, cfl):
     return period / (int(period / dt) + 1)
 
 
+def facet_centroids(mesh, boundary_data):
+    """(nf, 3) centroids of the facets ``boundary_data`` (rows (cell, local facet)) from their four
+    vertices."""
+    bd = np.asarray(boundary_data).reshape(-1, 2)
+    cen = np.zeros((bd.shape[0], 3), dtype=np.asarray(mesh.x_g).dtype)
+    for lf in np.unique(bd[:, 1]):
+        axis, side = S._FACE_AXIS[int(lf)]
+        fv = [v for v in range(8) if ((v >> axis) & 1) == side]
+        sel = bd[:, 1] == lf
+        cen[sel] = mesh.x_g[mesh.x_dofs[bd[sel, 0]][:, fv]].mean(axis=1)
+    return cen
+
+
+class TileArray:
+    """A planar transducer array of ``na x nb`` square elements of side ``pitch`` (no kerf) on a
+    source face, centred at the point ``centre`` of that face, its rows along ``axes[0]`` and its
+    columns along ``axes[1]``; the third axis is the face normal.  Element ``e = ia * nb + ib``.
+    The description is global: every rank holds the same ``centres``."""
+
+    def __init__(self, centre, na, nb, pitch, axes=(0, 1)):
+        self.centre = np.asarray(centre, dtype=np.float64).reshape(3)
+        self.na, self.nb, self.pitch = int(na), int(nb), float(pitch)
+        self.axes = tuple(int(a) for a in axes)
+        if self.na < 1 or self.nb < 1 or not self.pitch > 0 or len(set(self.axes)) != 2:
+            raise ValueError("TileArray: na, nb >= 1, pitch > 0 and two distinct in-plane axes")
+        self.E = self.na * self.nb
+        a, b = self.axes
+        ia, ib = np.divmod(np.arange(self.E), self.nb)
+        self.centres = np.tile(self.centre, (self.E, 1))
+        self.centres[:, a] += (ia - 0.5 * (self.na - 1)) * self.pitch
+        self.centres[:, b] += (ib - 0.5 * (self.nb - 1)) * self.pitch
+
+    def element_of(self, centroids):
+        """Element index of every facet centroid (nf, 3); -1 outside the aperture (such facets
+        are not part of the source)."""
+        c = np.asarray(centroids, dtype=np.float64).reshape(-1, 3)
+        a, b = self.axes
+        ia = np.floor((c[:, a] - self.centre[a]) / self.pitch + 0.5 * self.na)
+        ib = np.floor((c[:, b] - self.centre[b]) / self.pitch + 0.5 * self.nb)
+        inside = (ia >= 0) & (ia < self.na) & (ib >= 0) & (ib < self.nb)
+        return np.where(inside, ia * self.nb + ib, -1).astype(np.int64)
+
+
+def focus_delays(centres, focus, c0):
+    """Firing delays that focus an array on ``focus``: ``tau_e = (max_j r_j - r_e) / c0`` with
+    ``r_e`` the distance from element centre e, so every wave arrives at the same time and every
+    ``tau_e >= 0``."""
+    r = np.linalg.norm(np.asarray(centres, dtype=np.float64) - np.asarray(focus, dtype=np.float64), axis=1)
+    return (r.max() - r) / c0
+
+
+def element_source(base, amplitudes, delays):
+    """``t -> (A_e g(t - tau_e), A_e dg(t - tau_e))`` for the ``E`` elements of an array, from one
+    waveform ``base(t) -> (g, dg)`` that accepts an array ``t`` (``linear_source``,
+    ``westervelt_source``).  Element e is silent, both terms exactly 0, for ``t < tau_e``."""
+    A = np.asarray(amplitudes, dtype=np.float64)
+    tau = np.asarray(delays, dtype=np.float64)
+    if A.ndim != 1 or A.shape != tau.shape:
+        raise ValueError("element_source: amplitudes and delays must both have shape (E,)")
+
+    def source(t):
+        tl = t - tau
+        g, dg = base(tl)
+        on = tl >= 0.0
+        return np.where(on, A * g, 0.0), np.where(on, A * dg, 0.0)
+
+    return source
+
+
+def _array_source(su, source_facets, source_predicate, base, kw, source_elements, element_amplitudes,
+                  element_delays):
+    """The source facet group and the solver keywords of a single or a phased-array source.
+    ``source_elements``: a ``TileArray`` (the facets outside its aperture are dropped), or one
+    element index per row of the source facet group."""
+    tile = source_elements if isinstance(source_elements, TileArray) else None
+    if tile is not None:
+        pred = source_predicate
+        source_predicate = lambda cen: (tile.element_of(cen) >= 0) & (  # noqa: E731
+            True if pred is None else np.asarray(pred(cen), bool))
+    fd1, dJ1, bd1 = facet_group(su, source_facets, source_predicate)
+    if source_elements is None:
+        if element_amplitudes is not None or element_delays is not None:
+            raise ValueError("element_amplitudes / element_delays need source_elements")
+        kw["source"] = base
+        return fd1, dJ1, bd1
+    if tile is not None:
+        ids = tile.element_of(facet_centroids(su.mesh, bd1))
+        if (ids < 0).any():  # DOLFINx rows given directly: keep those inside the aperture
+            keep = np.flatnonzero(ids >= 0)
+            fd1, dJ1, bd1, ids = fd1[_d(keep)], dJ1[_d(keep)], bd1[keep], ids[keep]
+        E = tile.E
+    else:
+        ids = np.asarray(source_elements, dtype=np.int64).reshape(-1)
+        E = next((len(a) for a in (element_amplitudes, element_delays) if a is not None), None)
+    if E is None:
+        E = int(ids.max()) + 1 if ids.size else 1
+    A = np.ones(E) if element_amplitudes is None else np.asarray(element_amplitudes, dtype=np.float64)
+    tau = np.zeros(E) if element_delays is None else np.asarray(element_delays, dtype=np.float64)
+    if A.shape != (E,) or tau.shape != (E,):
+        raise ValueError(f"element_amplitudes and element_delays must have shape ({E},)")
+    kw.update(source=element_source(base, A, tau), source_elements=ids, num_elements=E)
+    return fd1, dJ1, bd1
+
+
 def linear_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0=1500.0, f0=0.5e6,
                   p0=60000.0, source_predicate=None, absorbing_predicate=None, integrator="rk4",
+                  source_elements=None, element_amplitudes=None, element_delays=None,
                   **kw) -> LinearSpectral3D:
     """cuda/demo_linear_box.py:336-345 coefficients + the fused solver (``integrator``: "rk4", the
-    reference's scheme, or "leapfrog")."""
+    reference's scheme, or "leapfrog").  ``source_elements`` (a ``TileArray``, or one element index
+    per source facet row) makes the source a phased array: element e emits
+    ``A_e g(t - tau_e)`` with ``A = element_amplitudes`` (default 1) and ``tau = element_delays``
+    (default 0; ``focus_delays`` focuses)."""
     if integrator not in ("rk4", "leapfrog"):
         raise ValueError("integrator must be 'rk4' or 'leapfrog'")
     cls = LinearLeapfrog3D if integrator == "leapfrog" else LinearSpectral3D
     nc = su.mesh.num_cells
     _geometry_kw(su, kw)
-    fd1, dJ1, bd1 = facet_group(su, source_facets, source_predicate)
+    fd1, dJ1, bd1 = _array_source(su, source_facets, source_predicate, lambda t: linear_source(t, f0, p0, c0), kw,
+                                  source_elements, element_amplitudes, element_delays)
     fd2, dJ2, bd2 = facet_group(su, absorbing_facets, absorbing_predicate)
     return cls(
         su.P, su.dtype, su.ndofs, su.dev["dofmap"], su.dev.get("G"), su.dev.get("detJ"), su.tables.dphi_1D,
         _full(su, nc, 1.0 / rho / c0 / c0), _full(su, nc, -1.0 / rho),
         fd1, dJ1, _full(su, bd1.shape[0], 1.0 / rho), fd2, dJ2, _full(su, bd2.shape[0], -1.0 / rho / c0),
-        halo=su.halo, source=lambda t: linear_source(t, f0, p0, c0), **kw)
+        halo=su.halo, **kw)
 
 
 def westervelt_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0=1480.0, f0=1.1e6,
                       p0=None, beta=3.5, alpha_dB=0.2, source_predicate=None, absorbing_predicate=None,
+                      source_elements=None, element_amplitudes=None, element_delays=None,
                       **kw) -> WesterveltSpectral3D:
-    """cuda/demo_nonlinear_bowl.py:358-374 coefficients + the fused solver."""
+    """cuda/demo_nonlinear_bowl.py:358-374 coefficients + the fused solver; phased-array keywords
+    as for ``linear_solver``."""
     if p0 is None:
         p0 = rho * c0 * 0.38557513826589934  # source velocity of the bowl demo (:66-67)
     delta = utils.compute_diffusivity_of_sound(2.0 * np.pi * f0, c0, alpha_dB)
     nc = su.mesh.num_cells
     _geometry_kw(su, kw)
-    fd1, dJ1, bd1 = facet_group(su, source_facets, source_predicate)
+    fd1, dJ1, bd1 = _array_source(su, source_facets, source_predicate, lambda t: westervelt_source(t, f0, p0, c0),
+                                  kw, source_elements, element_amplitudes, element_delays)
     fd2, dJ2, bd2 = facet_group(su, absorbing_facets, absorbing_predicate)
     n1, n2 = bd1.shape[0], bd2.shape[0]
     return WesterveltSpectral3D(
@@ -234,7 +346,7 @@ def westervelt_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0
         _full(su, nc, 2.0 * beta / rho / rho / c0**4),
         fd1, dJ1, _full(su, n1, 1.0 / rho), _full(su, n1, delta / rho / c0 / c0),
         fd2, dJ2, _full(su, n2, delta / rho / c0**3), _full(su, n2, -1.0 / rho / c0),
-        halo=su.halo, source=lambda t: westervelt_source(t, f0, p0, c0), **kw)
+        halo=su.halo, **kw)
 
 
 def disc(axis_a, axis_b, centre, radius):

@@ -97,21 +97,21 @@ def _dev(a, dtype=None):
 
 
 def linear_source(t, f0, p0, c0, alpha=4.0):
-    """``g(t)`` of cuda/demo_linear_box.py:511-530 (numba-cpu :341-358)."""
+    """``g(t)`` of cuda/demo_linear_box.py:511-530 (numba-cpu :341-358).  ``t`` may be an array
+    (one time per array element); a scalar ``t`` gives the same bits either way."""
     T = 1.0 / f0
-    window = 0.5 * (1.0 - np.cos(f0 * np.pi * t / alpha)) if t < T * alpha else 1.0
+    window = np.where(t < T * alpha, 0.5 * (1.0 - np.cos(f0 * np.pi * t / alpha)), 1.0)
     return window * p0 * 2.0 * np.pi * f0 / c0 * np.cos(2.0 * np.pi * f0 * t), 0.0
 
 
 def westervelt_source(t, f0, p0, c0, alpha=4.0):
-    """``g(t), dg/dt`` of cuda/demo_nonlinear_bowl.py:556-594."""
+    """``g(t), dg/dt`` of cuda/demo_nonlinear_bowl.py:556-594.  ``t`` may be an array, as for
+    ``linear_source``."""
     T = 1.0 / f0
     w0 = 2.0 * np.pi * f0
-    if t < T * alpha:
-        window = 0.5 * (1.0 - np.cos(f0 * np.pi * t / alpha))
-        dwindow = 0.5 * np.pi * f0 / alpha * np.sin(f0 * np.pi * t / alpha)
-    else:
-        window, dwindow = 1.0, 0.0
+    ramp = t < T * alpha
+    window = np.where(ramp, 0.5 * (1.0 - np.cos(f0 * np.pi * t / alpha)), 1.0)
+    dwindow = np.where(ramp, 0.5 * np.pi * f0 / alpha * np.sin(f0 * np.pi * t / alpha), 0.0)
     g = window * 2.0 * p0 * w0 / c0 * np.cos(w0 * t)
     dg = dwindow * 2.0 * p0 * w0 / c0 * np.cos(w0 * t) - window * 2.0 * p0 * w0**2 / c0 * np.sin(w0 * t)
     return g, dg
@@ -120,6 +120,14 @@ def westervelt_source(t, f0, p0, c0, alpha=4.0):
 class _RK4:
     """State vectors, boundary diagonals, graph capture, the stage sequence and the step loop
     shared by the linear and Westervelt solvers.
+
+    ``source_elements`` (phased-array sources): one element index in ``[0, E)`` per row of the
+    source facet group, ``E = num_elements`` (default: the largest index + 1; give it on every rank
+    of a partitioned run, where a rank may see only some elements or none).  ``source(t)`` then
+    returns ``(g, dg)`` as arrays of shape ``(E,)``, one waveform per element, and every source
+    launch reads the element's amplitudes from a device table of ``8 E`` values per step
+    (``fus_boundary_terms_elements_*``).  The table takes ``rows * 8 E * itemsize`` bytes: about
+    80 MB for E = 1024 over 1219 float64 steps.
 
     A solver class states its cell-kernel form (``form``: the kernels ``fus_<form>[_rect|_affine]``,
     and ``_operands``: their leading arguments for a cell range) and its close (``_close_name``:
@@ -131,7 +139,7 @@ class _RK4:
 
     def __init__(self, P, float_type, ndofs, dofmap, G, dphi_1D, halo=None, source=None,
                  source_at_stage_time=True, use_graph=True, geometry="stream", weights=None,
-                 split_cells=True, trilinear=None):
+                 split_cells=True, trilinear=None, source_elements=None, num_elements=None):
         torch = _torch()
         if not torch.cuda.is_available():
             raise _lib.FusError("no CUDA device: this package has no CPU path")
@@ -212,6 +220,24 @@ class _RK4:
         self._opened = False
         self._bdofs = None
         self._src = self._src2 = self._absb = None
+        # phased-array source (None: one waveform for every source facet)
+        self.num_elements = None
+        self._elem_ids = self._erow = self._eelem = self._ew = self._ew2 = self._etab1 = None
+        if source_elements is not None:
+            ids = _dev(source_elements, torch.int64)
+            if ids.dim() != 1:
+                raise ValueError("source_elements must be one element index per source facet row")
+            lo, hi = (int(ids.min().item()), int(ids.max().item())) if ids.numel() else (0, -1)
+            if num_elements is None:
+                if hi < 0:
+                    raise ValueError("source_elements is empty: give num_elements")
+                num_elements = hi + 1
+            self.num_elements = int(num_elements)
+            if self.num_elements < 1 or lo < 0 or hi >= self.num_elements:
+                raise ValueError(f"source_elements must lie in [0, {self.num_elements}), got [{lo}, {hi}]")
+            self._elem_ids = ids
+        elif num_elements is not None:
+            raise ValueError("num_elements needs source_elements")
         self.probe = None  # list: (start, stop) CUDA events around every stage-kernel launch (eager mode)
         self.geometry = geometry
         self._weights = None if weights is None else _dev(weights, self.T)
@@ -288,19 +314,60 @@ class _RK4:
     def _boundary_setup(self, **groups):
         """``groups``: slot ("src", "src2", "absb") -> facet group of ``_facets`` or None.  Builds
         the compact unique-dof list and the diagonals = the facet mass operator applied to ones
-        (cuda/demo_linear_box.py:546-551)."""
+        (cuda/demo_linear_box.py:546-551); with a phased-array source, the per-element rows of
+        the source slots instead (``_element_rows``)."""
         torch = _torch()
+        src = {slot: groups.pop(slot, None) for slot in ("src", "src2")} if self.num_elements is not None else {}
+        nonempty = {slot: g for slot, g in {**groups, **src}.items() if g is not None}
         groups = {slot: g for slot, g in groups.items() if g is not None}
-        if not groups:
+        if not nonempty:
             self._bdofs = torch.zeros(0, dtype=torch.int32, device="cuda")
-            return
-        self._bdofs = torch.unique(torch.cat([g[0].reshape(-1) for g in groups.values()])).to(torch.int32).contiguous()
+        else:
+            self._bdofs = torch.unique(torch.cat([g[0].reshape(-1) for g in nonempty.values()])).to(torch.int32).contiguous()
         idx = self._bdofs.to(torch.int64)
         ones = torch.ones(self.ndofs, dtype=self.T, device="cuda")
         for slot, (bdm, dJ, coeff) in groups.items():
             tmp = torch.zeros(self.ndofs, dtype=self.T, device="cuda")
             self._mass(ones, coeff, tmp, dJ, bdm)
             setattr(self, "_" + slot, tmp[idx].contiguous())
+        if self.num_elements is not None:
+            self._element_rows(src["src"], src["src2"])
+
+    def _element_rows(self, src, src2):
+        """CSR rows over ``_bdofs`` of the phased-array source: for every boundary dof, one entry
+        (element, w[, w2]) per element whose facets contain it, w = the facet coefficient times
+        detJ_f summed over those facets (the facet mass diagonal of the element).  Built on the
+        device: the facet rows are expanded into (dof, element, weight) entries, sorted by
+        (dof, element) and reduced per key, one pass per position inside a key, so that the sums
+        run in facet order and do not depend on the order of atomics."""
+        torch = _torch()
+        E = self.num_elements
+        nf = 0 if src is None else int(src[0].shape[0])
+        if self._elem_ids.numel() != nf:
+            raise ValueError(f"source_elements has {self._elem_ids.numel()} entries, the source facet group {nf} rows")
+        i64 = dict(dtype=torch.int64, device="cuda")
+        if nf:
+            bdm, dJ, coeff = src
+            key = bdm.reshape(-1).to(torch.int64) * E + self._elem_ids.repeat_interleave(bdm.shape[1])
+            key, order = torch.sort(key, stable=True)
+            vals = [(c[:, None] * dJ).reshape(-1)[order] for c in (coeff, None if src2 is None else src2[2])
+                    if c is not None]
+            ukey, inv, counts = torch.unique_consecutive(key, return_inverse=True, return_counts=True)
+            pos = torch.arange(key.numel(), **i64) - (torch.cumsum(counts, 0) - counts)[inv]
+            sums = [torch.zeros(ukey.numel(), dtype=self.T, device="cuda") for _ in vals]
+            for j in range(int(counts.max().item())):
+                sel = pos == j  # at most one entry per key: each sum gets one add per pass
+                for acc, v in zip(sums, vals):
+                    acc.index_add_(0, inv[sel], v[sel])
+        else:
+            ukey, sums = torch.zeros(0, **i64), [torch.zeros(0, dtype=self.T, device="cuda")] * (1 + (src2 is not None))
+        row = torch.searchsorted(ukey // E, self._bdofs.to(torch.int64))
+        self._erow = torch.cat([row, torch.tensor([ukey.numel()], **i64)]).to(torch.int32).contiguous()
+        # the kernel takes non-null element arrays whenever the dof list is not empty
+        pad = lambda t: (t if t.numel() else torch.zeros(1, dtype=t.dtype, device="cuda")).contiguous()  # noqa: E731
+        self._eelem = pad((ukey % E).to(torch.int32))
+        self._ew = pad(sums[0])
+        self._ew2 = pad(sums[1]) if len(sums) > 1 else None
 
     def _setup_geometry(self, detJ, cell_arrays):
         """Order the cells for the launches of a stage and build the launch ranges.
@@ -400,9 +467,21 @@ class _RK4:
 
     def _boundary(self, stage, g, dg, use_table, vn, signal=False, consume=False):
         """b += g*src + dg*src2 + vn*absb on the boundary dofs.  ``signal`` (peer-memory halo): the
-        launch also raises the "ghost sums complete" epoch (and happens even without boundary dofs)."""
+        launch also raises the "ghost sums complete" epoch (and happens even without boundary dofs).
+        Phased-array source: the element amplitudes come from the step's table row, or without the
+        table from the one-row table ``_load_eager_row`` wrote (``g``, ``dg`` are not used)."""
         nb = int(self._bdofs.numel())
         if not nb and not signal:
+            return
+        if self.num_elements is not None:
+            tab, step = (self.gtab, self.step_dev) if use_table else (self._etab1, None)
+            args = (self.b.data_ptr(), vn.data_ptr(), self._bdofs.data_ptr() if nb else None, self._erow.data_ptr(),
+                    self._eelem.data_ptr(), self._ew.data_ptr(), self._ptr(self._ew2), self._ptr(self._absb),
+                    tab.data_ptr(), self._ptr(step), self.num_elements, stage, nb)
+            name = "fus_boundary_terms_elements_signal" if signal else "fus_boundary_terms_elements"
+            extra = (self.halo.handle,) if signal else ()
+            tail = (int(consume),) if signal else ()
+            check(fn(name, self.dtype)(*extra, *args, *tail, current_stream()), name)
             return
         args = (self.b.data_ptr(), vn.data_ptr(), self._bdofs.data_ptr() if nb else None, self._ptr(self._src),
                 self._ptr(self._src2), self._ptr(self._absb), float(g), float(dg),
@@ -590,7 +669,10 @@ class _RK4:
 
     def source_table(self, t0, dt, nsteps):
         """(nsteps, 8) table of (g, dg) per stage, times accumulated as the
-        reference does (``t += dt``)."""
+        reference does (``t += dt``).  Phased-array source: (nsteps, 8 E), per stage the E values
+        of g, then the E values of dg."""
+        if self.num_elements is not None:
+            return self._element_table(t0, dt, nsteps)
         tab = np.zeros((max(nsteps, 1), 8), dtype=self.dtype)
         t = t0
         for k in range(nsteps):
@@ -598,6 +680,30 @@ class _RK4:
                 tab[k, 2 * i], tab[k, 2 * i + 1] = self._source_at(i, dt, t, False)
             t += dt
         return tab
+
+    def _element_table(self, t0, dt, nsteps):
+        E = self.num_elements
+        tab = np.zeros((max(nsteps, 1), 4, 2, E), dtype=self.dtype)
+        t = t0
+        for k in range(nsteps if self.source is not None else 0):
+            for i in range(4):
+                g, dg = self._source_at(i, dt, t, False)
+                if np.shape(g) != (E,) or np.shape(dg) not in ((E,), ()):
+                    raise ValueError(f"source(t) must return (g, dg) of shape ({E},), got {np.shape(g)} and "
+                                     f"{np.shape(dg)}")
+                tab[k, i, 0], tab[k, i, 1] = g, dg
+            t += dt
+        return tab.reshape(tab.shape[0], 8 * E)
+
+    def _load_eager_row(self, t, dt):
+        """Phased-array source without the table: the element amplitudes of the four stages of the
+        step from ``t`` into a one-row device table of its own (the step table and its graph are
+        not touched)."""
+        torch = _torch()
+        row = torch.from_numpy(self._element_table(t, dt, 1))
+        if self._etab1 is None:
+            self._etab1 = torch.zeros(row.shape, dtype=self.T, device="cuda")
+        self._etab1.copy_(row)
 
     def rk4(self, t0, dt, nsteps):
         """``nsteps`` RK4 steps of size ``dt`` from ``t0``; returns the final time.
@@ -636,7 +742,7 @@ class _RK4:
         rows = tab.shape[0]
         if self.gtab is None or self.gtab.shape[0] < rows:
             cap = max(rows, 256 if self.gtab is None else 2 * self.gtab.shape[0])
-            self.gtab = torch.zeros((cap, 8), dtype=self.T, device="cuda")
+            self.gtab = torch.zeros((cap, tab.shape[1]), dtype=self.T, device="cuda")
         self.gtab[:rows].copy_(torch.from_numpy(np.ascontiguousarray(tab)))
 
     def step_eager(self, dt):
@@ -644,6 +750,8 @@ class _RK4:
         self._set_tables()
         if not self._opened:
             self._open_first()
+        if self.num_elements is not None:
+            self._load_eager_row(self.t, dt)
         self.begin_steps()
         self._enqueue_step(dt, self.t, False)
         self._parity ^= 1
@@ -732,9 +840,10 @@ class LinearSpectral3D(_RK4):
                  bfacet_dofmap1=None, detJ_f1=None, facet_coeff1=None, bfacet_dofmap2=None,
                  detJ_f2=None, facet_coeff2=None, halo=None, source=None,
                  source_at_stage_time=True, use_graph=True, geometry="stream", weights=None,
-                 split_cells=True, trilinear=None):
+                 split_cells=True, trilinear=None, source_elements=None, num_elements=None):
         super().__init__(P, float_type, ndofs, dofmap, G, dphi_1D, halo, source,
-                         source_at_stage_time, use_graph, geometry, weights, split_cells, trilinear)
+                         source_at_stage_time, use_graph, geometry, weights, split_cells, trilinear,
+                         source_elements, num_elements)
         torch = _torch()
         self.cell_coeff2 = _dev(cell_coeff2, self.T)
         c1 = _dev(cell_coeff1, self.T)
@@ -816,6 +925,8 @@ class LinearLeapfrog3D(LinearSpectral3D):
     def _kick(self, t0, dt):
         """v(t0) -> v(t0 - dt/2): half a step backwards with the acceleration at t0."""
         g, dg = self._source_at(0, dt, t0, False)
+        if self.num_elements is not None:
+            self._load_eager_row(t0, dt)
         self._assemble_exchanged(0, g, dg, False, self.u, self.v)
         self._lf_close(self.m, -0.5 * dt, 0.0, False)
         if self.p2p and self.ndofs > self.nupd:
@@ -885,9 +996,11 @@ class WesterveltSpectral3D(_RK4):
                  facet_coeff1_1=None, facet_coeff2_1=None, bfacet_dofmap2=None, detJ_f2=None,
                  facet_coeff1_2=None, facet_coeff2_2=None, halo=None, source=None,
                  source_at_stage_time=True, use_graph=True, geometry="stream", weights=None,
-                 mass_form="pointwise", split_cells=True, trilinear=None):
+                 mass_form="pointwise", split_cells=True, trilinear=None, source_elements=None,
+                 num_elements=None):
         super().__init__(P, float_type, ndofs, dofmap, G, dphi_1D, halo, source,
-                         source_at_stage_time, use_graph, geometry, weights, split_cells, trilinear)
+                         source_at_stage_time, use_graph, geometry, weights, split_cells, trilinear,
+                         source_elements, num_elements)
         torch = _torch()
         if mass_form not in ("pointwise", "cells"):
             raise ValueError("mass_form must be 'pointwise' or 'cells'")

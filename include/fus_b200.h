@@ -490,6 +490,39 @@ int fus_boundary_terms_signal_f32(fus_halo_t* halo, float* b, const float* vn, c
                                   float dg, const float* gtab, const int64_t* step_dev, int gstride,
                                   int goff, int64_t n, int consume_forward, void* stream);
 
+/* Multi-element (phased-array) source: the same boundary terms with one waveform per array element.
+ * Over the compact list of unique dofs dof[0..n):
+ *   b[dof[i]] += sum_{k = row[i]}^{row[i+1]-1} (w[k] G[elem[k]] + w2[k] DG[elem[k]]) + vn[dof[i]] absb[i]
+ * with G = etab + s*8E + stage*2E, DG = G + E, s = *step_dev (0 when step_dev is NULL): the table has
+ * the layout (rows, 4 stages, 2, E) - per step and RK stage the E amplitudes g_e, then the E dg_e/dt.
+ * row: int32 CSR offsets, n + 1 entries (an absorbing-only dof has an empty row); elem: int32 element
+ * ids in [0, E); w: the source facet mass diagonal of element elem[k] at the dof (facet coefficient
+ * times detJ_f, summed over that element's facets containing the dof); w2: the same with the dg
+ * coefficient (Westervelt), may be NULL; absb may be NULL.  A dof on the seam of two elements has one
+ * entry per element.  One thread per dof, the sum in row order: deterministic, no atomics.
+ * Rejected before any launch: n < 0, num_elements < 1, stage outside 0..3, and with n > 0 a NULL
+ * b, dof, etab, row, elem or w. */
+int fus_boundary_terms_elements_f64(double* b, const double* vn, const int32_t* dof, const int32_t* row,
+                                    const int32_t* elem, const double* w, const double* w2,
+                                    const double* absb, const double* etab, const int64_t* step_dev,
+                                    int num_elements, int stage, int64_t n, void* stream);
+int fus_boundary_terms_elements_f32(float* b, const float* vn, const int32_t* dof, const int32_t* row,
+                                    const int32_t* elem, const float* w, const float* w2,
+                                    const float* absb, const float* etab, const int64_t* step_dev,
+                                    int num_elements, int stage, int64_t n, void* stream);
+/* The same, followed by the "my ghost sums are complete" signal of fus_boundary_terms_signal_*
+ * (n may be 0: the signalling block still runs). */
+int fus_boundary_terms_elements_signal_f64(fus_halo_t* halo, double* b, const double* vn, const int32_t* dof,
+                                           const int32_t* row, const int32_t* elem, const double* w,
+                                           const double* w2, const double* absb, const double* etab,
+                                           const int64_t* step_dev, int num_elements, int stage, int64_t n,
+                                           int consume_forward, void* stream);
+int fus_boundary_terms_elements_signal_f32(fus_halo_t* halo, float* b, const float* vn, const int32_t* dof,
+                                           const int32_t* row, const int32_t* elem, const float* w,
+                                           const float* w2, const float* absb, const float* etab,
+                                           const int64_t* step_dev, int num_elements, int stage, int64_t n,
+                                           int consume_forward, void* stream);
+
 /* Westervelt stage helpers (cuda/demo_nonlinear_bowl.py:603-650):
  *   w = vn*vn                                                   (:603)
  *   fused cell-mass pair sharing one read of detJ and the dofmap:
