@@ -46,36 +46,45 @@ class PlaneSampler:
     """The reference's "Collect data" block (cuda/demo_linear_piston.py:555-582): once
     ``t > t_from``, every step for ``ndumps`` steps, the field on the sampling points goes
     to ``pressure_field_<k>.txt`` as rows ``x, z, p``.  The reference copies the whole
-    vector to the host and evaluates there; here one kernel samples on the device and only
-    the sampled values are copied."""
+    vector to the host and evaluates there; here the solver records the points inside its
+    captured steps (``record_points``) and the rows are copied once, after the run.
+    ``out_dir=None`` writes no files; ``values`` holds the rows (ndumps', npts) either way."""
 
     def __init__(self, evaluator, coords2, t_from, ndumps, out_dir, rank):
-        self.ev, self.t_from, self.ndumps, self.k = evaluator, t_from, ndumps, 0
-        self.data = None
-        self.dir, self.rank = out_dir, rank
-        if evaluator.npts:
-            import numpy as np
+        self.ev, self.t_from, self.ndumps = evaluator, t_from, ndumps
+        self.coords2, self.dir, self.rank = coords2, out_dir, rank
+        self.rows = self.values = None
+        if out_dir is not None:
+            os.makedirs(out_dir, exist_ok=True)
 
-            self.data = np.zeros((evaluator.npts, 3))
-            self.data[:, :2] = coords2
-        os.makedirs(out_dir, exist_ok=True)
+    def attach(self, solver, t0, dt, nsteps):
+        """Attach the recorder of the window to ``solver``: from the first step count whose time,
+        accumulated as the solver does (``t += dt``), exceeds ``t_from``, ``ndumps`` rows clipped to
+        the ``nsteps`` steps of the run.  Every rank attaches the same window."""
+        t, first = t0, 0
+        while first < nsteps:
+            t += dt
+            first += 1
+            if t > self.t_from:
+                break
+        rows = min(self.ndumps, nsteps - first + 1) if t > self.t_from else 0
+        self.rows = solver.record_points(self.ev, first, rows) if rows > 0 else None
 
-    def active(self, t):
-        return t > self.t_from and self.k < self.ndumps
-
-    def dump(self, solver):
+    def collect(self):
+        """After the run: the recorded rows to the host, one file per row."""
         import numpy as np
 
-        # ghost entries of the solution are made current by the same forward halo the next step
-        # starts with - scatter_fwd(u_n_d) in the reference (:566).  Collective: every rank dumps
-        # at the same steps.
-        if solver.halo is not None:
-            solver.halo.forward(solver.u, solver.v)
-        if self.data is not None:
-            self.data[:, 2] = self.ev.to_host(solver.u)
-            with open(os.path.join(self.dir, f"pressure_field_{self.k}_rank{self.rank}.txt"), "a") as f:
-                np.savetxt(f, self.data, fmt="%.8f", delimiter=",")
-        self.k += 1
+        if self.rows is None:
+            return
+        self.values = self.rows.cpu().numpy()
+        if self.dir is None or not self.ev.npts:
+            return
+        data = np.zeros((self.ev.npts, 3))
+        data[:, :2] = self.coords2
+        for k, row in enumerate(self.values):
+            data[:, 2] = row
+            with open(os.path.join(self.dir, f"pressure_field_{k}_rank{self.rank}.txt"), "a") as f:
+                np.savetxt(f, data, fmt="%.8f", delimiter=",")
 
 
 def run(solver, t0, dt, nsteps, rank, report=100, sampler=None):
@@ -84,29 +93,22 @@ def run(solver, t0, dt, nsteps, rank, report=100, sampler=None):
     import torch
 
     solver.init()
+    if sampler is not None:
+        sampler.attach(solver, t0, dt, nsteps)
     torch.cuda.synchronize()
     t_start = time.perf_counter()
     done = 0
     while done < nsteps:
         k = min(report - done % report, nsteps - done)
-        if sampler is not None and sampler.k < sampler.ndumps:
-            # stop at the first step of the sampling window, then go step by step through it
-            t_next = solver.t if done else t0
-            if sampler.active(t_next + dt):
-                k = 1
-            elif sampler.t_from > t_next:
-                k = max(1, min(k, int((sampler.t_from - t_next) / dt)))
         solver.rk4(solver.t if done else t0, dt, k)
         done += k
-        if sampler is not None and sampler.active(solver.t):
-            sampler.dump(solver)
-        if done % report and done < nsteps:
-            continue
         u0 = float(solver.u[0])  # device -> host read of one value (synchronises)
         if rank == 0:
             print(f"t: {solver.t:5.5},\t Steps: {done}/{nsteps}, \t u[0] = {u0}", flush=True)
     torch.cuda.synchronize()
     el = time.perf_counter() - t_start
+    if sampler is not None:
+        sampler.collect()
     if rank == 0:
         print(f"Solve time: {el}")
         print(f"Solve time per step: {el / max(1, nsteps)}")

@@ -2,10 +2,8 @@
 wave equation, f = 0.5 MHz), every other facet absorbing.  Each element fires with the delay
 that focuses the array on ``--focus`` (metres from the centre of the array: lateral x, lateral
 y, depth z; off-axis points steer the focus electronically, on the same mesh).  The x-z plane
-through the focus is sampled during the last period; the script prints where |p| peaks there
+through the focus is recorded every step of the last period; the script prints where |p| peaks there
 and how far that is from the requested focus."""
-
-import tempfile
 
 import numpy as np
 
@@ -59,25 +57,15 @@ def main():
     x_eval, cell_eval = sampling.compute_eval_params(su.mesh, points, dtype)
     ev = sampling.PointEvaluator(a.degree, dtype, su.dev["dofmap"], su.mesh, x_eval, cell_eval, su.tables.pts_1d)
 
-    class PeakSampler(_common.PlaneSampler):
-        """The plane dumps of the last period, with the running maximum of |p| per point."""
-
-        peak = np.zeros(ev.npts)
-
-        def dump(self, s):
-            super().dump(s)
-            if self.data is not None:
-                self.peak = np.maximum(self.peak, np.abs(self.data[:, 2]))
-
-    sampler = PeakSampler(ev, x_eval[:, [0, 2]], (nsteps - period - 0.5) * dt, period,
-                          a.sample_dir or tempfile.mkdtemp(prefix="phased_array_"), rank)
+    sampler = _common.PlaneSampler(ev, x_eval[:, [0, 2]], (nsteps - period - 0.5) * dt, period, a.sample_dir, rank)
     _common.run(solver, 0.0, dt, nsteps, rank, sampler=sampler)
+    peak = np.zeros(ev.npts) if sampler.values is None else np.abs(sampler.values).max(axis=0, initial=0.0)
     # the peak beyond one wavelength from the array (the elements' own near field is excluded)
     far = x_eval[:, 2] > c0 / f0
     best = (-1.0, 0.0, 0.0)
     if far.any():
-        i = int(np.argmax(np.where(far, sampler.peak, -1.0)))
-        best = (float(sampler.peak[i]), float(x_eval[i, 0]), float(x_eval[i, 2]))
+        i = int(np.argmax(np.where(far, peak, -1.0)))
+        best = (float(peak[i]), float(x_eval[i, 0]), float(x_eval[i, 2]))
     if world > 1:
         import torch.distributed as dist
 

@@ -78,6 +78,7 @@ def _sigs():
         "fus_geometry": [P, P, P, P, P, P, L, I, P],
         "fus_facet_geometry": [P, P, P, P, P, P, L, I, P],
         "fus_eval_points": [P, P, P, P, P, L, I, P],
+        "fus_record_points": [P, P, P, P, P, L, I, P, P, L, L, P],
         "fus_stiffness_host": [P, P, L, P, P, P, P, P, P, L, I, I, P],
     }
     return s

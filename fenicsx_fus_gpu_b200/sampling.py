@@ -219,6 +219,17 @@ class PointEvaluator:
                                                 current_stream()), "fus_eval_points")
         return out
 
+    def record(self, u, out, step_dev, step_base, first, rows):
+        """``u`` into row ``step_base + step_dev - first`` of ``out`` (rows, npts), indices read on the
+        device (``step_dev`` may be None); nothing is written when that row is outside
+        ``[0, rows)``.  The sum of ``__call__``: the same bits.  Asynchronous on the current stream."""
+        ud = _lib.dev(u, self.dtype)
+        check(fn("fus_record_points", self.dtype)(
+            ud.ptr, self.dofmap.data_ptr(), self.cells.data_ptr(), self.phi.data_ptr(), out.data_ptr(), self.npts,
+            self.P, None if step_dev is None else step_dev.data_ptr(), step_base.data_ptr(), int(first), int(rows),
+            current_stream()), "fus_record_points")
+        return out
+
     def to_host(self, u):
         """Values as numpy: one launch + one device->host copy of npts values (pinned)."""
         import torch

@@ -64,6 +64,10 @@ from ._lib import FUS_TABLES_RESIDENT, check, current_stream, fn
 # of the range touch no ghost dof (peer-memory halo: the launch waits for the forward exchange only
 # before its remaining, interface, cells)
 Seg = namedtuple("Seg", "kind c0 n g0 ninterior")
+# a point recorder (record_points): the evaluator, its (rows, npts) rows, the window [first, first + rows)
+# of global step indices and the device int64 holding the global index of the call's step 0
+_Recorder = namedtuple("_Recorder", "ev out first rows base")
+_OUTSIDE = -(1 << 62)  # a base step index that puts every step of a run before any window
 KIND_SUFFIX = ("_rect", "_affine", "", "_vertex")  # cell-kernel symbol fus_<form><suffix> per Seg.kind
 
 A_RUNGE = (0.0, 0.5, 0.5, 1.0)
@@ -216,6 +220,8 @@ class _RK4:
         self._graph = None  # [graph of a step with parity 0, with parity 1]
         self._graph_dt = None
         self._graph_tab = None
+        self._graph_rec = None
+        self._rec = None  # _Recorder, or None: no record launch anywhere
         self.graph_error = None
         self._opened = False
         self._bdofs = None
@@ -553,12 +559,14 @@ class _RK4:
         """The cell kernels of a stage as one group for ``probe``."""
         self._probed(lambda: self._cell_kernels(x, vn, wait))
 
-    def _assemble_exchanged(self, stage, g, dg, use_table, x, vn):
+    def _assemble_exchanged(self, stage, g, dg, use_table, x, vn, record=False):
         """b (, m) of a stage with the halo as blocking rounds: forward exchange of the input, cell
-        kernels, boundary terms, reverse exchange of the sums."""
+        kernels, [the record launch,] boundary terms, reverse exchange of the sums."""
         if self.halo is not None:
             self.halo.forward(x, vn)
         self._assemble(x, vn)
+        if record:
+            self._record(x, use_table)
         self._boundary(stage, g, dg, use_table, vn)
         if self.halo is not None:
             self.halo.reverse(*((self.b, self.m) if self._m_accum else (self.b,)))
@@ -585,15 +593,24 @@ class _RK4:
         that are stream-ordered after kernels of EARLIER phases of this rank, so the step can be
         captured and replayed as a graph without deadlock.  A neighbour's put of stage i+1 is
         issued by the kernel that gathered (and cleared) my ghost sums of stage i, so its FWD epoch
-        also says the ghost accumulators are clean."""
+        also says the ghost accumulators are clean.
+
+        Point recorder (``record_points``): stage 0 records the base ``u``, the state at the start of
+        the step, with one launch after the cell kernels and before the boundary launch.  There its
+        ghost entries are current: the forward exchange (or the wait for the neighbours' puts) came
+        first, and in split modes "two" / "fused" the cell kernels that waited in-kernel precede the
+        record launch on this stream.  And no neighbour can overwrite them yet: a neighbour puts into
+        this rank's ghost slots only from a close that waits for the signal of this rank's stage-0
+        boundary launch, which comes after the record launch."""
         g, dg = self._source_at(stage, dt, t, use_table)
         # stage input: the base state itself in stage 0 (a_0 = 0), un / vn (= ku) afterwards; with the
         # peer-memory halo it is on its way to (or already in) the ghost slots: put there by
         # begin_steps() or by the previous stage's close of the shared dofs
         x, vn = base if stage == 0 else (self.un, self.ku)
+        record = stage == 0 and self._rec is not None
         h = self.halo
         if not self.p2p:
-            self._assemble_exchanged(stage, g, dg, use_table, x, vn)
+            self._assemble_exchanged(stage, g, dg, use_table, x, vn, record)
             self._close(stage, dt, use_table, base, acc)
             return
         # (the leapfrog step always waits before its launches)
@@ -603,6 +620,8 @@ class _RK4:
         else:
             h.wait_forward()
         self._assemble(x, vn, wait=in_kernel)
+        if record:
+            self._record(x, use_table)
         self._boundary(stage, g, dg, use_table, vn, signal=True, consume=in_kernel)
         h.fork()
         with h.side():
@@ -658,7 +677,49 @@ class _RK4:
             self.halo.handle, self._close_variant, 1, 1, u, v, u0, v0, ku, un, self.b.data_ptr(),
             *(self._ptr(t) for t in self._masses()), bdt, adt, mode, current_stream()), "fus_rk_close_shared")
 
+    def _record(self, u, use_table):
+        """The record launch: ``u`` into the recorder's row of global step ``base + step_dev`` (without
+        the table: ``base``)."""
+        r = self._rec
+        r.ev.record(u, r.out, self.step_dev if use_table else None, r.base, r.first, r.rows)
+
+    def _record_last(self):
+        """After a call: one eager record of the state after its last step, when that row is in the
+        window.  The ghost entries of ``u`` are current: with the peer-memory halo ``end_steps`` has
+        waited for the neighbours' puts; the NCCL-shaped halo exchanges ``u`` forward here (every rank
+        must then record the same window: the exchange is collective)."""
+        r = self._rec
+        if r is None or not 0 <= self.nstep - r.first < r.rows:
+            return
+        if self.halo is not None and not self.p2p:
+            self.halo.forward(self.u)
+        r.base.fill_(self.nstep)
+        self._record(self.u, False)
+
     # ---- public --------------------------------------------------------------
+    def record_points(self, evaluator, first=0, rows=1):
+        """Record ``u`` at the points of ``evaluator`` (``sampling.PointEvaluator``) at every step,
+        inside the captured step graphs: returns a device tensor ``(rows, evaluator.npts)`` of the
+        solver's float type, filled with NaN, whose row ``j`` receives ``u`` after ``first + j`` steps
+        counted from ``init()`` (``nstep``).  After any ``rk4`` / ``step_eager`` call every row with
+        ``first + j <= nstep`` is filled, bit-identical to ``evaluator(u)`` on the same state.
+        ``record_points(None)`` detaches the recorder; ``init()`` keeps it and its rows.  With a halo,
+        every rank attaches a recorder with the same window (its own points, possibly none)."""
+        if evaluator is None:
+            self._rec = None
+            return None
+        torch = _torch()
+        first, rows = int(first), int(rows)
+        if np.dtype(evaluator.dtype) != self.dtype:
+            raise ValueError(f"record_points: the evaluator is {np.dtype(evaluator.dtype)}, the solver {self.dtype}")
+        if int(evaluator.P) != self.P:
+            raise ValueError(f"record_points: the evaluator has degree {evaluator.P}, the solver {self.P}")
+        if first < 0 or rows < 1:
+            raise ValueError(f"record_points: need first >= 0 and rows >= 1, got first = {first}, rows = {rows}")
+        out = torch.full((rows, evaluator.npts), float("nan"), dtype=self.T, device="cuda")
+        self._rec = _Recorder(evaluator, out, first, rows, torch.zeros(1, dtype=torch.int64, device="cuda"))
+        return out
+
     def init(self):
         """Zero initial state (cpp/common/Linear.hpp:146-154)."""
         for t in (*self._uv[0], *self._uv[1], self.ku, self.un, self.b):
@@ -717,9 +778,12 @@ class _RK4:
             return self.t
         self._load_table(self.source_table(self.t, dt, nsteps))
         self.step_dev.zero_()
+        if self.use_graph and (self._graph_dt != dt or self._graph_tab != self.gtab.data_ptr()
+                               or self._graph_rec is not self._rec):
+            self._capture(dt)
+        if self._rec is not None:
+            self._rec.base.fill_(self.nstep)  # stream-ordered: the graphs' arguments stay as captured
         if self.use_graph:
-            if self._graph_dt != dt or self._graph_tab != self.gtab.data_ptr():
-                self._capture(dt)
             self.begin_steps()
             for _ in range(nsteps):
                 self._replay_step(dt)
@@ -733,6 +797,7 @@ class _RK4:
         for _ in range(nsteps):
             self.t += dt
         self.nstep += nsteps
+        self._record_last()
         return self.t
 
     def _load_table(self, tab):
@@ -752,12 +817,15 @@ class _RK4:
             self._open_first()
         if self.num_elements is not None:
             self._load_eager_row(self.t, dt)
+        if self._rec is not None:
+            self._rec.base.fill_(self.nstep)
         self.begin_steps()
         self._enqueue_step(dt, self.t, False)
         self._parity ^= 1
         self.end_steps()
         self.t += dt
         self.nstep += 1
+        self._record_last()
         return self.t
 
     def _replay_step(self, dt):
@@ -779,6 +847,8 @@ class _RK4:
         # warm up outside capture (lazy NCCL communicators, module loading)
         saved = [t.clone() for t in self._state()]
         step0 = self.step_dev.clone()
+        if self._rec is not None:
+            self._rec.base.fill_(_OUTSIDE)  # the warm-up steps record no row (rk4 sets the base next)
         self.begin_steps()
         for parity in (self._parity, 1 - self._parity):  # both buffer roles, each step feeding the next
             self._enqueue_step(dt, 0.0, True, parity)
@@ -789,7 +859,7 @@ class _RK4:
         self.step_dev.copy_(step0)
         if self.p2p:
             self.halo.barrier()  # every rank has restored its ghost slots before anyone's next put
-        self._graph_dt, self._graph_tab = dt, self.gtab.data_ptr()
+        self._graph_dt, self._graph_tab, self._graph_rec = dt, self.gtab.data_ptr(), self._rec
         try:
             graphs = []
             for parity in (0, 1):  # base / accumulator buffers swap roles every step

@@ -593,6 +593,19 @@ int fus_eval_points_f64(const double* u, const int32_t* dofmap, const int32_t* c
 int fus_eval_points_f32(const float* u, const int32_t* dofmap, const int32_t* cells,
                         const float* phi, float* out, int64_t npts, int P, void* stream);
 
+/* The same sum, as one row of a recording in out (rows, npts): out[row * npts + p] with
+ * row = *step_base + (step_dev ? *step_dev : 0) - first, read on the device, so a launch captured
+ * in a CUDA graph fills the right row at every replay; a row outside [0, rows) writes nothing.
+ * Bit-identical to fus_eval_points_* on the same vector.  npts < 0, rows < 1, first < 0, a degree
+ * outside 1..15 and (npts > 0) null u, dofmap, cells, phi, out or step_base are rejected before any
+ * launch; npts == 0 launches nothing. */
+int fus_record_points_f64(const double* u, const int32_t* dofmap, const int32_t* cells,
+                          const double* phi, double* out, int64_t npts, int P, const int64_t* step_dev,
+                          const int64_t* step_base, int64_t first, int64_t rows, void* stream);
+int fus_record_points_f32(const float* u, const int32_t* dofmap, const int32_t* cells,
+                          const float* phi, float* out, int64_t npts, int P, const int64_t* step_dev,
+                          const int64_t* step_base, int64_t first, int64_t rows, void* stream);
+
 /* --------------------------------------------------------------------- *
  * Host-buffer entry points (the end-to-end path: host <-> device copies are
  * inside the call).  x_host / y_host are HOST pointers (pinned for full
