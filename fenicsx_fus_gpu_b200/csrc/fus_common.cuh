@@ -29,12 +29,6 @@ int fus_num_sms();
 struct FusHaloDev;
 bool fus_take_armed_wait(const FusHaloDev** h, long long* first_interface_cell);
 
-// stiffness_affine.cu keeps its own copy of the derivative tables (fus_set_dphi_* fills both)
-int fus_affine_set_dphi_f64(int P, const double* dphi, void* stream);
-int fus_affine_set_dphi_f32(int P, const float* dphi, void* stream);
-int fus_vertex_set_dphi_f64(int P, const double* dphi, void* stream);  // stiffness_vertex.cu's copy
-int fus_vertex_set_dphi_f32(int P, const float* dphi, void* stream);
-
 // ---- device-side PTX wrappers ---------------------------------------------
 #ifdef __CUDACC__
 

@@ -40,45 +40,12 @@
 
 #include "stiffness_kernel.cuh"
 
-namespace {
-
 template <typename T>
-int stiffness_entry(const T* xa, const T* ca, const T* xb, const T* cb, T* y, const T* G,
-                    const int32_t* dofmap, const T* dphi, int64_t ncells, int P, int flags,
-                    void* stream, int mode, const T* detJ = nullptr, const T* cm = nullptr,
-                    const T* cy = nullptr, T* m = nullptr) {
-  if (ncells < 0) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness: ncells < 0");
-  if (P < 2 || P > 7) return fus_set_error(FUS_ERR_BAD_DEGREE, "stiffness: degree must be 2..7");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (!(flags & FUS_TABLES_RESIDENT)) {
-    int rc = set_dphi<T>(P, dphi, st);
-    if (rc) return rc;
-  }
-  if (ncells == 0) return 0;
-  StiffArgs<T> a;
-  a.xa = xa;
-  a.ca = ca;
-  a.xb = xb;
-  a.cb = cb;
-  a.y = y;
-  a.G = G;
-  a.dofmap = dofmap;
-  a.detJ = detJ;
-  a.cm = cm;
-  a.cy = cy;
-  a.m = m;
-  a.Gc = nullptr;
-  a.wq = nullptr;
-  a.detJc = nullptr;
-  a.ncells = ncells;
-  a.bulk_ok = (reinterpret_cast<uintptr_t>(G) & (2 * sizeof(T) - 1)) == 0;  // 16-byte record loads
-  if (mode == 2) {
-    if (flags & FUS_NO_ATOMICS)
-      return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness_westervelt: FUS_NO_ATOMICS not supported");
-    return launch<T, 2, 0>(a, P, flags, st);
-  }
-  return mode == 1 ? launch<T, 1, 0>(a, P, flags, st) : launch<T, 0, 0>(a, P, flags, st);
-}
+int fus_affine_set_dphi(int P, const T* dphi, cudaStream_t stream);  // stiffness_affine.cu
+template <typename T>
+int fus_vertex_set_dphi(int P, const T* dphi, cudaStream_t stream);  // stiffness_vertex.cu
+
+namespace {
 
 // ---- host-buffer entry point: H2D of x (and y), the action, D2H of y, pipelined -------------
 //
@@ -155,6 +122,11 @@ int stiffness_host(const T* x_host, T* y_host, int64_t nd, T* x_dev, T* y_dev, c
   const int kflags = flags & ~FUS_HOST_Y_ZERO;
   const int Nd = (P + 1) * (P + 1) * (P + 1);
   HostPipe* hp = host_pipe();
+  auto action = [&](long long c0, long long nc, int fl) {  // y_dev += K x_dev on cells [c0, c0 + nc)
+    StiffArgs<T> a{};
+    a.xa = x_dev, a.ca = coeff + c0, a.y = y_dev, a.G = G + c0 * Nd * 6, a.dofmap = dofmap + c0 * Nd, a.ncells = nc;
+    return cell_entry<T, 0, 0>(a, dphi, P, fl, stream, "stiffness_host");
+  };
   // cells per range: even, so that every range's G slice keeps the 16-byte alignment of the base
   long long cpc = ((ncells + kHostChunks - 1) / kHostChunks + 1) / 2 * 2;
   if (hp == nullptr || ncells < 64 * kHostChunks) {
@@ -165,8 +137,7 @@ int stiffness_host(const T* x_host, T* y_host, int64_t nd, T* x_dev, T* y_dev, c
     } else {
       FUS_CUDA(cudaMemcpyAsync(y_dev, y_host, sizeof(T) * nd, cudaMemcpyHostToDevice, st));
     }
-    if (int rc = stiffness_entry<T>(x_dev, coeff, nullptr, nullptr, y_dev, G, dofmap, dphi, ncells, P, kflags, stream, 0))
-      return rc;
+    if (int rc = action(0, ncells, kflags)) return rc;
     FUS_CUDA(cudaMemcpyAsync(y_host, y_dev, sizeof(T) * nd, cudaMemcpyDeviceToHost, st));
     FUS_CUDA(cudaStreamSynchronize(st));
     return 0;
@@ -220,9 +191,7 @@ int stiffness_host(const T* x_host, T* y_host, int64_t nd, T* x_dev, T* y_dev, c
     FUS_CUDA(cudaEventRecord(hp->up[c], hp->in));
     FUS_CUDA(cudaStreamWaitEvent(st, hp->up[c], 0));
     if (nc > 0) {
-      if (int rc = stiffness_entry<T>(x_dev, coeff + c0, nullptr, nullptr, y_dev, G + c0 * (long long)Nd * 6,
-                                      dofmap + c0 * (long long)Nd, dphi, nc, P, kflags | FUS_TABLES_RESIDENT, stream, 0))
-        return rc;
+      if (int rc = action(c0, nc, kflags | FUS_TABLES_RESIDENT)) return rc;
     }
     FUS_CUDA(cudaEventRecord(hp->done[c], st));
     const long long fin = L[c + 1];  // y[0, fin) is final now
@@ -238,70 +207,28 @@ int stiffness_host(const T* x_host, T* y_host, int64_t nd, T* x_dev, T* y_dev, c
   return 0;
 }
 
+// every unit that includes stiffness_kernel.cuh holds its own copy of the derivative table
+template <typename T>
+int set_dphi_all(int P, const T* dphi, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc = set_dphi<T>(P, dphi, st);
+  if (!rc) rc = fus_affine_set_dphi<T>(P, dphi, st);
+  return rc ? rc : fus_vertex_set_dphi<T>(P, dphi, st);
+}
+
 }  // namespace
 
+#define FUS_STREAMED_API(SFX, T)                                                        \
+  FUS_CELL_API(SFX, T, , 0, (const T* G), a.G = G, (const T* G, const T* detJ), a.G = G; a.detJ = detJ) \
+  int fus_set_dphi_##SFX(int P, const T* dphi, void* stream) { return set_dphi_all<T>(P, dphi, stream); } \
+  int fus_stiffness_host_##SFX(const T* x_host, T* y_host, int64_t nd, T* x_dev, T* y_dev, const T* coeff,  \
+                               const T* G, const int32_t* dofmap, const T* dphi, int64_t ncells, int P,     \
+                               int flags, void* stream) {                                                    \
+    return stiffness_host<T>(x_host, y_host, nd, x_dev, y_dev, coeff, G, dofmap, dphi, ncells, P, flags, stream); \
+  }
+
 extern "C" {
-
-int fus_set_dphi_f64(int P, const double* dphi, void* stream) {
-  int rc = set_dphi<double>(P, dphi, static_cast<cudaStream_t>(stream));
-  if (!rc) rc = fus_affine_set_dphi_f64(P, dphi, stream);  // the affine kernels' copy of the table
-  return rc ? rc : fus_vertex_set_dphi_f64(P, dphi, stream);
-}
-int fus_set_dphi_f32(int P, const float* dphi, void* stream) {
-  int rc = set_dphi<float>(P, dphi, static_cast<cudaStream_t>(stream));
-  if (!rc) rc = fus_affine_set_dphi_f32(P, dphi, stream);
-  return rc ? rc : fus_vertex_set_dphi_f32(P, dphi, stream);
-}
-
-int fus_stiffness_f64(const double* x, const double* coeff, double* y, const double* G,
-                      const int32_t* dofmap, const double* dphi, int64_t ncells, int P, int flags,
-                      void* stream) {
-  return stiffness_entry<double>(x, coeff, nullptr, nullptr, y, G, dofmap, dphi, ncells, P, flags,
-                                 stream, 0);
-}
-int fus_stiffness_f32(const float* x, const float* coeff, float* y, const float* G,
-                      const int32_t* dofmap, const float* dphi, int64_t ncells, int P, int flags,
-                      void* stream) {
-  return stiffness_entry<float>(x, coeff, nullptr, nullptr, y, G, dofmap, dphi, ncells, P, flags,
-                                stream, 0);
-}
-int fus_stiffness2_f64(const double* xa, const double* ca, const double* xb, const double* cb,
-                       double* y, const double* G, const int32_t* dofmap, const double* dphi,
-                       int64_t ncells, int P, int flags, void* stream) {
-  return stiffness_entry<double>(xa, ca, xb, cb, y, G, dofmap, dphi, ncells, P, flags, stream, 1);
-}
-int fus_stiffness2_f32(const float* xa, const float* ca, const float* xb, const float* cb, float* y,
-                       const float* G, const int32_t* dofmap, const float* dphi, int64_t ncells,
-                       int P, int flags, void* stream) {
-  return stiffness_entry<float>(xa, ca, xb, cb, y, G, dofmap, dphi, ncells, P, flags, stream, 1);
-}
-
-int fus_stiffness_westervelt_f64(const double* un, const double* c3, const double* vn,
-                                 const double* c4, const double* c2, const double* c5, double* m,
-                                 double* b, const double* G, const double* detJ,
-                                 const int32_t* dofmap, const double* dphi, int64_t ncells, int P,
-                                 int flags, void* stream) {
-  return stiffness_entry<double>(un, c3, vn, c4, b, G, dofmap, dphi, ncells, P, flags, stream, 2, detJ,
-                                 c2, c5, m);
-}
-int fus_stiffness_westervelt_f32(const float* un, const float* c3, const float* vn, const float* c4,
-                                 const float* c2, const float* c5, float* m, float* b,
-                                 const float* G, const float* detJ, const int32_t* dofmap,
-                                 const float* dphi, int64_t ncells, int P, int flags, void* stream) {
-  return stiffness_entry<float>(un, c3, vn, c4, b, G, dofmap, dphi, ncells, P, flags, stream, 2, detJ,
-                                c2, c5, m);
-}
-
-int fus_stiffness_host_f64(const double* x_host, double* y_host, int64_t nd, double* x_dev,
-                           double* y_dev, const double* coeff, const double* G,
-                           const int32_t* dofmap, const double* dphi, int64_t ncells, int P,
-                           int flags, void* stream) {
-  return stiffness_host<double>(x_host, y_host, nd, x_dev, y_dev, coeff, G, dofmap, dphi, ncells, P, flags, stream);
-}
-int fus_stiffness_host_f32(const float* x_host, float* y_host, int64_t nd, float* x_dev,
-                           float* y_dev, const float* coeff, const float* G, const int32_t* dofmap,
-                           const float* dphi, int64_t ncells, int P, int flags, void* stream) {
-  return stiffness_host<float>(x_host, y_host, nd, x_dev, y_dev, coeff, G, dofmap, dphi, ncells, P, flags, stream);
-}
-
+FUS_STREAMED_API(f64, double)
+FUS_STREAMED_API(f32, float)
 }  // extern "C"
+#undef FUS_STREAMED_API

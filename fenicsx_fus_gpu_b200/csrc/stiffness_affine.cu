@@ -29,49 +29,6 @@ int set_rect_tables(int P, const T* k1, const T* w1, cudaStream_t stream) {
   return 0;
 }
 
-// geo: 1 = affine (Gc x wq), 2 = rectilinear (diagonal Gc, tensor-product weights; wq unused)
-template <typename T>
-int affine_entry(const T* xa, const T* ca, const T* xb, const T* cb, T* y, const T* Gc,
-                 const T* wq, const int32_t* dofmap, const T* dphi, int64_t ncells, int P,
-                 int flags, void* stream, int mode, const T* detJc = nullptr,
-                 const T* cm = nullptr, const T* cy = nullptr, T* m = nullptr, int geo = 1) {
-  if (ncells < 0) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness_affine: ncells < 0");
-  if (P < 2 || P > 7) return fus_set_error(FUS_ERR_BAD_DEGREE, "stiffness_affine: degree must be 2..7");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (!(flags & FUS_TABLES_RESIDENT)) {
-    int rc = set_dphi<T>(P, dphi, st);
-    if (rc) return rc;
-  }
-  if (ncells == 0) return 0;
-  if (Gc == nullptr || (geo == 1 && wq == nullptr))
-    return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness_affine: null Gc / wq");
-  StiffArgs<T> a;
-  a.xa = xa;
-  a.ca = ca;
-  a.xb = xb;
-  a.cb = cb;
-  a.y = y;
-  a.G = nullptr;
-  a.dofmap = dofmap;
-  a.detJ = nullptr;
-  a.cm = cm;
-  a.cy = cy;
-  a.m = m;
-  a.Gc = Gc;
-  a.wq = wq;
-  a.detJc = detJc;
-  a.ncells = ncells;
-  a.bulk_ok = 0;
-  if (mode == 2) {
-    if (flags & FUS_NO_ATOMICS)
-      return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness_westervelt_affine: FUS_NO_ATOMICS not supported");
-    if (detJc == nullptr) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness_westervelt_affine: null detJc");
-    return geo == 2 ? launch<T, 2, 2>(a, P, flags, st) : launch<T, 2, 1>(a, P, flags, st);
-  }
-  if (mode == 1) return geo == 2 ? launch<T, 1, 2>(a, P, flags, st) : launch<T, 1, 1>(a, P, flags, st);
-  return geo == 2 ? launch<T, 0, 2>(a, P, flags, st) : launch<T, 0, 1>(a, P, flags, st);
-}
-
 // one CTA per cell: mean of the weight-normalised records and their largest deviation from it
 template <typename T>
 __global__ void compress_geometry_kernel(const T* __restrict__ G, const T* __restrict__ detJ,
@@ -146,44 +103,21 @@ int compress_entry(const T* G, const T* detJ, const T* wq, T* Gc, T* detJc, int3
 
 }  // namespace
 
-int fus_affine_set_dphi_f64(int P, const double* dphi, void* stream) {
-  return set_dphi<double>(P, dphi, static_cast<cudaStream_t>(stream));
-}
-int fus_affine_set_dphi_f32(int P, const float* dphi, void* stream) {
-  return set_dphi<float>(P, dphi, static_cast<cudaStream_t>(stream));
-}
+FUS_CELL_TABLES(affine)
+
+// GEO 1 = affine cells (Gc x wq), GEO 2 = rectilinear cells (diagonal Gc, tensor-product weights
+// from fus_set_rect_tables; no wq)
+#define FUS_AFFINE_API(SFX, T)                                                                      \
+  FUS_CELL_API(SFX, T, _affine, 1, (const T* Gc, const T* wq), a.Gc = Gc; a.wq = wq,                \
+               (const T* Gc, const T* detJc, const T* wq), a.Gc = Gc; a.detJc = detJc; a.wq = wq)   \
+  FUS_CELL_API(SFX, T, _rect, 2, (const T* Gc), a.Gc = Gc, (const T* Gc, const T* detJc),           \
+               a.Gc = Gc; a.detJc = detJc)
 
 extern "C" {
 
-int fus_stiffness_affine_f64(const double* x, const double* coeff, double* y, const double* Gc,
-                             const double* wq, const int32_t* dofmap, const double* dphi,
-                             int64_t ncells, int P, int flags, void* stream) {
-  return affine_entry<double>(x, coeff, nullptr, nullptr, y, Gc, wq, dofmap, dphi, ncells, P, flags,
-                              stream, 0);
-}
-int fus_stiffness_affine_f32(const float* x, const float* coeff, float* y, const float* Gc,
-                             const float* wq, const int32_t* dofmap, const float* dphi,
-                             int64_t ncells, int P, int flags, void* stream) {
-  return affine_entry<float>(x, coeff, nullptr, nullptr, y, Gc, wq, dofmap, dphi, ncells, P, flags,
-                             stream, 0);
-}
-int fus_stiffness_westervelt_affine_f64(const double* un, const double* c3, const double* vn,
-                                        const double* c4, const double* c2, const double* c5,
-                                        double* m, double* b, const double* Gc,
-                                        const double* detJc, const double* wq,
-                                        const int32_t* dofmap, const double* dphi, int64_t ncells,
-                                        int P, int flags, void* stream) {
-  return affine_entry<double>(un, c3, vn, c4, b, Gc, wq, dofmap, dphi, ncells, P, flags, stream, 2,
-                              detJc, c2, c5, m);
-}
-int fus_stiffness_westervelt_affine_f32(const float* un, const float* c3, const float* vn,
-                                        const float* c4, const float* c2, const float* c5, float* m,
-                                        float* b, const float* Gc, const float* detJc,
-                                        const float* wq, const int32_t* dofmap, const float* dphi,
-                                        int64_t ncells, int P, int flags, void* stream) {
-  return affine_entry<float>(un, c3, vn, c4, b, Gc, wq, dofmap, dphi, ncells, P, flags, stream, 2,
-                             detJc, c2, c5, m);
-}
+FUS_AFFINE_API(f64, double)
+FUS_AFFINE_API(f32, float)
+#undef FUS_AFFINE_API
 
 int fus_set_rect_tables_f64(int P, const double* k1, const double* w1, void* stream) {
   return set_rect_tables<double>(P, k1, w1, static_cast<cudaStream_t>(stream));
@@ -191,58 +125,6 @@ int fus_set_rect_tables_f64(int P, const double* k1, const double* w1, void* str
 int fus_set_rect_tables_f32(int P, const float* k1, const float* w1, void* stream) {
   return set_rect_tables<float>(P, k1, w1, static_cast<cudaStream_t>(stream));
 }
-int fus_stiffness_rect_f64(const double* x, const double* coeff, double* y, const double* Gc,
-                           const int32_t* dofmap, const double* dphi, int64_t ncells, int P,
-                           int flags, void* stream) {
-  return affine_entry<double>(x, coeff, nullptr, nullptr, y, Gc, nullptr, dofmap, dphi, ncells, P,
-                              flags, stream, 0, nullptr, nullptr, nullptr, nullptr, 2);
-}
-int fus_stiffness_rect_f32(const float* x, const float* coeff, float* y, const float* Gc,
-                           const int32_t* dofmap, const float* dphi, int64_t ncells, int P, int flags,
-                           void* stream) {
-  return affine_entry<float>(x, coeff, nullptr, nullptr, y, Gc, nullptr, dofmap, dphi, ncells, P, flags,
-                             stream, 0, nullptr, nullptr, nullptr, nullptr, 2);
-}
-int fus_stiffness_westervelt_rect_f64(const double* un, const double* c3, const double* vn,
-                                      const double* c4, const double* c2, const double* c5,
-                                      double* m, double* b, const double* Gc, const double* detJc,
-                                      const int32_t* dofmap, const double* dphi, int64_t ncells,
-                                      int P, int flags, void* stream) {
-  return affine_entry<double>(un, c3, vn, c4, b, Gc, nullptr, dofmap, dphi, ncells, P, flags, stream,
-                              2, detJc, c2, c5, m, 2);
-}
-int fus_stiffness_westervelt_rect_f32(const float* un, const float* c3, const float* vn,
-                                      const float* c4, const float* c2, const float* c5, float* m,
-                                      float* b, const float* Gc, const float* detJc,
-                                      const int32_t* dofmap, const float* dphi, int64_t ncells, int P,
-                                      int flags, void* stream) {
-  return affine_entry<float>(un, c3, vn, c4, b, Gc, nullptr, dofmap, dphi, ncells, P, flags, stream, 2,
-                             detJc, c2, c5, m, 2);
-}
-
-int fus_stiffness2_affine_f64(const double* xa, const double* ca, const double* xb, const double* cb,
-                              double* y, const double* Gc, const double* wq, const int32_t* dofmap,
-                              const double* dphi, int64_t ncells, int P, int flags, void* stream) {
-  return affine_entry<double>(xa, ca, xb, cb, y, Gc, wq, dofmap, dphi, ncells, P, flags, stream, 1);
-}
-int fus_stiffness2_affine_f32(const float* xa, const float* ca, const float* xb, const float* cb,
-                              float* y, const float* Gc, const float* wq, const int32_t* dofmap,
-                              const float* dphi, int64_t ncells, int P, int flags, void* stream) {
-  return affine_entry<float>(xa, ca, xb, cb, y, Gc, wq, dofmap, dphi, ncells, P, flags, stream, 1);
-}
-int fus_stiffness2_rect_f64(const double* xa, const double* ca, const double* xb, const double* cb,
-                            double* y, const double* Gc, const int32_t* dofmap, const double* dphi,
-                            int64_t ncells, int P, int flags, void* stream) {
-  return affine_entry<double>(xa, ca, xb, cb, y, Gc, nullptr, dofmap, dphi, ncells, P, flags, stream,
-                              1, nullptr, nullptr, nullptr, nullptr, 2);
-}
-int fus_stiffness2_rect_f32(const float* xa, const float* ca, const float* xb, const float* cb,
-                            float* y, const float* Gc, const int32_t* dofmap, const float* dphi,
-                            int64_t ncells, int P, int flags, void* stream) {
-  return affine_entry<float>(xa, ca, xb, cb, y, Gc, nullptr, dofmap, dphi, ncells, P, flags, stream, 1,
-                             nullptr, nullptr, nullptr, nullptr, 2);
-}
-
 int fus_compress_geometry_f64(const double* G, const double* detJ, const double* wq, double* Gc,
                               double* detJc, int32_t* affine, int64_t ncells, int nq, double tol,
                               void* stream) {

@@ -1,7 +1,12 @@
-// Shared by stiffness.cu (G streamed through the TMA ring) and stiffness_affine.cu
-// (affine cells, G = wq x Gc): the kernel template, its layouts and launch helpers.
-// Each translation unit gets its own copy of the __constant__ derivative tables.
+// Shared by stiffness.cu (G streamed through the TMA ring), stiffness_affine.cu (affine cells,
+// G = wq x Gc, and rectilinear cells) and stiffness_vertex.cu (trilinear cells, geometry rebuilt
+// from Tc): the kernel template, its layouts, launch helpers, the host entry and the extern "C"
+// symbol table of the cell kernels.  Each translation unit gets its own copy of the __constant__
+// tables (one shared copy would need relocatable device code); FUS_CELL_TABLES defines the setter
+// of a unit's copy of the derivative table, and fus_set_dphi_* (stiffness.cu) calls all three.
 #pragma once
+
+#include <cstdio>
 
 #include "halo_internal.cuh"
 
@@ -832,4 +837,76 @@ int set_dphi(int P, const T* dphi, cudaStream_t stream) {
   return 0;
 }
 
+int cell_error(int code, const char* what, const char* msg) {
+  char buf[96];
+  snprintf(buf, sizeof(buf), "%s: %s", what, msg);
+  return fus_set_error(code, buf);
+}
+
+// The host side of every cell-kernel symbol.  `a` carries the call's pointers and ncells, every
+// other field zero; `what` is the symbol stem the error messages carry.  A null pointer that this
+// (MODE, GEO) reads is rejected here instead of faulting in the kernel.
+template <typename T, int MODE, int GEO>
+int cell_entry(StiffArgs<T> a, const T* dphi, int P, int flags, void* stream, const char* what) {
+  if (a.ncells < 0) return cell_error(FUS_ERR_BAD_ARGUMENT, what, "ncells < 0");
+  if (P < 2 || P > 7) return cell_error(FUS_ERR_BAD_DEGREE, what, "degree must be 2..7");
+  if (MODE == 2 && (flags & FUS_NO_ATOMICS)) return cell_error(FUS_ERR_BAD_ARGUMENT, what, "FUS_NO_ATOMICS not supported");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (!(flags & FUS_TABLES_RESIDENT)) {
+    if (int rc = set_dphi<T>(P, dphi, st)) return rc;
+  }
+  if (a.ncells == 0) return 0;
+  bool ok = a.dofmap && a.xa && a.ca && a.y;
+  if (MODE >= 1) ok = ok && a.xb && a.cb;
+  if (MODE == 2) ok = ok && a.cm && a.cy && a.m;
+  if (GEO == 0) ok = ok && a.G && (MODE < 2 || a.detJ);
+  if (GEO == 1 || GEO == 2) ok = ok && a.Gc && (GEO == 2 || a.wq) && (MODE < 2 || a.detJc);
+  if (GEO == 3) ok = ok && a.Tc;
+  if (!ok) return cell_error(FUS_ERR_BAD_ARGUMENT, what, "null pointer");
+  if (GEO == 0) a.bulk_ok = (reinterpret_cast<uintptr_t>(a.G) & (2 * sizeof(T) - 1)) == 0;  // 16-byte record loads
+  return launch<T, MODE, GEO>(a, P, flags, st);
+}
+
 }  // namespace
+
+// The setter of this unit's copy of the derivative table, fus_<UNIT>_set_dphi<T>, for
+// fus_set_dphi_* (stiffness.cu).  Expanded at namespace scope.
+#define FUS_CELL_TABLES(UNIT)                                                    \
+  template <typename T>                                                          \
+  int fus_##UNIT##_set_dphi(int P, const T* dphi, cudaStream_t stream) {         \
+    return set_dphi<T>(P, dphi, stream);                                         \
+  }                                                                              \
+  template int fus_##UNIT##_set_dphi<double>(int, const double*, cudaStream_t);  \
+  template int fus_##UNIT##_set_dphi<float>(int, const float*, cudaStream_t);
+
+// The three cell forms on one geometry for one float type, fus_stiffness<G>_<SFX>,
+// fus_stiffness2<G>_<SFX> and fus_stiffness_westervelt<G>_<SFX> of include/fus_b200.h.  GP / GW:
+// the geometry parameters of the linear / Westervelt prototypes, parenthesised, in header order;
+// GSET / WSET store them in `a`.  Expanded inside extern "C", once per float type.
+#define FUS_PARAMS(...) __VA_ARGS__
+#define FUS_CELL_API(SFX, T, G, GEO, GP, GSET, GW, WSET)                                                \
+  int fus_stiffness##G##_##SFX(const T* x, const T* coeff, T* y, FUS_PARAMS GP, const int32_t* dofmap, \
+                               const T* dphi, int64_t ncells, int P, int flags, void* stream) {       \
+    StiffArgs<T> a{};                                                                                  \
+    a.xa = x, a.ca = coeff, a.y = y, a.dofmap = dofmap, a.ncells = ncells;                             \
+    GSET;                                                                                              \
+    return cell_entry<T, 0, GEO>(a, dphi, P, flags, stream, "stiffness" #G);                           \
+  }                                                                                                    \
+  int fus_stiffness2##G##_##SFX(const T* xa, const T* ca, const T* xb, const T* cb, T* y,               \
+                                FUS_PARAMS GP, const int32_t* dofmap, const T* dphi, int64_t ncells,   \
+                                int P, int flags, void* stream) {                                      \
+    StiffArgs<T> a{};                                                                                  \
+    a.xa = xa, a.ca = ca, a.xb = xb, a.cb = cb, a.y = y, a.dofmap = dofmap, a.ncells = ncells;         \
+    GSET;                                                                                              \
+    return cell_entry<T, 1, GEO>(a, dphi, P, flags, stream, "stiffness2" #G);                          \
+  }                                                                                                    \
+  int fus_stiffness_westervelt##G##_##SFX(const T* un, const T* c3, const T* vn, const T* c4,           \
+                                          const T* c2, const T* c5, T* m, T* b, FUS_PARAMS GW,         \
+                                          const int32_t* dofmap, const T* dphi, int64_t ncells, int P, \
+                                          int flags, void* stream) {                                   \
+    StiffArgs<T> a{};                                                                                  \
+    a.xa = un, a.ca = c3, a.xb = vn, a.cb = c4, a.cm = c2, a.cy = c5, a.m = m, a.y = b;                \
+    a.dofmap = dofmap, a.ncells = ncells;                                                              \
+    WSET;                                                                                              \
+    return cell_entry<T, 2, GEO>(a, dphi, P, flags, stream, "stiffness_westervelt" #G);                \
+  }

@@ -82,43 +82,6 @@ int set_vertex_tables(int P, const T* x1, const T* w1, cudaStream_t stream) {
   return 0;
 }
 
-template <typename T>
-int vertex_entry(const T* xa, const T* ca, const T* xb, const T* cb, const T* cm, const T* cy, T* m, T* y,
-                 const T* Tc, const int32_t* dofmap, const T* dphi, int64_t ncells, int P, int flags, void* stream,
-                 int mode) {
-  if (ncells < 0) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness_vertex: ncells < 0");
-  if (P < 2 || P > 7) return fus_set_error(FUS_ERR_BAD_DEGREE, "stiffness_vertex: degree must be 2..7");
-  if (mode == 2 && (flags & FUS_NO_ATOMICS))
-    return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness_westervelt_vertex: FUS_NO_ATOMICS not supported");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (!(flags & FUS_TABLES_RESIDENT)) {
-    int rc = set_dphi<T>(P, dphi, st);
-    if (rc) return rc;
-  }
-  if (ncells == 0) return 0;
-  if (Tc == nullptr) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "stiffness_vertex: null Tc");
-  StiffArgs<T> a;
-  a.xa = xa;
-  a.ca = ca;
-  a.xb = xb;
-  a.cb = cb;
-  a.y = y;
-  a.G = nullptr;
-  a.dofmap = dofmap;
-  a.detJ = nullptr;
-  a.cm = cm;
-  a.cy = cy;
-  a.m = m;
-  a.Gc = nullptr;
-  a.wq = nullptr;
-  a.detJc = nullptr;
-  a.Tc = Tc;
-  a.ncells = ncells;
-  a.bulk_ok = 0;
-  if (mode == 2) return launch<T, 2, 3>(a, P, flags, st);
-  return mode == 1 ? launch<T, 1, 3>(a, P, flags, st) : launch<T, 0, 3>(a, P, flags, st);
-}
-
 constexpr int kMassThreads = 256;
 
 // Lumped mass on trilinear cells, one thread per (cell, point):
@@ -184,12 +147,9 @@ int mass_vertex_entry(const T* x, const T* coeff, T* y, const T* Tc, const int32
 
 }  // namespace
 
-int fus_vertex_set_dphi_f64(int P, const double* dphi, void* stream) {
-  return set_dphi<double>(P, dphi, static_cast<cudaStream_t>(stream));
-}
-int fus_vertex_set_dphi_f32(int P, const float* dphi, void* stream) {
-  return set_dphi<float>(P, dphi, static_cast<cudaStream_t>(stream));
-}
+FUS_CELL_TABLES(vertex)
+
+#define FUS_VERTEX_API(SFX, T) FUS_CELL_API(SFX, T, _vertex, 3, (const T* Tc), a.Tc = Tc, (const T* Tc), a.Tc = Tc)
 
 extern "C" {
 
@@ -207,43 +167,9 @@ int fus_set_vertex_tables_f64(int P, const double* x1, const double* w1, void* s
 int fus_set_vertex_tables_f32(int P, const float* x1, const float* w1, void* stream) {
   return set_vertex_tables<float>(P, x1, w1, static_cast<cudaStream_t>(stream));
 }
-int fus_stiffness_vertex_f64(const double* x, const double* coeff, double* y, const double* Tc,
-                             const int32_t* dofmap, const double* dphi, int64_t ncells, int P, int flags,
-                             void* stream) {
-  return vertex_entry<double>(x, coeff, nullptr, nullptr, nullptr, nullptr, nullptr, y, Tc, dofmap, dphi, ncells, P, flags,
-                              stream, 0);
-}
-int fus_stiffness_vertex_f32(const float* x, const float* coeff, float* y, const float* Tc,
-                             const int32_t* dofmap, const float* dphi, int64_t ncells, int P, int flags,
-                             void* stream) {
-  return vertex_entry<float>(x, coeff, nullptr, nullptr, nullptr, nullptr, nullptr, y, Tc, dofmap, dphi, ncells, P, flags,
-                             stream, 0);
-}
-int fus_stiffness2_vertex_f64(const double* xa, const double* ca, const double* xb, const double* cb,
-                              double* y, const double* Tc, const int32_t* dofmap, const double* dphi,
-                              int64_t ncells, int P, int flags, void* stream) {
-  return vertex_entry<double>(xa, ca, xb, cb, nullptr, nullptr, nullptr, y, Tc, dofmap, dphi, ncells, P, flags,
-                              stream, 1);
-}
-int fus_stiffness2_vertex_f32(const float* xa, const float* ca, const float* xb, const float* cb, float* y,
-                              const float* Tc, const int32_t* dofmap, const float* dphi, int64_t ncells,
-                              int P, int flags, void* stream) {
-  return vertex_entry<float>(xa, ca, xb, cb, nullptr, nullptr, nullptr, y, Tc, dofmap, dphi, ncells, P, flags,
-                             stream, 1);
-}
-
-int fus_stiffness_westervelt_vertex_f64(const double* un, const double* c3, const double* vn, const double* c4,
-                                        const double* c2, const double* c5, double* m, double* b, const double* Tc,
-                                        const int32_t* dofmap, const double* dphi, int64_t ncells, int P, int flags,
-                                        void* stream) {
-  return vertex_entry<double>(un, c3, vn, c4, c2, c5, m, b, Tc, dofmap, dphi, ncells, P, flags, stream, 2);
-}
-int fus_stiffness_westervelt_vertex_f32(const float* un, const float* c3, const float* vn, const float* c4,
-                                        const float* c2, const float* c5, float* m, float* b, const float* Tc,
-                                        const int32_t* dofmap, const float* dphi, int64_t ncells, int P, int flags,
-                                        void* stream) {
-  return vertex_entry<float>(un, c3, vn, c4, c2, c5, m, b, Tc, dofmap, dphi, ncells, P, flags, stream, 2);
-}
+FUS_VERTEX_API(f64, double)
+FUS_VERTEX_API(f32, float)
+#undef FUS_VERTEX_API
 int fus_mass_vertex_f64(const double* x, const double* coeff, double* y, const double* Tc, const int32_t* dofmap,
                         int64_t ncells, int P, void* stream) {
   return mass_vertex_entry<double>(x, coeff, y, Tc, dofmap, ncells, P, stream);

@@ -58,16 +58,39 @@ class _Mass(_Kernel):
 mass_operator = _Mass()
 
 
-class _Stiffness(_Kernel):
+class _CellKernel(_Kernel):
+    """What every stiffness kernel checks: the degree and float type up front, and per call the
+    dofmap shape, the sizes of the per-cell arrays and a non-empty launch, in that order."""
+
+    name = ""
+
+    def __init__(self, P: int, float_type):
+        if not 2 <= int(P) <= 7:
+            raise ValueError(f"{self.name}: degree {P} not in 2..7")
+        self.P, self.n, self.float_type = int(P), int(P) + 1, np.dtype(float_type)
+        _lib.sfx(self.float_type)  # validates
+
+    def _dofmap(self, entity_dofmap, sizes):
+        """The dofmap on the device.  ``sizes(ncells)`` lists (ok, message) for the other arrays."""
+        dm = dev(entity_dofmap, np.int32)
+        nd3 = self.n**3
+        if len(dm.shape) != 2 or dm.shape[1] != nd3:
+            raise _lib.FusError(f"{self.name}: dofmap must be (ncells, {nd3}), got {dm.shape}")
+        for ok, msg in sizes(dm.shape[0]):
+            if not ok:
+                raise _lib.FusError(f"{self.name}: {msg}")
+        if dm.shape[0] == 0:
+            raise ValueError(f"{self.name}: zero cells (empty launch)")
+        return dm
+
+
+class _Stiffness(_CellKernel):
     """Sum-factorised stiffness action - cuda/operators.py:87-190."""
 
+    name = "stiffness_operator"
+
     def __init__(self, P: int, float_type, colour_offsets=None):
-        if not 2 <= int(P) <= 7:
-            raise ValueError(f"stiffness_operator: degree {P} not in 2..7")
-        self.P = int(P)
-        self.n = self.P + 1
-        self.float_type = np.dtype(float_type)
-        _lib.sfx(self.float_type)  # validates
+        super().__init__(P, float_type)
         self.flags = 0
         self.colour_offsets = None
         if colour_offsets is not None:
@@ -79,16 +102,9 @@ class _Stiffness(_Kernel):
     def __call__(self, x, entity_constants, y, G_entity, entity_dofmap, dphi):
         T = self.float_type
         xd, yd, cd, gd = dev(x, T), dev(y, T), dev(entity_constants, T), dev(G_entity, T)
-        dm = dev(entity_dofmap, np.int32)
         nd3 = self.n**3
-        if len(dm.shape) != 2 or dm.shape[1] != nd3:
-            raise _lib.FusError(f"stiffness_operator: dofmap must be (ncells, {nd3}), got {dm.shape}")
-        if gd.size != dm.shape[0] * nd3 * 6:
-            raise _lib.FusError("stiffness_operator: G must be (ncells, n^3, 6)")
-        if cd.size != dm.shape[0]:
-            raise _lib.FusError("stiffness_operator: one constant per cell expected")
-        if dm.shape[0] == 0:
-            raise ValueError("stiffness_operator: zero cells (empty launch)")
+        dm = self._dofmap(entity_dofmap, lambda nc: [(gd.size == nc * nd3 * 6, "G must be (ncells, n^3, 6)"),
+                                                     (cd.size == nc, "one constant per cell expected")])
         if isinstance(dphi, np.ndarray):  # host table is fine: it goes to the constant bank
             tab = np.ascontiguousarray(dphi, dtype=T)
             if tab.size != self.n**2:
@@ -131,69 +147,61 @@ def stiffness_operator(P, float_type, colour_offsets=None):
     return _Stiffness(P, float_type, colour_offsets)
 
 
-class _StiffnessAffine(_Kernel):
+class _StiffnessAffine(_CellKernel):
     """The stiffness action on cells with a constant Jacobian: ``G[c, q, :] = weights[q] *
     Gc[c, :]`` (``precompute.compress_geometry``), so only 6 factors per cell are read."""
 
-    def __init__(self, P: int, float_type):
-        if not 2 <= int(P) <= 7:
-            raise ValueError(f"stiffness_operator_affine: degree {P} not in 2..7")
-        self.P, self.n, self.float_type = int(P), int(P) + 1, np.dtype(float_type)
-        _lib.sfx(self.float_type)
+    name = "stiffness_operator_affine"
 
     def __call__(self, x, entity_constants, y, Gc, weights, entity_dofmap, dphi):
         T = self.float_type
         xd, yd, cd, gd, wd = dev(x, T), dev(y, T), dev(entity_constants, T), dev(Gc, T), dev(weights, T)
-        dm = dev(entity_dofmap, np.int32)
         nd3 = self.n**3
-        if len(dm.shape) != 2 or dm.shape[1] != nd3:
-            raise _lib.FusError(f"stiffness_operator_affine: dofmap must be (ncells, {nd3}), got {dm.shape}")
-        if gd.size != dm.shape[0] * 6 or cd.size != dm.shape[0] or wd.size != nd3:
-            raise _lib.FusError("stiffness_operator_affine: Gc (ncells, 6), constants (ncells,), weights (n^3,)")
-        if dm.shape[0] == 0:
-            raise ValueError("stiffness_operator_affine: zero cells (empty launch)")
+        dm = self._dofmap(entity_dofmap, lambda nc: [(gd.size == nc * 6 and cd.size == nc and wd.size == nd3,
+                                                      "Gc (ncells, 6), constants (ncells,), weights (n^3,)")])
         tab = np.ascontiguousarray(dphi, dtype=T) if isinstance(dphi, np.ndarray) else None
         ptr = tab.ctypes.data if tab is not None else dev(dphi, T).ptr
         check(fn("fus_stiffness_affine", T)(xd.ptr, cd.ptr, yd.ptr, gd.ptr, wd.ptr, dm.ptr, ptr, dm.shape[0],
                                             self.P, 0, current_stream()), "fus_stiffness_affine")
 
 
-def rect_tables(dphi_1D, weights, float_type):
+def tensor_tables(dphi_1D, weights, float_type):
     """``(K1, w1)`` for the rectilinear kernels from the 1-D derivative table ``dphi_1D[q, i]``
     and the tensor quadrature weights (n^3,): ``w1`` with ``weights = w1 x w1 x w1`` and
-    ``K1 = D^T diag(w1) D``.  Raises when the weights are not a tensor product."""
+    ``K1 = D^T diag(w1) D``, or None when the weights are not a tensor product."""
     D = np.asarray(dphi_1D, dtype=np.float64)
     n = D.shape[0]
     wq = np.asarray(weights, dtype=np.float64).reshape(n, n, n)
-    w1 = wq.sum(axis=(1, 2)) / wq.sum() ** (2.0 / 3.0)
+    tot = wq.sum()
+    if not tot > 0:
+        return None
+    w1 = wq.sum(axis=(1, 2)) / tot ** (2.0 / 3.0)
     rtol = 1e-12 if np.dtype(float_type) == np.float64 else 1e-5
     if not np.allclose(w1[:, None, None] * w1[None, :, None] * w1[None, None, :], wq, rtol=rtol, atol=0.0):
-        raise ValueError("rect_tables: the quadrature weights are not a tensor product")
+        return None
     k1 = (D.T * w1[None, :]) @ D
     return np.ascontiguousarray(k1, dtype=float_type), np.ascontiguousarray(w1, dtype=float_type)
 
 
-class _StiffnessRect(_Kernel):
+def rect_tables(dphi_1D, weights, float_type):
+    """``tensor_tables``; raises when the weights are not a tensor product."""
+    tabs = tensor_tables(dphi_1D, weights, float_type)
+    if tabs is None:
+        raise ValueError("rect_tables: the quadrature weights are not a tensor product")
+    return tabs
+
+
+class _StiffnessRect(_CellKernel):
     """The stiffness action on rectilinear cells (affine with diagonal ``Gc``): three decoupled
     1-D products with ``K1 = D^T diag(w1) D``.  Same call as ``stiffness_operator_affine``."""
 
-    def __init__(self, P: int, float_type):
-        if not 2 <= int(P) <= 7:
-            raise ValueError(f"stiffness_operator_rect: degree {P} not in 2..7")
-        self.P, self.n, self.float_type = int(P), int(P) + 1, np.dtype(float_type)
-        _lib.sfx(self.float_type)
+    name = "stiffness_operator_rect"
 
     def __call__(self, x, entity_constants, y, Gc, weights, entity_dofmap, dphi):
         T = self.float_type
         xd, yd, cd, gd = dev(x, T), dev(y, T), dev(entity_constants, T), dev(Gc, T)
-        dm = dev(entity_dofmap, np.int32)
-        nd3 = self.n**3
-        if len(dm.shape) != 2 or dm.shape[1] != nd3:
-            raise _lib.FusError(f"stiffness_operator_rect: dofmap must be (ncells, {nd3}), got {dm.shape}")
-        if gd.size != dm.shape[0] * 6 or cd.size != dm.shape[0]:
-            raise _lib.FusError("stiffness_operator_rect: Gc (ncells, 6), constants (ncells,)")
-        if dm.shape[0] == 0:
-            raise ValueError("stiffness_operator_rect: zero cells (empty launch)")
+        dm = self._dofmap(entity_dofmap, lambda nc: [(gd.size == nc * 6 and cd.size == nc,
+                                                      "Gc (ncells, 6), constants (ncells,)")])
         if not isinstance(dphi, np.ndarray) or not isinstance(weights, np.ndarray):
             raise _lib.FusError("stiffness_operator_rect: dphi and weights are host tables (numpy)")
         k1, w1 = rect_tables(dphi, weights, T)
@@ -209,28 +217,18 @@ def stiffness_operator_rect(P, float_type):
     return _StiffnessRect(P, float_type)
 
 
-class _StiffnessVertex(_Kernel):
+class _StiffnessVertex(_CellKernel):
     """The stiffness action with the geometric factors recomputed in the kernel from the cells'
     trilinear maps (``csrc/stiffness_vertex.cu``): ``Tc`` from ``precompute.trilinear_coefficients``
     takes the place of the ``G`` table - 36 values per cell instead of 6 n^3."""
 
-    def __init__(self, P: int, float_type):
-        if not 2 <= int(P) <= 7:
-            raise ValueError(f"stiffness_operator_vertex: degree {P} not in 2..7")
-        self.P, self.n, self.float_type = int(P), int(P) + 1, np.dtype(float_type)
-        _lib.sfx(self.float_type)
+    name = "stiffness_operator_vertex"
 
     def __call__(self, x, entity_constants, y, Tc, points_1d, weights_1d, entity_dofmap, dphi):
         T = self.float_type
         xd, yd, cd, td = dev(x, T), dev(y, T), dev(entity_constants, T), dev(Tc, T)
-        dm = dev(entity_dofmap, np.int32)
-        nd3 = self.n**3
-        if len(dm.shape) != 2 or dm.shape[1] != nd3:
-            raise _lib.FusError(f"stiffness_operator_vertex: dofmap must be (ncells, {nd3}), got {dm.shape}")
-        if td.size != dm.shape[0] * 36 or cd.size != dm.shape[0]:
-            raise _lib.FusError("stiffness_operator_vertex: Tc (ncells, 36), constants (ncells,)")
-        if dm.shape[0] == 0:
-            raise ValueError("stiffness_operator_vertex: zero cells (empty launch)")
+        dm = self._dofmap(entity_dofmap, lambda nc: [(td.size == nc * 36 and cd.size == nc,
+                                                      "Tc (ncells, 36), constants (ncells,)")])
         tabs = []
         for name, a, size in (("dphi", dphi, self.n * self.n), ("points_1d", points_1d, self.n),
                               ("weights_1d", weights_1d, self.n)):

@@ -57,6 +57,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import FUS_TABLES_RESIDENT, check, current_stream, fn
+from .operators import tensor_tables
 
 # a contiguous range of (permuted) cells that one kernel launch covers:
 # kind 0 rectilinear, 1 affine, 2 streamed G, 3 trilinear (geometry rebuilt from Tc); c0/n cell range;
@@ -279,20 +280,6 @@ class _RK4:
             check(fn("fus_set_vertex_tables", self.dtype)(self.P, x1.ctypes.data, w1.ctypes.data, current_stream()),
                   "fus_set_vertex_tables")
 
-    def _tensor_weights(self):
-        """1-D weights w1 with weights[i n^2 + j n + k] = w1[i] w1[j] w1[k], or None when the rule
-        is not a tensor product (then no cell takes the rectilinear path)."""
-        n = self.n
-        wq = self._weights.cpu().numpy().astype(np.float64).reshape(n, n, n)
-        tot = wq.sum()
-        if not tot > 0:
-            return None
-        w1 = wq.sum(axis=(1, 2)) / tot ** (2.0 / 3.0)
-        rtol = 1e-12 if self.dtype == np.float64 else 1e-5
-        if not np.allclose(w1[:, None, None] * w1[None, :, None] * w1[None, None, :], wq, rtol=rtol, atol=0.0):
-            return None
-        return w1
-
     def _mass(self, x, coeff, y, detJ, dofmap):
         if dofmap.shape[0]:
             check(fn("fus_mass", self.dtype)(x.data_ptr(), coeff.data_ptr(), y.data_ptr(), detJ.data_ptr(),
@@ -400,19 +387,18 @@ class _RK4:
             else:
                 affine, Gc, detJc = pre.compress_geometry(self.G, detJ, self._weights)
             # rectilinear = affine with a diagonal Gc (off-diagonal factors at rounding-noise level)
-            w1 = self._tensor_weights()
+            # no cell takes the rectilinear path unless the rule is a tensor product
+            tabs = tensor_tables(self._dphi_host, self._weights.cpu().numpy(), self.dtype)
             tol = 2048.0 * float(np.finfo(self.dtype).eps)
             diag = Gc[:, [0, 3, 5]].abs().amax(dim=1)
             off = Gc[:, [1, 2, 4]].abs().amax(dim=1)
-            rect = (affine > 0) & (off <= tol * diag) if w1 is not None else torch.zeros_like(affine, dtype=torch.bool)
+            rect = (affine > 0) & (off <= tol * diag) if tabs is not None else torch.zeros_like(affine, dtype=torch.bool)
             kind = torch.where(rect, 0, torch.where(affine > 0, 1, other)).to(torch.int32)
             self.naff = int((kind < 2).sum().item())
             self.ntri = int((kind == 3).sum().item())
             self.nrect = int((kind == 0).sum().item())
             if self.nrect:
-                D = self._dphi_host.astype(np.float64)
-                k1 = np.ascontiguousarray((D.T * w1[None, :]) @ D, dtype=self.dtype)  # K1 = D^T diag(w1) D
-                self._rect_tables = (k1, np.ascontiguousarray(w1, dtype=self.dtype))
+                self._rect_tables = tabs
         split = self.p2p and self.split_cells
         if split:
             iface = (self.dofmap >= self.halo.N).any(dim=1)

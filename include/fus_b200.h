@@ -37,7 +37,9 @@ extern "C" {
 #define FUS_ERR_BAD_ARGUMENT 100002
 #define FUS_ERR_HALO_TIMEOUT 100003
 
-/* flags for fus_stiffness* */
+/* flags for fus_stiffness*.  Every cell-kernel call (fus_stiffness{,2,_westervelt}{,_affine,_rect,_vertex}_*)
+ * checks, in this order: ncells >= 0, 2 <= P <= 7, no FUS_NO_ATOMICS on a Westervelt form, the table upload,
+ * then, for ncells > 0, that no pointer it reads is null (FUS_ERR_BAD_ARGUMENT); zero cells launch nothing. */
 #define FUS_TABLES_RESIDENT 1 /* dphi for this (P, type) already uploaded: skip the table copy */
 #define FUS_NO_ATOMICS 2      /* caller guarantees no two cells of this launch share a dof (colouring) */
 #define FUS_HOST_Y_ZERO 4     /* fus_stiffness_host_*: y_host holds zeros - skip its upload, clear y on the device */

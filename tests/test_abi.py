@@ -69,6 +69,45 @@ def test_error_reporting_without_gpu():
     assert lib.fus_compress_geometry_f32(None, None, None, None, None, None, 4, 0, 1e-6, None) == 100002
 
 
+def _cell_kernel_params():
+    """symbol -> parameter names of every cell-kernel prototype (fus_stiffness{,2,_westervelt}{,_affine,
+    _rect,_vertex}_{f64,f32})."""
+    src = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "fus_b200.h")).read(), flags=re.S)
+    protos = dict(re.findall(r"\b(fus_stiffness(?:2|_westervelt)?(?:_affine|_rect|_vertex)?_f(?:64|32))\s*\(([^)]*)\)\s*;",
+                             src))
+    return {name: [re.findall(r"\w+", p)[-1] for p in args.split(",")] for name, args in protos.items()}
+
+
+def test_cell_kernels_validate_arguments_without_gpu():
+    """Every cell-kernel symbol checks its arguments in one order before any launch: negative ncells,
+    the degree, zero cells (no launch even with null pointers), then every pointer the form and its
+    geometry read - a null one is FUS_ERR_BAD_ARGUMENT instead of a fault in the kernel."""
+    lib = _lib.lib()
+    params = _cell_kernel_params()
+    assert len(params) == 24
+    fake = 256  # never dereferenced: each call below has a null pointer and returns before any CUDA call
+    for name, names in params.items():
+        f = getattr(lib, name)
+        ptrs = [p for p in names if p not in ("dphi", "ncells", "P", "flags", "stream")]
+        assert "dofmap" in ptrs and len(ptrs) == len(names) - 5, (name, names)
+
+        def call(null=(), ncells=5, P=4, flags=_lib.FUS_TABLES_RESIDENT):
+            vals = {p: (None if p in null else fake) for p in ptrs}
+            vals.update(dphi=None, ncells=ncells, P=P, flags=flags, stream=None)
+            return f(*(vals[p] for p in names))
+
+        assert call(ptrs, P=9, flags=0) == 100001, name
+        assert b"degree" in lib.fus_last_error()
+        assert call(ptrs, ncells=-1) == 100002, name
+        assert call(ptrs, ncells=0) == 0, name
+        for p in ptrs:
+            assert call((p,)) == 100002, (name, p)
+            assert b"null" in lib.fus_last_error(), (name, p)
+            assert lib.fus_last_error().startswith(name[4:-4].encode() + b":"), (name, lib.fus_last_error())
+        if "westervelt" in name:
+            assert call(ptrs, ncells=0, flags=_lib.FUS_TABLES_RESIDENT | _lib.FUS_NO_ATOMICS) == 100002, name
+
+
 def test_product_never_imports_oracle():
     """oracle/ is test infrastructure: nothing in the package may reference it."""
     pkg = os.path.join(ROOT, "fenicsx_fus_gpu_b200")

@@ -141,6 +141,24 @@ def test_rect_stiffness_vs_oracle(P, tag):
         ops.rect_tables(tb.dphi_1D, rng.uniform(1, 2, n**3), dt)  # not a tensor-product rule
 
 
+@pytest.mark.parametrize("P", range(2, 8))
+@pytest.mark.parametrize("tag", ["f64", "f32"])
+def test_solver_rect_tables_match_operator(P, tag):
+    """The (K1, w1) a geometry='auto' solver uploads for its rectilinear cells are bit for bit those
+    of ``operators.rect_tables`` on the weights and derivative table in the solver's float type."""
+    import problems
+    import test_gpu_solver as tgs
+    from fenicsx_fus_gpu_b200 import operators as ops
+
+    dtt = np.float64 if tag == "f64" else np.float32
+    dd = problems.linear_problem(P, 2, 0.01, dtt, perturb=0.0)  # axis-aligned: every cell rectilinear
+    s = tgs._linear_solver(dd, dtt, geometry="auto", weights=dd.tb.wts, use_graph=False)
+    assert s.nrect == s.ncells > 0
+    k1, w1 = ops.rect_tables(np.asarray(dd.tb.dphi_1D, dtt), np.asarray(dd.tb.wts, dtt), dtt)
+    for got, want in zip(s._rect_tables, (k1, w1)):
+        assert got.dtype == want.dtype == dtt and got.tobytes() == want.tobytes()
+
+
 @pytest.mark.parametrize("P,N,tag,jitter,shear", [(4, 5, "f64", None, True), (4, 5, "f64", 0.5, True),
                                                   (3, 6, "f32", 0.5, True), (5, 3, "f64", 0.4, True),
                                                   (2, 7, "f64", 1.1, True), (4, 5, "f64", None, False),

@@ -384,3 +384,22 @@ def test_partition_properties_on_random_grids():
             dest = p.index_map.index_to_dest_ranks()
             for i in range(p.index_map.size_local):
                 assert set(int(r) for r in dest.links(i)) == ghosted_by.get((p.rank, i), set())
+
+
+@pytest.mark.parametrize("dt", [np.float64, np.float32])
+def test_tensor_tables(dt):
+    """(K1, w1) of a tensor-product rule; None (rect_tables: ValueError) for any other weights."""
+    from fenicsx_fus_gpu_b200 import operators as ops
+
+    tb = S.element_tables(4, "basix", dt)
+    k1, w1 = ops.tensor_tables(tb.dphi_1D, tb.wts, dt)
+    assert k1.dtype == w1.dtype == dt and k1.shape == (5, 5)
+    tol = 1e-12 if dt == np.float64 else 1e-5
+    np.testing.assert_allclose(np.einsum("i,j,k->ijk", w1, w1, w1).ravel(), tb.wts, rtol=tol)
+    np.testing.assert_allclose(k1, k1.T, rtol=tol, atol=tol)
+    np.testing.assert_allclose(k1.sum(axis=1), 0.0, atol=100 * tol)  # K1 annihilates constants
+    rng = np.random.default_rng(0)
+    for w in (rng.uniform(1, 2, 125), np.zeros(125), -np.asarray(tb.wts)):
+        assert ops.tensor_tables(tb.dphi_1D, w, dt) is None
+        with pytest.raises(ValueError):
+            ops.rect_tables(tb.dphi_1D, w, dt)
