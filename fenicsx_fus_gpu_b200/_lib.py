@@ -79,6 +79,8 @@ def _sigs():
         "fus_facet_geometry": [P, P, P, P, P, P, L, I, P],
         "fus_eval_points": [P, P, P, P, P, L, I, P],
         "fus_record_points": [P, P, P, P, P, L, I, P, P, L, L, P],
+        "fus_eval_elements": [P, P, P, P, P, P, P, L, L, P],
+        "fus_record_elements": [P, P, P, P, P, P, P, L, L, P, P, L, L, P],
         "fus_stiffness_host": [P, P, L, P, P, P, P, P, P, L, I, I, P],
     }
     return s

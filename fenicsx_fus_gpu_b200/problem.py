@@ -265,30 +265,37 @@ def element_source(base, amplitudes, delays):
     return source
 
 
+def _element_facets(su, facets, predicate, elements):
+    """``(bfacet_dofmap, detJ_f, boundary_data, ids, E)`` of an array's facets: ``elements`` is a
+    ``TileArray`` (the facets outside its aperture are dropped, ``E = tile.E``) or one element index
+    per row of the facet group (``E`` None: the caller decides)."""
+    tile = elements if isinstance(elements, TileArray) else None
+    if tile is not None:
+        pred = predicate
+        predicate = lambda cen: (tile.element_of(cen) >= 0) & (  # noqa: E731
+            True if pred is None else np.asarray(pred(cen), bool))
+    fd, dJ, bd = facet_group(su, facets, predicate)
+    if tile is None:
+        return fd, dJ, bd, np.asarray(elements, dtype=np.int64).reshape(-1), None
+    ids = tile.element_of(facet_centroids(su.mesh, bd))
+    if (ids < 0).any():  # DOLFINx rows given directly: keep those inside the aperture
+        keep = np.flatnonzero(ids >= 0)
+        fd, dJ, bd, ids = fd[_d(keep)], dJ[_d(keep)], bd[keep], ids[keep]
+    return fd, dJ, bd, ids, tile.E
+
+
 def _array_source(su, source_facets, source_predicate, base, kw, source_elements, element_amplitudes,
                   element_delays):
     """The source facet group and the solver keywords of a single or a phased-array source.
     ``source_elements``: a ``TileArray`` (the facets outside its aperture are dropped), or one
     element index per row of the source facet group."""
-    tile = source_elements if isinstance(source_elements, TileArray) else None
-    if tile is not None:
-        pred = source_predicate
-        source_predicate = lambda cen: (tile.element_of(cen) >= 0) & (  # noqa: E731
-            True if pred is None else np.asarray(pred(cen), bool))
-    fd1, dJ1, bd1 = facet_group(su, source_facets, source_predicate)
     if source_elements is None:
         if element_amplitudes is not None or element_delays is not None:
             raise ValueError("element_amplitudes / element_delays need source_elements")
         kw["source"] = base
-        return fd1, dJ1, bd1
-    if tile is not None:
-        ids = tile.element_of(facet_centroids(su.mesh, bd1))
-        if (ids < 0).any():  # DOLFINx rows given directly: keep those inside the aperture
-            keep = np.flatnonzero(ids >= 0)
-            fd1, dJ1, bd1, ids = fd1[_d(keep)], dJ1[_d(keep)], bd1[keep], ids[keep]
-        E = tile.E
-    else:
-        ids = np.asarray(source_elements, dtype=np.int64).reshape(-1)
+        return facet_group(su, source_facets, source_predicate)
+    fd1, dJ1, bd1, ids, E = _element_facets(su, source_facets, source_predicate, source_elements)
+    if E is None:
         E = next((len(a) for a in (element_amplitudes, element_delays) if a is not None), None)
     if E is None:
         E = int(ids.max()) + 1 if ids.size else 1
@@ -298,6 +305,25 @@ def _array_source(su, source_facets, source_predicate, base, kw, source_elements
         raise ValueError(f"element_amplitudes and element_delays must have shape ({E},)")
     kw.update(source=element_source(base, A, tau), source_elements=ids, num_elements=E)
     return fd1, dJ1, bd1
+
+
+def element_receiver(su: Setup, facets, elements, predicate=None, num_elements=None):
+    """``sampling.ElementReceiver`` of an array on the exterior facets ``facets`` (as for
+    ``facet_group``), optionally filtered by ``predicate``.  ``elements`` is a ``TileArray`` (the
+    facets outside its aperture are dropped; ``E = tile.E`` on every rank) or one element index per
+    row of the facet group, with ``E = num_elements`` (default: the largest index + 1; give it on
+    every rank of a partitioned run).  The facets and element assignment of the solvers'
+    ``source_elements`` with the same arguments: an array receives on the facets it transmits from."""
+    from .sampling import ElementReceiver
+
+    fd, dJ, _, ids, E = _element_facets(su, facets, predicate, elements)
+    if E is None:
+        E = num_elements if num_elements is not None else (int(ids.max()) + 1 if ids.size else None)
+        if E is None:
+            raise ValueError("element_receiver: no facet here: give num_elements")
+    elif num_elements is not None and int(num_elements) != E:
+        raise ValueError(f"element_receiver: the TileArray has {E} elements, num_elements = {num_elements}")
+    return ElementReceiver(su.dtype, fd, dJ, ids, E)
 
 
 def linear_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0=1500.0, f0=0.5e6,

@@ -14,7 +14,10 @@ trees (``cuda/utils.py:117-154`` ``compute_eval_params``).  Here
   cell boxes + a Newton pull-back instead of the DOLFINx tree);
 * ``PointEvaluator`` tabulates the 1-D Lagrange values at the points' reference
   coordinates once and then evaluates ``u`` at all points with one kernel launch
-  (``csrc/sampling.cu``): only the sampled values cross PCIe.
+  (``csrc/sampling.cu``): only the sampled values cross PCIe;
+* ``ElementReceiver`` integrates ``u`` over the facets of each element of a
+  transducer array (the signal each element receives), with two launches and a
+  deterministic reduction.
 
 DOLFINx is absent from this image, so parity with ``Function.eval`` is pinned
 through known answers only (polynomials of degree <= P are reproduced exactly;
@@ -239,3 +242,125 @@ class PointEvaluator:
         self._host.copy_(self(u), non_blocking=True)
         torch.cuda.current_stream().synchronize()
         return self._host.numpy().copy()
+
+
+def reduce_by_key(key, vals):
+    """``(ukey, sums)``: the sorted distinct values of ``key`` (int64 device tensor) and, for every
+    tensor of ``vals`` (one value per entry of ``key``), the sum of its values per key.  Each sum runs
+    in the order of the entries: a stable sort, then one pass per position inside a key (at most one
+    add per key and pass), so no sum depends on the order of atomics."""
+    import torch
+
+    key, order = torch.sort(key, stable=True)
+    vals = [v[order] for v in vals]
+    ukey, inv, counts = torch.unique_consecutive(key, return_inverse=True, return_counts=True)
+    pos = torch.arange(key.numel(), dtype=torch.int64, device=key.device) - (torch.cumsum(counts, 0) - counts)[inv]
+    sums = [torch.zeros(ukey.numel(), dtype=v.dtype, device=v.device) for v in vals]
+    for j in range(int(counts.max().item()) if counts.numel() else 0):
+        sel = pos == j
+        for acc, v in zip(sums, vals):
+            acc.index_add_(0, inv[sel], v[sel])
+    return ukey, sums
+
+
+#: entries per chunk of a receiver's rows: the work of one warp in the first launch
+CHUNK = 256
+
+
+class ElementReceiver:
+    """The signal each element of a transducer array receives: ``r_e = int_{Gamma_e} u dS`` over the
+    facets of element e, on the device.  ``bfacet_dofmap`` (nf, n^2) and ``detJ_f`` (nf, n^2) are a
+    facet group as ``problem.facet_group`` returns it, ``elements`` holds one element index in
+    ``[0, num_elements)`` per facet row.
+
+    The rows are built once: for every element and dof, ``w`` = the sum of ``detJ_f`` over the
+    element's facets that contain the dof (``reduce_by_key``, facet order), element-major and sorted
+    by dof, cut into chunks of ``CHUNK`` entries (``fus_record_elements_*``).  With partitioned meshes
+    each rank integrates over the facets of its own cells: summing ``receiver(u)`` (or ``areas``) over
+    the ranks gives the integral (the area) up to rounding.  A rank without any of the facets gets
+    zeros."""
+
+    def __init__(self, float_type, bfacet_dofmap, detJ_f, elements, num_elements):
+        import torch
+
+        if not torch.cuda.is_available():
+            raise _lib.FusError("no CUDA device: this package has no CPU path")
+        self.dtype = np.dtype(float_type)
+        self.T = torch.float64 if self.dtype == np.float64 else torch.float32
+        self.E = int(num_elements)
+        if self.E < 1:
+            raise ValueError(f"ElementReceiver: num_elements must be >= 1, got {self.E}")
+
+        def dev(a, dt):
+            t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a))
+            return t.to(device="cuda", dtype=dt).contiguous()
+
+        bdm, dJ, ids = dev(bfacet_dofmap, torch.int32), dev(detJ_f, self.T), dev(elements, torch.int64)
+        if bdm.dim() != 2 or tuple(dJ.shape) != tuple(bdm.shape):
+            raise ValueError(f"ElementReceiver: bfacet_dofmap {tuple(bdm.shape)} and detJ_f {tuple(dJ.shape)} must "
+                             "both be (facets, n^2)")
+        nf = int(bdm.shape[0])
+        if ids.dim() != 1 or ids.numel() != nf:
+            raise ValueError(f"ElementReceiver: elements has {ids.numel()} entries, the facet group {nf} rows")
+        if nf:
+            lo, hi = int(ids.min().item()), int(ids.max().item())
+            if lo < 0 or hi >= self.E:
+                raise ValueError(f"ElementReceiver: elements must lie in [0, {self.E}), got [{lo}, {hi}]")
+            if int(bdm.min().item()) < 0:
+                raise ValueError("ElementReceiver: negative dof in bfacet_dofmap")
+        # u must hold every dof the facets touch
+        self.ndofs = int(bdm.max().item()) + 1 if bdm.numel() else 0
+        i64 = dict(dtype=torch.int64, device="cuda")
+        if bdm.numel():
+            key = ids.repeat_interleave(bdm.shape[1]) * self.ndofs + bdm.reshape(-1).to(torch.int64)
+            ukey, (w,) = reduce_by_key(key, [dJ.reshape(-1)])
+        else:
+            ukey, w = torch.zeros(0, **i64), torch.zeros(0, dtype=self.T, device="cuda")
+        nnz = int(ukey.numel())
+        if nnz >= 2**31:
+            raise ValueError(f"ElementReceiver: {nnz} entries do not fit the int32 chunk table")
+        elem = ukey // max(self.ndofs, 1)
+        self.dof = (ukey - elem * self.ndofs).to(torch.int32)
+        self.w = w.contiguous()
+        count = torch.bincount(elem, minlength=self.E)
+        nch = (count + CHUNK - 1) // CHUNK
+        self.elem_chunk = torch.cat([torch.zeros(1, **i64), torch.cumsum(nch, 0)]).to(torch.int32)
+        self.nchunks = int(self.elem_chunk[-1].item())
+        ce = torch.repeat_interleave(torch.arange(self.E, **i64), nch)  # element of every chunk
+        j = torch.arange(self.nchunks, **i64) - self.elem_chunk[:-1].to(torch.int64)[ce]
+        start = torch.cumsum(count, 0) - count
+        self.chunk_beg = torch.cat([start[ce] + j * CHUNK, torch.tensor([nnz], **i64)]).to(torch.int32)
+        self.partial = torch.empty(max(self.nchunks, 1), dtype=self.T, device="cuda")  # scratch of the first launch
+        self.out = torch.zeros(self.E, dtype=self.T, device="cuda")
+        self.areas = self(torch.ones(max(self.ndofs, 1), dtype=self.T, device="cuda")).clone()
+
+    @property
+    def nbytes(self):
+        """Device bytes of the rows, the chunk tables and the scratch."""
+        return sum(t.numel() * t.element_size() for t in (self.dof, self.w, self.elem_chunk, self.chunk_beg,
+                                                          self.partial, self.out))
+
+    def _args(self, u):
+        ud = _lib.dev(u, self.dtype)
+        if ud.size < self.ndofs:
+            raise ValueError(f"ElementReceiver: u has {ud.size} entries, the facets reach dof {self.ndofs - 1}")
+        return (ud.ptr, self.dof.data_ptr(), self.w.data_ptr(), self.chunk_beg.data_ptr(), self.elem_chunk.data_ptr(),
+                self.partial.data_ptr())
+
+    def __call__(self, u, out=None):
+        """Device tensor (E,) of this rank's ``r_e``; asynchronous on the current stream."""
+        out = self.out if out is None else out
+        if self.nchunks == 0:
+            return out.zero_()  # no facet here: this rank's part of every integral is 0
+        check(fn("fus_eval_elements", self.dtype)(*self._args(u), out.data_ptr(), self.nchunks, self.E,
+                                                  current_stream()), "fus_eval_elements")
+        return out
+
+    def record(self, u, out, step_dev, step_base, first, rows):
+        """``r_e`` into row ``step_base + step_dev - first`` of ``out`` (rows, E), indices read on the
+        device (``step_dev`` may be None); nothing is written when that row is outside ``[0, rows)``.
+        The sums of ``__call__``: the same bits.  Asynchronous on the current stream."""
+        check(fn("fus_record_elements", self.dtype)(
+            *self._args(u), out.data_ptr(), self.nchunks, self.E, None if step_dev is None else step_dev.data_ptr(),
+            step_base.data_ptr(), int(first), int(rows), current_stream()), "fus_record_elements")
+        return out

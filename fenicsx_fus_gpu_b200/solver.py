@@ -58,6 +58,7 @@ import numpy as np
 from . import _lib
 from ._lib import FUS_TABLES_RESIDENT, check, current_stream, fn
 from .operators import tensor_tables
+from .sampling import reduce_by_key
 
 # a contiguous range of (permuted) cells that one kernel launch covers:
 # kind 0 rectilinear, 1 affine, 2 streamed G, 3 trilinear (geometry rebuilt from Tc); c0/n cell range;
@@ -65,8 +66,9 @@ from .operators import tensor_tables
 # of the range touch no ghost dof (peer-memory halo: the launch waits for the forward exchange only
 # before its remaining, interface, cells)
 Seg = namedtuple("Seg", "kind c0 n g0 ninterior")
-# a point recorder (record_points): the evaluator, its (rows, npts) rows, the window [first, first + rows)
-# of global step indices and the device int64 holding the global index of the call's step 0
+# a recorder (record_points: a PointEvaluator, record_elements: an ElementReceiver): its rows, the window
+# [first, first + rows) of global step indices and the device int64 holding the global index of the call's
+# step 0
 _Recorder = namedtuple("_Recorder", "ev out first rows base")
 _OUTSIDE = -(1 << 62)  # a base step index that puts every step of a run before any window
 KIND_SUFFIX = ("_rect", "_affine", "", "_vertex")  # cell-kernel symbol fus_<form><suffix> per Seg.kind
@@ -222,7 +224,9 @@ class _RK4:
         self._graph_dt = None
         self._graph_tab = None
         self._graph_rec = None
-        self._rec = None  # _Recorder, or None: no record launch anywhere
+        # "points" / "elements" -> _Recorder (empty: no record launch anywhere).  Replaced, never mutated,
+        # when a recorder is attached or detached, so `is` against _graph_rec tells when to recapture
+        self._recs = {}
         self.graph_error = None
         self._opened = False
         self._bdofs = None
@@ -266,6 +270,11 @@ class _RK4:
     @property
     def v(self):
         return self._uv[self._parity][1]
+
+    @property
+    def _rec(self):
+        """The point recorder, or None."""
+        return self._recs.get("points")
 
     # ---- set-up helpers ------------------------------------------------------
     def _set_tables(self):
@@ -331,8 +340,7 @@ class _RK4:
         (element, w[, w2]) per element whose facets contain it, w = the facet coefficient times
         detJ_f summed over those facets (the facet mass diagonal of the element).  Built on the
         device: the facet rows are expanded into (dof, element, weight) entries, sorted by
-        (dof, element) and reduced per key, one pass per position inside a key, so that the sums
-        run in facet order and do not depend on the order of atomics."""
+        (dof, element) and reduced per key in facet order (``sampling.reduce_by_key``)."""
         torch = _torch()
         E = self.num_elements
         nf = 0 if src is None else int(src[0].shape[0])
@@ -342,16 +350,8 @@ class _RK4:
         if nf:
             bdm, dJ, coeff = src
             key = bdm.reshape(-1).to(torch.int64) * E + self._elem_ids.repeat_interleave(bdm.shape[1])
-            key, order = torch.sort(key, stable=True)
-            vals = [(c[:, None] * dJ).reshape(-1)[order] for c in (coeff, None if src2 is None else src2[2])
-                    if c is not None]
-            ukey, inv, counts = torch.unique_consecutive(key, return_inverse=True, return_counts=True)
-            pos = torch.arange(key.numel(), **i64) - (torch.cumsum(counts, 0) - counts)[inv]
-            sums = [torch.zeros(ukey.numel(), dtype=self.T, device="cuda") for _ in vals]
-            for j in range(int(counts.max().item())):
-                sel = pos == j  # at most one entry per key: each sum gets one add per pass
-                for acc, v in zip(sums, vals):
-                    acc.index_add_(0, inv[sel], v[sel])
+            ukey, sums = reduce_by_key(key, [(c[:, None] * dJ).reshape(-1)
+                                             for c in (coeff, None if src2 is None else src2[2]) if c is not None])
         else:
             ukey, sums = torch.zeros(0, **i64), [torch.zeros(0, dtype=self.T, device="cuda")] * (1 + (src2 is not None))
         row = torch.searchsorted(ukey // E, self._bdofs.to(torch.int64))
@@ -581,8 +581,9 @@ class _RK4:
         issued by the kernel that gathered (and cleared) my ghost sums of stage i, so its FWD epoch
         also says the ghost accumulators are clean.
 
-        Point recorder (``record_points``): stage 0 records the base ``u``, the state at the start of
-        the step, with one launch after the cell kernels and before the boundary launch.  There its
+        Recorders (``record_points``, ``record_elements``): stage 0 records the base ``u``, the state
+        at the start of the step, with the record launches after the cell kernels and before the
+        boundary launch.  There its
         ghost entries are current: the forward exchange (or the wait for the neighbours' puts) came
         first, and in split modes "two" / "fused" the cell kernels that waited in-kernel precede the
         record launch on this stream.  And no neighbour can overwrite them yet: a neighbour puts into
@@ -593,7 +594,7 @@ class _RK4:
         # peer-memory halo it is on its way to (or already in) the ghost slots: put there by
         # begin_steps() or by the previous stage's close of the shared dofs
         x, vn = base if stage == 0 else (self.un, self.ku)
-        record = stage == 0 and self._rec is not None
+        record = stage == 0 and bool(self._recs)
         h = self.halo
         if not self.p2p:
             self._assemble_exchanged(stage, g, dg, use_table, x, vn, record)
@@ -663,24 +664,41 @@ class _RK4:
             self.halo.handle, self._close_variant, 1, 1, u, v, u0, v0, ku, un, self.b.data_ptr(),
             *(self._ptr(t) for t in self._masses()), bdt, adt, mode, current_stream()), "fus_rk_close_shared")
 
-    def _record(self, u, use_table):
-        """The record launch: ``u`` into the recorder's row of global step ``base + step_dev`` (without
-        the table: ``base``)."""
-        r = self._rec
-        r.ev.record(u, r.out, self.step_dev if use_table else None, r.base, r.first, r.rows)
+    def _record(self, u, use_table, recs=None):
+        """The record launches: ``u`` into every recorder's (or every one of ``recs``) row of global step
+        ``base + step_dev`` (without the table: ``base``)."""
+        for r in self._recs.values() if recs is None else recs:
+            r.ev.record(u, r.out, self.step_dev if use_table else None, r.base, r.first, r.rows)
+
+    def _set_bases(self, step):
+        for r in self._recs.values():
+            r.base.fill_(step)
 
     def _record_last(self):
-        """After a call: one eager record of the state after its last step, when that row is in the
-        window.  The ghost entries of ``u`` are current: with the peer-memory halo ``end_steps`` has
-        waited for the neighbours' puts; the NCCL-shaped halo exchanges ``u`` forward here (every rank
-        must then record the same window: the exchange is collective)."""
-        r = self._rec
-        if r is None or not 0 <= self.nstep - r.first < r.rows:
+        """After a call: one eager record of the state after its last step, by every recorder whose
+        window holds that row.  The ghost entries of ``u`` are current: with the peer-memory halo
+        ``end_steps`` has waited for the neighbours' puts; the NCCL-shaped halo exchanges ``u`` forward
+        here, once (every rank must then record the same windows: the exchange is collective)."""
+        due = [r for r in self._recs.values() if 0 <= self.nstep - r.first < r.rows]
+        if not due:
             return
         if self.halo is not None and not self.p2p:
             self.halo.forward(self.u)
-        r.base.fill_(self.nstep)
-        self._record(self.u, False)
+        for r in due:
+            r.base.fill_(self.nstep)
+        self._record(self.u, False, due)
+
+    def _attach(self, kind, ev, first, rows, width, fill):
+        """Attach (``ev`` not None) or detach the recorder of ``kind``; returns its rows."""
+        torch = _torch()
+        if ev is None:
+            if kind in self._recs:
+                self._recs = {k: r for k, r in self._recs.items() if k != kind}
+            return None
+        out = torch.full((rows, width), fill, dtype=self.T, device="cuda")
+        self._recs = {**self._recs, kind: _Recorder(ev, out, first, rows, torch.zeros(1, dtype=torch.int64,
+                                                                                      device="cuda"))}
+        return out
 
     # ---- public --------------------------------------------------------------
     def record_points(self, evaluator, first=0, rows=1):
@@ -692,9 +710,7 @@ class _RK4:
         ``record_points(None)`` detaches the recorder; ``init()`` keeps it and its rows.  With a halo,
         every rank attaches a recorder with the same window (its own points, possibly none)."""
         if evaluator is None:
-            self._rec = None
-            return None
-        torch = _torch()
+            return self._attach("points", None, 0, 1, 0, 0.0)
         first, rows = int(first), int(rows)
         if np.dtype(evaluator.dtype) != self.dtype:
             raise ValueError(f"record_points: the evaluator is {np.dtype(evaluator.dtype)}, the solver {self.dtype}")
@@ -702,9 +718,30 @@ class _RK4:
             raise ValueError(f"record_points: the evaluator has degree {evaluator.P}, the solver {self.P}")
         if first < 0 or rows < 1:
             raise ValueError(f"record_points: need first >= 0 and rows >= 1, got first = {first}, rows = {rows}")
-        out = torch.full((rows, evaluator.npts), float("nan"), dtype=self.T, device="cuda")
-        self._rec = _Recorder(evaluator, out, first, rows, torch.zeros(1, dtype=torch.int64, device="cuda"))
-        return out
+        return self._attach("points", evaluator, first, rows, evaluator.npts, float("nan"))
+
+    def record_elements(self, receiver, first=0, rows=1):
+        """Record what the elements of an array receive (``sampling.ElementReceiver``) at every step,
+        inside the captured step graphs: returns a device tensor ``(rows, receiver.E)`` of the solver's
+        float type, filled with NaN, whose row ``j`` receives this rank's ``r_e`` (the integral of ``u``
+        over element e's facets of this rank) after ``first + j`` steps counted from ``init()``; a rank
+        without any receiver facet gets zeros.  After any ``rk4`` / ``step_eager`` call every row with
+        ``first + j <= nstep`` is filled, bit-identical to ``receiver(u)`` on the same state.
+        ``record_elements(None)`` detaches the receiver; a point recorder may be attached beside it.
+        With a halo, every rank attaches a receiver with the same window and E; the sum over ranks is
+        the caller's (one ``all_reduce`` after the run)."""
+        if receiver is None:
+            return self._attach("elements", None, 0, 1, 0, 0.0)
+        first, rows = int(first), int(rows)
+        if np.dtype(receiver.dtype) != self.dtype:
+            raise ValueError(f"record_elements: the receiver is {np.dtype(receiver.dtype)}, the solver {self.dtype}")
+        if receiver.ndofs > self.ndofs:
+            raise ValueError(f"record_elements: the receiver reaches dof {receiver.ndofs - 1}, the solver has "
+                             f"{self.ndofs} dofs")
+        if first < 0 or rows < 1:
+            raise ValueError(f"record_elements: need first >= 0 and rows >= 1, got first = {first}, rows = {rows}")
+        return self._attach("elements", receiver, first, rows, receiver.E,
+                            float("nan") if receiver.nchunks else 0.0)
 
     def init(self):
         """Zero initial state (cpp/common/Linear.hpp:146-154)."""
@@ -765,10 +802,9 @@ class _RK4:
         self._load_table(self.source_table(self.t, dt, nsteps))
         self.step_dev.zero_()
         if self.use_graph and (self._graph_dt != dt or self._graph_tab != self.gtab.data_ptr()
-                               or self._graph_rec is not self._rec):
+                               or self._graph_rec is not self._recs):
             self._capture(dt)
-        if self._rec is not None:
-            self._rec.base.fill_(self.nstep)  # stream-ordered: the graphs' arguments stay as captured
+        self._set_bases(self.nstep)  # stream-ordered: the graphs' arguments stay as captured
         if self.use_graph:
             self.begin_steps()
             for _ in range(nsteps):
@@ -803,8 +839,7 @@ class _RK4:
             self._open_first()
         if self.num_elements is not None:
             self._load_eager_row(self.t, dt)
-        if self._rec is not None:
-            self._rec.base.fill_(self.nstep)
+        self._set_bases(self.nstep)
         self.begin_steps()
         self._enqueue_step(dt, self.t, False)
         self._parity ^= 1
@@ -833,8 +868,7 @@ class _RK4:
         # warm up outside capture (lazy NCCL communicators, module loading)
         saved = [t.clone() for t in self._state()]
         step0 = self.step_dev.clone()
-        if self._rec is not None:
-            self._rec.base.fill_(_OUTSIDE)  # the warm-up steps record no row (rk4 sets the base next)
+        self._set_bases(_OUTSIDE)  # the warm-up steps record no row (rk4 sets the base next)
         self.begin_steps()
         for parity in (self._parity, 1 - self._parity):  # both buffer roles, each step feeding the next
             self._enqueue_step(dt, 0.0, True, parity)
@@ -845,7 +879,7 @@ class _RK4:
         self.step_dev.copy_(step0)
         if self.p2p:
             self.halo.barrier()  # every rank has restored its ghost slots before anyone's next put
-        self._graph_dt, self._graph_tab, self._graph_rec = dt, self.gtab.data_ptr(), self._rec
+        self._graph_dt, self._graph_tab, self._graph_rec = dt, self.gtab.data_ptr(), self._recs
         try:
             graphs = []
             for parity in (0, 1):  # base / accumulator buffers swap roles every step

@@ -608,6 +608,34 @@ int fus_record_points_f32(const float* u, const int32_t* dofmap, const int32_t* 
                           const float* phi, float* out, int64_t npts, int P, const int64_t* step_dev,
                           const int64_t* step_base, int64_t first, int64_t rows, void* stream);
 
+/* Element receivers: out[e] = sum_k w[k] * u[dof[k]] over the entries k of element e, for the E
+ * elements (this rank's part of the integral of u over the element's facets).  The entries are
+ * element-major and cut into nchunks chunks that do not straddle two elements: chunk c holds
+ * entries [chunk_beg[c], chunk_beg[c + 1]) (nchunks + 1 values), the chunks of element e are
+ * [elem_chunk[e], elem_chunk[e + 1]) (E + 1 values).  Two launches: one warp per chunk writes
+ * partial[c] (nchunks values of scratch), one warp per element sums its partials; both sums run in
+ * an order fixed by the format alone, not by the grid or the device, so results are
+ * bit-reproducible.  fus_eval_elements_* writes out[0 .. E); fus_record_elements_* writes row
+ * row = *step_base + (step_dev ? *step_dev : 0) - first of out (rows, E), read on the device, and
+ * nothing when that row is outside [0, rows) - the same bits as fus_eval_elements_* on the same
+ * vector.  nchunks < 0, E < 0, rows < 1, first < 0 and (E > 0, nchunks > 0) null u, dof, w,
+ * chunk_beg, elem_chunk, partial, out or (record) step_base are rejected before any launch;
+ * E == 0 or nchunks == 0 launches nothing. */
+int fus_eval_elements_f64(const double* u, const int32_t* dof, const double* w, const int32_t* chunk_beg,
+                          const int32_t* elem_chunk, double* partial, double* out, int64_t nchunks, int64_t E,
+                          void* stream);
+int fus_eval_elements_f32(const float* u, const int32_t* dof, const float* w, const int32_t* chunk_beg,
+                          const int32_t* elem_chunk, float* partial, float* out, int64_t nchunks, int64_t E,
+                          void* stream);
+int fus_record_elements_f64(const double* u, const int32_t* dof, const double* w, const int32_t* chunk_beg,
+                            const int32_t* elem_chunk, double* partial, double* out, int64_t nchunks, int64_t E,
+                            const int64_t* step_dev, const int64_t* step_base, int64_t first, int64_t rows,
+                            void* stream);
+int fus_record_elements_f32(const float* u, const int32_t* dof, const float* w, const int32_t* chunk_beg,
+                            const int32_t* elem_chunk, float* partial, float* out, int64_t nchunks, int64_t E,
+                            const int64_t* step_dev, const int64_t* step_base, int64_t first, int64_t rows,
+                            void* stream);
+
 /* --------------------------------------------------------------------- *
  * Host-buffer entry points (the end-to-end path: host <-> device copies are
  * inside the call).  x_host / y_host are HOST pointers (pinned for full
