@@ -36,7 +36,7 @@ def parser(desc, degree, cells):
                          "other cells rebuild their geometry from 36 values instead of streaming it (no per-point "
                          "tables; same results to rounding)")
     ap.add_argument("--integrator", default="rk4", choices=["rk4", "leapfrog"],
-                    help="time integrator of the linear demos: rk4 (the reference's) or leapfrog")
+                    help="time integrator: rk4 (the reference's) or leapfrog (one stiffness action per step)")
     ap.add_argument("--sample-dir", default=None,
                     help="write pressure_field_<k>.txt dumps of the sampling plane here (device-side sampling)")
     return ap

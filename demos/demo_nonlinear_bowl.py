@@ -26,7 +26,8 @@ def main():
     centre = (0.5 * lengths[1], 0.5 * lengths[2])
     solver = problem.westervelt_solver(
         su, source_facets=[2], absorbing_facets=[0, 1, 2, 3, 4, 5], rho=rho, c0=c0, f0=f0, p0=p0, beta=3.5,
-        alpha_dB=0.2, source_predicate=problem.disc(1, 2, centre, 0.3 * lengths[1]), geometry=a.geometry)
+        alpha_dB=0.2, source_predicate=problem.disc(1, 2, centre, 0.3 * lengths[1]), geometry=a.geometry,
+        integrator=a.integrator)
     dt = problem.cfl_time_step(a.degree, h, c0, f0, 0.40)  # :122
     tf = lengths[0] / c0 + 8.0 / f0
     nsteps = a.steps or int(tf / dt) + 1

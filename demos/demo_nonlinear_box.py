@@ -21,7 +21,8 @@ def main():
     lengths = tuple(h * n for n in ncells)
     su = problem.box_setup(a.degree, ncells, lengths, dtype, rank, world, grid=grid, geometry=a.geometry)
     solver = problem.westervelt_solver(su, source_facets=[2], absorbing_facets=[3], rho=rho, c0=c0, f0=f0,
-                                       p0=p0, beta=100.0, alpha_dB=50.0, geometry=a.geometry)
+                                       p0=p0, beta=100.0, alpha_dB=50.0, geometry=a.geometry,
+                                       integrator=a.integrator)
     dt = problem.cfl_time_step(a.degree, h, c0, f0, 0.70)  # :128
     tf = lengths[0] / c0 + 2.0 / f0
     nsteps = a.steps or int(tf / dt) + 1

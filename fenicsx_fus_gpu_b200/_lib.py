@@ -69,6 +69,8 @@ def _sigs():
         "fus_rk_close": [P, P, P, P, P, P, P, P, P, T, T, I, L, P, P, P],
         "fus_rk_close_shared": [P, I, I, I, P, P, P, P, P, P, P, P, P, P, P, T, T, I, P],
         "fus_leapfrog_close": [P, P, P, P, T, T, L, P, P, P],
+        "fus_westervelt_leapfrog_close": [P, P, P, P, P, P, P, P, T, T, T, L, P, P, P],
+        "fus_westervelt_leapfrog_close_shared": [P, I, I, P, P, P, P, P, P, P, P, T, T, T, P],
         "fus_rk_close_westervelt": [P, P, P, P, P, P, P, P, P, P, T, T, I, L, P, P, P],
         "fus_boundary_terms": [P, P, P, P, P, P, T, T, P, P, I, I, L, P],
         "fus_boundary_terms_signal": [P, P, P, P, P, P, P, T, T, P, P, I, I, L, I, P],

@@ -142,6 +142,9 @@ struct CloseArgs {
   // multi-GPU: bit d set <=> dof d is shared with a neighbour and is closed by
   // rk_close_shared_kernel once the reverse halo has landed (null: close everything)
   const unsigned char* skip;
+  // Westervelt leapfrog (WEST == 4) only: the owner-complete absorbing diagonal and the w step
+  const T* absd;
+  T cdt;
 };
 
 // WEST 0: linear (kv = b / m).  WEST 1: m += m0, kv = b / m, m = 0 (the cell-mass pair was
@@ -154,10 +157,33 @@ struct CloseArgs {
 //   v += bdt * b / m ; u += adt_next * v ; b = 0
 // with m = m_lumped - (dt/2) absb, which makes the absorbing term a (v+ + v-)/2 time-centred
 // (second order, unconditionally damping) at no extra cost.  4 reads + 3 writes per dof.
+// WEST 4: a whole LEAPFROG step of the Westervelt equation, pointwise mass form (u at whole steps, v at
+// half steps, w = ku the velocity extrapolated to the whole step, the second cell-kernel operand):
+//   a = (b + m5 w^2 + absd v) / (m + m2 u) ; v += bdt a ; w = v + cdt a ; u += adt_next v ; b = 0
+// with m = m0 - (dt/2) absd in the steps (m0 in the kick-off).  The mass is taken at u^n and the
+// velocity terms at the extrapolated w^n, so the step stays explicit.  8 reads + 4 writes per dof.
 template <typename T, bool VEC, int WEST>
 __device__ __forceinline__ void close_body(const CloseArgs<T>& a, long long k) {
   constexpr int W = VEC ? Vec<T>::W : 1;
   using P = Pack<T, Vec<T>::W>;
+  if constexpr (WEST == 4) {
+    const P b = ld<T, VEC>(a.b, k), m = ld<T, VEC>(a.m, k), m2 = ld<T, VEC>(a.m2, k), m5 = ld<T, VEC>(a.m5, k),
+            ad = ld<T, VEC>(a.absd, k);
+    P u = ld<T, VEC>(a.u, k), v = ld<T, VEC>(a.v, k), w = ld<T, VEC>(a.ku, k), z;
+#pragma unroll
+    for (int i = 0; i < W; ++i) {
+      const T acc = (b.v[i] + m5.v[i] * (w.v[i] * w.v[i]) + ad.v[i] * v.v[i]) / (m.v[i] + m2.v[i] * u.v[i]);
+      v.v[i] = a.bdt * acc + v.v[i];
+      w.v[i] = a.cdt * acc + v.v[i];
+      u.v[i] = a.adt_next * v.v[i] + u.v[i];
+      z.v[i] = T(0);
+    }
+    st<T, VEC>(a.u, k, u);
+    st<T, VEC>(a.v, k, v);
+    st<T, VEC>(a.ku, k, w);
+    st<T, VEC>(a.b, k, z);
+    return;
+  }
   if constexpr (WEST == 3) {
     const P b = ld<T, VEC>(a.b, k), m = ld<T, VEC>(a.m, k);
     P u = ld<T, VEC>(a.u, k), v = ld<T, VEC>(a.v, k), z;
@@ -298,8 +324,9 @@ template <typename T, int WEST>
 __global__ void __launch_bounds__(kSharedThreads) rk_close_shared_kernel(const CloseArgs<T> a, const FusHaloDev h, int put,
                                                                          int gather) {
   const long long stride = (long long)gridDim.x * kSharedThreads;
+  // the Westervelt leapfrog puts (u, w): w lives in ku
   T* const xa = a.next_mode == 4 ? a.u : a.un;
-  T* const xb = a.next_mode == 4 ? a.v : a.ku;
+  T* const xb = (a.next_mode == 4 && WEST != 4) ? a.v : a.ku;
   for (long long i = (long long)blockIdx.x * kSharedThreads + threadIdx.x; i < h.nu; i += stride) {
     const long long k = h.uniq[i];
     const long long j0 = h.uoff[i], j1 = h.uoff[i + 1];
@@ -444,7 +471,7 @@ int open_entry(const T* u, const T* v, T* u0, T* v0, T* ku, const T* kv, T* un, 
 template <typename T, int WEST>
 int close_entry(T* u, T* v, T* u0, T* v0, T* ku, T* kv, T* un, T* b, T* m, const T* m0, T bdt,
                 T adt_next, int next_mode, int64_t n, int64_t* step, const uint8_t* skip, void* stream,
-                const T* m2 = nullptr, const T* m5 = nullptr) {
+                const T* m2 = nullptr, const T* m5 = nullptr, const T* absd = nullptr, T cdt = T(0)) {
   if (n < 0) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close: n < 0");
   if (next_mode < 0 || next_mode > 4) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close: next_mode");
   if (next_mode == 0 && kv == nullptr)
@@ -453,16 +480,19 @@ int close_entry(T* u, T* v, T* u0, T* v0, T* ku, T* kv, T* un, T* b, T* m, const
     return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close_westervelt_pw: null m0 / m2 / m5");
   if (WEST == 3 && (u == nullptr || v == nullptr || b == nullptr || m == nullptr))
     return fus_set_error(FUS_ERR_BAD_ARGUMENT, "leapfrog_close: null vector");
+  if (WEST == 4 && n > 0 && (u == nullptr || v == nullptr || ku == nullptr || b == nullptr || m == nullptr ||
+                             m2 == nullptr || m5 == nullptr || absd == nullptr))
+    return fus_set_error(FUS_ERR_BAD_ARGUMENT, "westervelt_leapfrog_close: null vector");
   const bool counts_step = step != nullptr && (next_mode == 2 || next_mode == 4);
   if (n == 0 && !counts_step) return 0;
   CloseArgs<T> a{u, v, u0, v0, ku, kv, un, b, m, m0, m2, m5, bdt, adt_next, next_mode, n,
-                 reinterpret_cast<long long*>(step), skip};
+                 reinterpret_cast<long long*>(step), skip, absd, cdt};
   cudaStream_t st_ = static_cast<cudaStream_t>(stream);
   if (n == 0) {
     // an empty range still ends the step (a rank whose owned dofs are all closed by
     // fus_rk_close_shared_*): one block touches no dof and advances the counter
     rk_close_kernel<T, false, WEST><<<1, kThreads, 0, st_>>>(a);
-  } else if (aligned16({u, v, u0, v0, ku, kv, un, b, m, m0, m2, m5})) {
+  } else if (aligned16({u, v, u0, v0, ku, kv, un, b, m, m0, m2, m5, absd})) {
     rk_close_kernel<T, true, WEST><<<grid_for(n / Vec<T>::W + 1), kThreads, 0, st_>>>(a);
   } else {
     rk_close_kernel<T, false, WEST><<<grid_for(n), kThreads, 0, st_>>>(a);
@@ -471,23 +501,27 @@ int close_entry(T* u, T* v, T* u0, T* v0, T* ku, T* kv, T* un, T* b, T* m, const
   return 0;
 }
 
-// variant 0: linear, 1: Westervelt "cells" form, 2: Westervelt pointwise form
+// variant 0: linear, 1: Westervelt "cells" form, 2: Westervelt pointwise form, 3: leapfrog, 4: Westervelt
+// leapfrog (reached through fus_westervelt_leapfrog_close_shared_* only: it also takes absd and cdt)
 template <typename T>
 int close_shared_entry(fus_halo* halo, int variant, int put_next, int gather, T* u, T* v, T* u0, T* v0, T* ku, T* un, T* b,
                        T* m, const T* m0, const T* m2, const T* m5, T bdt, T adt_next, int next_mode,
-                       void* stream) {
+                       void* stream, const T* absd = nullptr, T cdt = T(0)) {
   if (halo == nullptr) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close_shared: null halo handle");
-  if (variant < 0 || variant > 3) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close_shared: variant");
+  if (variant < 0 || variant > 4) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close_shared: variant");
   if (next_mode < 1 || next_mode > 4) return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close_shared: next_mode 1..4");
   if (((variant == 1 || variant == 2) && m0 == nullptr) || (variant == 2 && (m2 == nullptr || m5 == nullptr)) ||
       ((variant <= 1 || variant == 3) && m == nullptr))
     return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close_shared: null mass vector");
   if (variant == 3 && next_mode != 4)
     return fus_set_error(FUS_ERR_BAD_ARGUMENT, "rk_close_shared: the leapfrog variant takes next_mode 4");
+  if (variant == 4 && (u == nullptr || v == nullptr || ku == nullptr || b == nullptr || m == nullptr ||
+                       m2 == nullptr || m5 == nullptr || absd == nullptr))
+    return fus_set_error(FUS_ERR_BAD_ARGUMENT, "westervelt_leapfrog_close_shared: null vector");
   const FusHaloDev& h = *fus_halo_dev_of(halo);
   if (h.nu == 0) return 0;  // nothing shared: nobody ghosts my dofs, nobody waits for my signal
   CloseArgs<T> a{u, v, u0, v0, ku, nullptr, un, b, m, m0, m2, m5, bdt, adt_next, next_mode, h.size_local,
-                 nullptr, nullptr};
+                 nullptr, nullptr, absd, cdt};
   long long blocks = (h.nu + kSharedThreads - 1) / kSharedThreads;
   const long long cap = (long long)fus_num_sms() * 2;
   if (blocks > cap) blocks = cap;
@@ -499,6 +533,8 @@ int close_shared_entry(fus_halo* halo, int variant, int put_next, int gather, T*
     rk_close_shared_kernel<T, 1><<<(unsigned)blocks, kSharedThreads, 0, st_>>>(a, h, put, gat);
   } else if (variant == 3) {
     rk_close_shared_kernel<T, 3><<<(unsigned)blocks, kSharedThreads, 0, st_>>>(a, h, put, gat);
+  } else if (variant == 4) {
+    rk_close_shared_kernel<T, 4><<<(unsigned)blocks, kSharedThreads, 0, st_>>>(a, h, put, gat);
   } else {
     rk_close_shared_kernel<T, 2><<<(unsigned)blocks, kSharedThreads, 0, st_>>>(a, h, put, gat);
   }
@@ -592,6 +628,22 @@ extern "C" {
     return close_entry<T, 3>(u, v, nullptr, nullptr, nullptr, nullptr, nullptr, b,               \
                              const_cast<T*>(m), nullptr, dt_v, dt_u, 4, n, step_dev, skip_mask,  \
                              s);                                                                 \
+  }                                                                                              \
+  int fus_westervelt_leapfrog_close_##SFX(T* u, T* v, T* w, T* b, const T* m, const T* m2,       \
+                                          const T* m5, const T* absd, T bdt, T cdt, T adt,       \
+                                          int64_t n, int64_t* step_dev,                          \
+                                          const uint8_t* skip_mask, void* s) {                   \
+    return close_entry<T, 4>(u, v, nullptr, nullptr, w, nullptr, nullptr, b, const_cast<T*>(m),  \
+                             nullptr, bdt, adt, 4, n, step_dev, skip_mask, s, m2, m5, absd,      \
+                             cdt);                                                               \
+  }                                                                                              \
+  int fus_westervelt_leapfrog_close_shared_##SFX(fus_halo_t* halo, int put_next, int gather,     \
+                                                 T* u, T* v, T* w, T* b, const T* m,             \
+                                                 const T* m2, const T* m5, const T* absd, T bdt, \
+                                                 T cdt, T adt, void* s) {                        \
+    return close_shared_entry<T>(halo, 4, put_next, gather, u, v, nullptr, nullptr, w, nullptr,  \
+                                 b, const_cast<T*>(m), nullptr, m2, m5, bdt, adt, 4, s, absd,    \
+                                 cdt);                                                           \
   }                                                                                              \
   int fus_boundary_terms_##SFX(T* b, const T* vn, const int32_t* dof, const T* src,              \
                                const T* src2, const T* absb, T g, T dg, const T* gtab,           \

@@ -26,7 +26,8 @@ from . import precompute as pre
 from . import substrate as S
 from . import utils
 from .scatterer import HaloExchange, P2PHaloExchange, SymmFabric
-from .solver import LinearLeapfrog3D, LinearSpectral3D, WesterveltSpectral3D, linear_source, westervelt_source
+from .solver import (LinearLeapfrog3D, LinearSpectral3D, WesterveltLeapfrog3D, WesterveltSpectral3D, linear_source,
+                     westervelt_source)
 
 
 @dataclass
@@ -352,10 +353,14 @@ def linear_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0=150
 
 def westervelt_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0=1480.0, f0=1.1e6,
                       p0=None, beta=3.5, alpha_dB=0.2, source_predicate=None, absorbing_predicate=None,
-                      source_elements=None, element_amplitudes=None, element_delays=None,
+                      source_elements=None, element_amplitudes=None, element_delays=None, integrator="rk4",
                       **kw) -> WesterveltSpectral3D:
-    """cuda/demo_nonlinear_bowl.py:358-374 coefficients + the fused solver; phased-array keywords
-    as for ``linear_solver``."""
+    """cuda/demo_nonlinear_bowl.py:358-374 coefficients + the fused solver (``integrator``: "rk4", the
+    reference's scheme, or "leapfrog", pointwise mass form only); phased-array keywords as for
+    ``linear_solver``."""
+    if integrator not in ("rk4", "leapfrog"):
+        raise ValueError("integrator must be 'rk4' or 'leapfrog'")
+    cls = WesterveltLeapfrog3D if integrator == "leapfrog" else WesterveltSpectral3D
     if p0 is None:
         p0 = rho * c0 * 0.38557513826589934  # source velocity of the bowl demo (:66-67)
     delta = utils.compute_diffusivity_of_sound(2.0 * np.pi * f0, c0, alpha_dB)
@@ -365,7 +370,7 @@ def westervelt_solver(su: Setup, source_facets, absorbing_facets, rho=1000.0, c0
                                   kw, source_elements, element_amplitudes, element_delays)
     fd2, dJ2, bd2 = facet_group(su, absorbing_facets, absorbing_predicate)
     n1, n2 = bd1.shape[0], bd2.shape[0]
-    return WesterveltSpectral3D(
+    return cls(
         su.P, su.dtype, su.ndofs, su.dev["dofmap"], su.dev.get("G"), su.dev.get("detJ"), su.tables.dphi_1D,
         _full(su, nc, 1.0 / rho / c0 / c0), _full(su, nc, -2.0 * beta / rho / rho / c0**4),
         _full(su, nc, -1.0 / rho), _full(su, nc, -delta / rho / c0 / c0),

@@ -63,7 +63,7 @@ def multi_gpu_parity(P=4, n_per_rank=6, dtype=np.float64, nsteps=8, workload="li
     dt = problem.cfl_time_step(P, h * (1.0 - 2.0 * perturb), c0, f0, cfl)
     kw = dict(geometry=geometry, use_graph=use_graph)
     if integrator != "rk4":
-        kw["integrator"] = integrator  # linear workloads only
+        kw["integrator"] = integrator  # "leapfrog": linear, piston and westervelt (pointwise) workloads
         dt = 0.5 * dt
 
     su = problem.box_setup(P, ncells, lengths, dtype, rank, world, comm=group, grid=grid, perturb=perturb, seed=7,

@@ -335,6 +335,20 @@ class _RK4:
         if self.num_elements is not None:
             self._element_rows(src["src"], src["src2"])
 
+    def _facet_diagonal(self, group):
+        """Owner-complete diagonal of a facet group (``_facets``): its facet mass operator applied to
+        ones, reverse-exchanged once (peer-addressable with the peer-memory halo).  The compact lists
+        of ``_boundary_setup`` hold this rank's partial sums instead, which is what an assembly needs;
+        a close that applies the diagonal pointwise needs the complete one."""
+        torch = _torch()
+        d = torch.zeros(self.ndofs, dtype=self.T, device="cuda") if not self.p2p else self._zx()
+        if group is not None:
+            bd, dJ, fc = group
+            self._mass(torch.ones(self.ndofs, dtype=self.T, device="cuda"), fc, d, dJ, bd)
+        if self.halo is not None:
+            self.halo.reverse(d)
+        return d
+
     def _element_rows(self, src, src2):
         """CSR rows over ``_bdofs`` of the phased-array source: for every boundary dof, one entry
         (element, w[, w2]) per element whose facets contain it, w = the facet coefficient times
@@ -985,16 +999,7 @@ class LinearLeapfrog3D(LinearSpectral3D):
 
     def __init__(self, *args, **kw):
         super().__init__(*args, **kw)
-        torch = _torch()
-        # owner-complete diagonal of the absorbing facet term (the compact list of _boundary_setup
-        # holds this rank's partial sums, which is what the assembly needs)
-        self._absd = torch.zeros(self.ndofs, dtype=self.T, device="cuda") if not self.p2p else self._zx()
-        if self._abs_facets is not None:
-            bd2, dJ2, fc2 = self._abs_facets
-            ones = torch.ones(self.ndofs, dtype=self.T, device="cuda")
-            self._mass(ones, fc2, self._absd, dJ2, bd2)
-        if self.halo is not None:
-            self.halo.reverse(self._absd)
+        self._absd = self._facet_diagonal(self._abs_facets)
         self._mlf = None
         self._mlf_dt = None
 
@@ -1110,9 +1115,12 @@ class WesterveltSpectral3D(_RK4):
             self._mass(ones, fc, self.m0, dJ2, bd2)
         if self.halo is not None:
             self.halo.reverse(self.m0)
+        # the -1/(rho c) absorbing facets: a boundary-launch term of every RK stage; the leapfrog step
+        # applies them in its close instead (WesterveltLeapfrog3D)
+        self._abs_facets = self._facets(bfacet_dofmap2, detJ_f2, facet_coeff2_2)
         self._boundary_setup(src=self._facets(bfacet_dofmap1, detJ_f1, facet_coeff1_1),
                              src2=self._facets(bfacet_dofmap1, detJ_f1, facet_coeff2_1),
-                             absb=self._facets(bfacet_dofmap2, detJ_f2, facet_coeff2_2))
+                             absb=self._abs_facets if self.integrator == "rk4" else None)
         self.m.zero_()  # "cells" form: state-dependent part, accumulated per stage, zeroed by the close kernel
         self.m2 = self.m5 = None
         if not self._m_accum:
@@ -1154,3 +1162,110 @@ class WesterveltSpectral3D(_RK4):
             return super().stage_bytes() + (self.ncells - self.naff - self.ntri) * Nd * s + 6 * s * self.ndofs
         # pointwise: + second gather (vn) in the stage kernel; close passes 11 + 15 + 15 + 11 per step
         return super().stage_bytes() + s * self.ndofs + (13 - 10.25) * s * self.ndofs
+
+
+class WesterveltLeapfrog3D(WesterveltSpectral3D):
+    """The Westervelt problem of ``WesterveltSpectral3D`` (pointwise mass form) advanced with an
+    explicit second-order LEAPFROG scheme: ``u`` lives at whole steps, ``v`` at half steps and ``w``
+    is the velocity extrapolated to the whole step,
+
+        b = K(c3; u^n) + K(c4; w^n) + g(t_n) src + dg(t_n) src2
+        a = (b + m5 (w^n)^2 + absd v^{n-1/2}) / (m0 - dt/2 absd + m2 u^n)
+        v^{n+1/2} = v^{n-1/2} + dt a
+        w^{n+1}   = v^{n+1/2} + dt/2 a                      (= 1.5 v^{n+1/2} - 0.5 v^{n-1/2})
+        u^{n+1}   = u^n + dt v^{n+1/2}
+
+    with ``absd`` the owner-complete diagonal of the -1/(rho c) absorbing facets (time-centred by the
+    -dt/2 absd in the mass, as in ``LinearLeapfrog3D``).  The mass is diagonal and taken at ``u^n``,
+    the velocity terms at ``w^n``, so the step is explicit: ONE dual stiffness action
+    (``fus_stiffness2_*``) and 12 vector passes per step (``fus_westervelt_leapfrog_close_*``), against
+    RK4's four and 52.  The reference implements RK4 only, so the scheme is pinned to its numpy
+    restatement (``tests/westervelt_leapfrog_oracle.py``) and to its convergence order against RK4.
+
+    Same constructor as ``WesterveltSpectral3D``; ``mass_form="cells"`` raises ``ValueError``.  The
+    first ``rk4`` / ``steps`` call after ``init()`` kicks off from ``(u0, v0)`` with one eager pass
+    (``w = v0``, mass ``m0``: ``v`` goes back half a step).  After ``n`` steps ``u`` is ``u(t_n)`` and
+    ``v`` is ``v(t_n - dt/2)``."""
+
+    integrator = "leapfrog"
+
+    def __init__(self, *args, **kw):
+        super().__init__(*args, **kw)
+        if self.mass_form != "pointwise":
+            raise ValueError("WesterveltLeapfrog3D: only mass_form='pointwise' (the mass must be diagonal)")
+        self._absd = self._facet_diagonal(self._abs_facets)
+        # w is the velocity operand of the cell kernels, the role ku (vn) has in an RK stage: it takes that
+        # buffer, which is peer-addressable (the neighbours put w into its ghost slots), zeroed by init()
+        # and part of _state(); the 12 vectors then fit the peer-memory arena of problem.box_setup
+        self.w = self.ku
+        self._mm = None
+        self._mm_dt = None
+
+    @property
+    def u(self):
+        return self._uv[0][0]
+
+    @property
+    def v(self):
+        return self._uv[0][1]
+
+    def _wl_close(self, m, bdt, cdt, adt, count_step, skip=None, n=None):
+        u, v = self._uv[0]
+        check(fn("fus_westervelt_leapfrog_close", self.dtype)(
+            u.data_ptr(), v.data_ptr(), self.w.data_ptr(), self.b.data_ptr(), m.data_ptr(), self.m2.data_ptr(),
+            self.m5.data_ptr(), self._absd.data_ptr(), bdt, cdt, adt, self.nupd if n is None else n,
+            self.step_dev.data_ptr() if count_step else None, skip, current_stream()), "fus_westervelt_leapfrog_close")
+
+    def _kick(self, t0, dt):
+        """(u0, v0) -> v(t0 - dt/2), w = v0: half a step backwards with the acceleration at t0."""
+        self.w.copy_(self.v)
+        g, dg = self._source_at(0, dt, t0, False)
+        if self.num_elements is not None:
+            self._load_eager_row(t0, dt)
+        self._assemble_exchanged(0, g, dg, False, self.u, self.w)
+        self._wl_close(self.m0, -0.5 * dt, 0.5 * dt, 0.0, False)
+        if self.p2p and self.ndofs > self.nupd:
+            self.b[self.nupd:].zero_()  # the stand-alone reverse keeps the ghost sums; the steps expect them cleared
+
+    def rk4(self, t0, dt, nsteps):
+        """``nsteps`` leapfrog steps of size ``dt`` from ``t0`` (the name is the solvers' common
+        stepping entry point); returns the final time."""
+        if self._mm_dt != dt:
+            self._mm = (self.m0 - (0.5 * dt) * self._absd).contiguous()
+            self._mm_dt = dt
+        if not self._opened:
+            self._set_tables()
+            self._open_first()
+            self._kick(float(t0), dt)
+        return super().rk4(t0, dt, nsteps)
+
+    steps = rk4
+
+    def step_eager(self, dt):
+        raise NotImplementedError("WesterveltLeapfrog3D: use rk4 / steps")
+
+    def begin_steps(self):
+        """Peer-memory halo: put (u, w), the pair the next step's cell kernels read."""
+        if self.p2p:
+            self.halo.barrier()
+            self.halo.put(self.u, self.w)
+
+    def _enqueue_step(self, dt, t, use_table, parity=None):
+        """One leapfrog step: one stage whose cell-kernel input is (u, w) (``parity`` plays no role)."""
+        self._stage(0, dt, t, use_table, (self.u, self.w), None)
+
+    def _close(self, stage, dt, count_step, base, acc, skip=None, n=None):
+        self._wl_close(self._mm, dt, 0.5 * dt, dt, count_step, skip, n)
+
+    def _close_shared(self, stage, dt, base, acc):
+        u, v = self._uv[0]
+        check(fn("fus_westervelt_leapfrog_close_shared", self.dtype)(
+            self.halo.handle, 1, 1, u.data_ptr(), v.data_ptr(), self.w.data_ptr(), self.b.data_ptr(),
+            self._mm.data_ptr(), self.m2.data_ptr(), self.m5.data_ptr(), self._absd.data_ptr(), dt, 0.5 * dt, dt,
+            current_stream()), "fus_westervelt_leapfrog_close_shared")
+
+    def stage_bytes(self):
+        """Algorithmic HBM bytes of one leapfrog STEP: one dual stiffness action (two gathers) + 12
+        vector passes (8 reads + 4 writes per dof)."""
+        s = self.dtype.itemsize
+        return self._stiffness_bytes() + s * self.ndofs + 12 * s * self.ndofs

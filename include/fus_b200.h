@@ -461,6 +461,37 @@ int fus_leapfrog_close_f64(double* u, double* v, double* b, const double* m, dou
 int fus_leapfrog_close_f32(float* u, float* v, float* b, const float* m, float dt_v, float dt_u,
                            int64_t n, int64_t* step_dev, const uint8_t* skip_mask, void* stream);
 
+/* One LEAPFROG step of the Westervelt equation, pointwise mass form (u at whole steps, v at half
+ * steps, w the velocity extrapolated to the whole step):
+ *   a = (b + m5*w^2 + absd*v) / (m + m2*u) ; v += bdt*a ; w = v + cdt*a ; u += adt*v ; b = 0
+ * b = K(c3; u) + K(c4; w) + g src + dg src2 as assembled by fus_stiffness2_* (x = u, vn = w) and
+ * fus_boundary_terms_* with no absorbing diagonal: the absorbing term absd*v is taken here, with absd
+ * the owner-complete absorbing facet diagonal (-1/(rho c) facets applied to ones).  m2 = M(c2; 1),
+ * m5 = M(c5; 1).  The steps use m = m0 - (dt/2) absd and (bdt, cdt, adt) = (dt, dt/2, dt), which
+ * leaves w = 1.5 v^{n+1/2} - 0.5 v^{n-1/2}; the kick-off from (u0, v0) uses w = v0, m = m0 and
+ * (-dt/2, dt/2, 0).  8 reads + 4 writes per dof.  step_dev / skip_mask as for fus_rk_close_*. */
+int fus_westervelt_leapfrog_close_f64(double* u, double* v, double* w, double* b, const double* m,
+                                      const double* m2, const double* m5, const double* absd,
+                                      double bdt, double cdt, double adt, int64_t n, int64_t* step_dev,
+                                      const uint8_t* skip_mask, void* stream);
+int fus_westervelt_leapfrog_close_f32(float* u, float* v, float* w, float* b, const float* m,
+                                      const float* m2, const float* m5, const float* absd, float bdt,
+                                      float cdt, float adt, int64_t n, int64_t* step_dev,
+                                      const uint8_t* skip_mask, void* stream);
+
+/* The multi-GPU twin of fus_westervelt_leapfrog_close_*: variant 4 of the shared close of
+ * fus_rk_close_shared_* (which accepts variants 0-3 only, since its signature has no absd and no
+ * cdt).  Gathers the ghost sums of b, closes the shared dofs and, with put_next != 0, puts (u, w)
+ * into the neighbours' ghost slots - the pair the next step's cell kernels read. */
+int fus_westervelt_leapfrog_close_shared_f64(fus_halo_t* halo, int put_next, int gather, double* u,
+                                             double* v, double* w, double* b, const double* m,
+                                             const double* m2, const double* m5, const double* absd,
+                                             double bdt, double cdt, double adt, void* stream);
+int fus_westervelt_leapfrog_close_shared_f32(fus_halo_t* halo, int put_next, int gather, float* u,
+                                             float* v, float* w, float* b, const float* m,
+                                             const float* m2, const float* m5, const float* absd,
+                                             float bdt, float cdt, float adt, void* stream);
+
 /* Boundary-facet terms of one stage through precomputed diagonals on a compact
  * list of UNIQUE dofs: b[dof[i]] += g * src[i] + dg * src2[i] + vn[dof[i]] * absb[i].
  * Replaces the facet `mass_operator` launches of :546-551 (and
